@@ -2,7 +2,7 @@
 """bench.py -- GP vector-field evals/s of the multiple-shooting ELBO forward+backward step (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--scaling weak|strong]
-                    [--rows-scale F] [--no-parity-check] [--no-cpu-baseline]
+                    [--rows-scale F] [--no-parity-check] [--no-cpu-baseline] [--dump-outputs DIR]
 
 Workload (``config.workload``): BASELINE.json configs[3], "MoCap GPODE shooting variant on long synthetic
 MoCap-shaped trajectories": latent D=5 -> D_obs=50 through a fixed orthonormal decoder, M=100 inducing points, S=256
@@ -23,6 +23,10 @@ every parameter gradient of a 60 000-segment problem of the same shape -- the sa
 value = segments x 4 vector-field evaluations (the reference's own NFE count for this step) / step time, aggregated
 over all GPUs. ``e2e`` repeats the measurement with the observations copied from pinned host memory and the loss
 read back to the host inside every timed step.
+
+``--dump-outputs DIR`` writes what the last timed step returned to its caller on rank 0: ``loss.npy`` and one
+``grad.<parameter name>.npy`` per parameter gradient. Inputs, initial parameters and the random draws are seeded, so
+two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -49,6 +53,33 @@ UNIT = "evals/s"
 def f_vf(D, S, M):
     """Algorithmic flops of one vector-field evaluation of one row (SURVEY.md section 8d)."""
     return D * (S * (2 * D + 4) + M * (3 * D + 4))
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def step_outputs(model, loss):
+    """What one ELBO step hands its caller, copied to the host: the loss and every parameter's gradient."""
+    out = {"loss": loss.detach().cpu().numpy()}
+    for name, p in model.named_parameters():
+        if p.grad is not None:
+            out["grad." + name] = p.grad.detach().cpu().numpy()
+    return out
+
+
+def write_outputs(out_dir, arrays, limit=DUMP_LIMIT_BYTES):
+    """One float32 / float64 ``<name>.npy`` per array, at most ``limit`` bytes in all. If the arrays are larger, each
+    one above its equal share of the limit is replaced by a fixed, seeded sample of its flattened elements (in index
+    order), so that the files of two runs still correspond element for element."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = limit // max(1, len(arrays)) - 4096   # 4 KB per file for the .npy header
+    too_big = sum(a.nbytes + 4096 for a in arrays.values()) > limit
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64 if a.dtype == np.float64 else np.float32)
+        if too_big and a.nbytes > share:
+            idx = np.random.default_rng(0).choice(a.size, share // a.itemsize, replace=False)
+            a = a.reshape(-1)[np.sort(idx)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ----------------------------------------------------------------------------------------------------------------------
@@ -241,7 +272,7 @@ def run_reference(args):
     if rank != 0:
         return
     w = WORKLOAD
-    cb = cpu_elbo_timing(w, steps=max(args.steps, 3), warmup=max(args.warmup, 1))
+    cb = cpu_elbo_timing(w, steps=args.steps, warmup=args.warmup)
     line = {"impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": cb["ms_per_step"], "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -376,7 +407,14 @@ def run_ours(args):
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    ms_total = timed(args.steps, lambda: step(resident))
+    last = {}
+
+    def timed_step():
+        last["loss"] = step(resident)
+
+    ms_total = timed(args.steps, timed_step)
+    # copied now: the graph's loss and gradient buffers are overwritten by the passes below
+    outputs = step_outputs(model, last["loss"]) if args.dump_outputs and rank == 0 else None
     _lib.reset_launch_count()
     for _ in range(args.steps):   # the kernels a step launches are counted on eager launches (a graph replay runs the same)
         eager_step(ys_dev)
@@ -451,7 +489,7 @@ def run_ours(args):
                   "last one is awaited inside the timed region", "cpu_affinity_rank0": cpus}
 
     # ---- per-kernel breakdown (separate pass: CUDA events around every C-ABI call, MEDIAN over n_prof steps) ----
-    n_prof = max(10, args.steps)
+    n_prof = args.steps
     _lib.profile_start()
     for _ in range(n_prof):
         eager_step(ys_dev)   # eager launches: the events bracket the individual C-ABI calls
@@ -553,6 +591,8 @@ def run_ours(args):
                 "kernels_ms_per_step": kern, "own_kernels_share_of_step": ours_ms / ms_per_step,
                 "roofline": roof, "cpu_baseline": cpu, "clocks": clocks, "parity_precheck": parity,
                 "loss": getattr(e2e_body, "last", None)}
+        if outputs is not None:
+            write_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     if world > 1:
         torch.distributed.destroy_process_group()
@@ -570,7 +610,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="time eager launches instead of the captured CUDA graph")
     ap.add_argument("--no-parity-check", action="store_true", help="skip the oracle check before timing (profiling)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss and parameter gradients of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup not negative")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the CUDA path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

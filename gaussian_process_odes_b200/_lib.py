@@ -75,6 +75,8 @@ SIGNATURES = {
     "gpode_rk4_bwd_large": (_I, [_P, _CP, _P, _I, _L, _P, _P, _P, _P, _P, _P, _P]),
     "gpode_dopri5_large_work_floats": (_L, [_I, _L]),
     "gpode_dopri5_fwd_large": (_I, [_P, _CP, _P, _P, _I, _L, _D, _D, _P, _P, _P, _I, _P]),
+    "gpode_dopri5_fwd_large_ckpt": (_I, [_P, _CP, _P, _P, _I, _L, _D, _D, _P, _P, _P, _I, _P, _I, _P]),
+    "gpode_dopri5_bwd_large": (_I, [_P, _CP, _P, _I, _L, _P, _P, _I, _I, _P, _P, _P, _P]),
     "gpode_shoot_fwd": (_I, [_P, _I, _I, _I, ctypes.POINTER(GpodeShoot), _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "gpode_shoot_bwd": (_I, [_P, _I, _I, _I, ctypes.POINTER(GpodeShoot), _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "gpode_acc_header_floats": (_L, []),
@@ -178,7 +180,9 @@ KERNELS_PER_CALL = {
     # per RK4 step: forward 4 evaluations x 2 kernels + 4 stage kernels; adjoint 4 VJPs + 8 element-wise kernels
     "gpode_rk4_fwd_large_dev": 12, "gpode_rk4_bwd_large": 16,
     # start: 2 evaluations (2 kernels each) + 6 small kernels; every attempt of the device-side loop launches 21 more
-    "gpode_dopri5_fwd_large": 10 + 21,
+    "gpode_dopri5_fwd_large": 10 + 21, "gpode_dopri5_fwd_large_ckpt": 10 + 21,
+    # per accepted step: 6 VJPs (2 kernels each) + 7 element-wise kernels; once: the VJP at x0 + the grad_x0 kernel
+    "gpode_dopri5_bwd_large": 19 + 3,
 }
 assert all(isinstance(v, int) for v in KERNELS_PER_CALL.values()), "KERNELS_PER_CALL holds launch counts"
 assert set(KERNELS_PER_CALL) <= set(SIGNATURES), sorted(set(KERNELS_PER_CALL) - set(SIGNATURES))

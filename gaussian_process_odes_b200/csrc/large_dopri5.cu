@@ -1,4 +1,4 @@
-// Adaptive dopri5 for 8 < D <= 64 with the controller ON THE DEVICE (forward only).
+// Adaptive dopri5 for 8 < D <= 64 with the controller ON THE DEVICE, and its discrete adjoint.
 //
 // torchdiffeq 0.2.0's dopri5 as called by Flow.forward (reference src/core/flow.py:84-90; restated in
 // oracle/torchdiffeq_shim): Dormand-Prince 5(4), FSAL, whole-batch RMS error norm, float64 time, Hairer initial step,
@@ -10,6 +10,13 @@
 // of a CUDA-graph WHILE node whose condition the controller kernel sets with cudaGraphSetConditional: the loop runs on
 // the device until the last output time is covered, the host enqueues one graph launch and never reads a value.
 // Arithmetic (operation order, float32 state, float64 time) follows dopri5_impl.cuh, which serves D <= 8.
+//
+// Training: the accept kernel can also record every accepted step (state at its start, the seven raw stage values, the
+// float32 step size, and which step / abscissa produced each output) in the checkpoint block of
+// gpode_dopri5_ckpt_floats. gpode_dopri5_bwd_large walks those steps backwards -- the algorithm of
+// dopri5_impl.cuh::dopri5_bwd_kernel as a stream-ordered chain of launches around the large-D VJP (large_bwd.cu), the
+// way gpode_rk4_bwd_large restates rk4_bwd_kernel. Step sizes are constants there, as in torchdiffeq, whose controller
+// runs on a detached error ratio, so the two initial-step evaluations get no cotangent.
 #include "common.cuh"
 #include "../../include/gpode_b200.h"
 #include <deque>
@@ -44,7 +51,28 @@ struct LdCtrl {
     float dts_used, h0, d1;
     int jout, jlo, jhi, accept, done;
     int nfe, n_acc, n_rej, status, attempt, max_attempts;
+    int cap;                   // checkpoint capacity in accepted steps; 0: no checkpoints
 };
+
+// checkpoint block (layout of gpode_dopri5_ckpt_floats): y [cap][B][D] | k [cap][7][B][D] | dt [cap] | out_x [Tg] |
+// out_step [Tg]. k holds the RAW vector-field values (the direction sign is applied where they are used).
+struct LdCkpt {
+    float* y;
+    float* k;
+    float* dt;
+    float* out_x;
+    int32_t* out_step;
+};
+
+LdCkpt ld_ckpt(float* ckpt, int cap, int64_t n, int Tg) {
+    LdCkpt k;
+    k.y = ckpt;
+    k.k = ckpt ? ckpt + (int64_t)cap * n : nullptr;
+    k.dt = ckpt ? k.k + (int64_t)cap * 7 * n : nullptr;
+    k.out_x = ckpt ? k.dt + cap : nullptr;
+    k.out_step = ckpt ? reinterpret_cast<int32_t*>(k.out_x + Tg) : nullptr;
+    return k;
+}
 
 constexpr int kLdThreads = 256;
 constexpr int kLdMaxBlocks = 2368;
@@ -96,13 +124,22 @@ __device__ double ld_total(const double* __restrict__ partial, const int n) {
     return t;
 }
 
-__global__ void ld_start_kernel(LdCtrl* c, const double* __restrict__ t, const int Tg, const int max_attempts) {
-    const double dir = (Tg > 1 && t[Tg - 1] < t[0]) ? -1.0 : 1.0;
+// +1 / -1: a decreasing grid is integrated as -f over -t
+__device__ __forceinline__ double ld_dir(const double* __restrict__ t, const int Tg) {
+    return (Tg > 1 && t[Tg - 1] < t[0]) ? -1.0 : 1.0;
+}
+
+__global__ void ld_start_kernel(LdCtrl* c, const double* __restrict__ t, const int Tg, const int max_attempts,
+                                const int cap, int32_t* __restrict__ out_step) {
+    const double dir = ld_dir(t, Tg);
     c->dir = dir;
     c->t1 = dir * t[0];
     c->dt = 0.0;
     c->jout = 1; c->jlo = c->jhi = 0; c->accept = 0; c->done = Tg <= 1;
     c->nfe = 2; c->n_acc = 0; c->n_rej = 0; c->status = 0; c->attempt = 0; c->max_attempts = max_attempts;
+    c->cap = cap;
+    if (out_step != nullptr)   // outputs no accepted step produces (output 0, or a failed solve) stay -1
+        for (int j = 0; j < Tg; ++j) out_step[j] = -1;
 }
 
 // s0 = sum (y / sc)^2, s1 = sum (f / sc)^2, sc = atol + |y| rtol
@@ -157,6 +194,9 @@ __device__ void ld_loop_head(LdCtrl* c, const double* __restrict__ t, const int 
     } else if (c->attempt >= c->max_attempts || !(c->t1 + c->dt > c->t1)) {
         c->status = c->attempt >= c->max_attempts ? 1 : 2;   // attempt limit / step-size underflow
         c->done = 1;
+    } else if (c->cap > 0 && c->n_acc >= c->cap) {
+        c->status = 3;   // checkpoint capacity exhausted: the caller retries with a larger one
+        c->done = 1;
     }
 }
 
@@ -184,21 +224,29 @@ struct LdBufs {
     float* tmp;    // scratch of the vector-field evaluation
 };
 
-// stage input i (1..6): Y_i = Y + sum_{l < i} (fsign K_l) (beta_{i-1,l} dt)
+// stage input i (1..6) at element e: Y_i = Y + sum_{l < i} (fsign K_l) (beta_{i-1,l} dt), bd[l] = beta_{i-1,l} dt.
+// The forward and the backward both evaluate it here, so the adjoint linearises at bit-identical stage inputs.
+__device__ __forceinline__ void ld_stage_coefs(const int i, const float dts, float (&bd)[6]) {
+#pragma unroll
+    for (int l = 0; l < 6; ++l) bd[l] = __fmul_rn(ldBeta[i - 1][l], dts);
+}
+__device__ __forceinline__ float ld_stage_input(const LdBufs& b, const int i, const float (&bd)[6], const float fs,
+                                                const int64_t e) {
+    float s = 0.f;
+#pragma unroll
+    for (int l = 0; l < 6; ++l)
+        if (l < i) s = fmaf(fs * b.K[l][e], bd[l], s);
+    return b.Y[e] + s;
+}
+
 __global__ void ld_stage_kernel(const LdCtrl* __restrict__ c, const int i, const LdBufs b, float* __restrict__ out,
                                 const int64_t n) {
     if (c->done) return;
-    const float dts = (float)c->dt, fs = (float)c->dir;
+    const float fs = (float)c->dir;
     float bd[6];
-#pragma unroll
-    for (int l = 0; l < 6; ++l) bd[l] = __fmul_rn(ldBeta[i - 1][l], dts);
-    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (int64_t)gridDim.x * blockDim.x) {
-        float s = 0.f;
-#pragma unroll
-        for (int l = 0; l < 6; ++l)
-            if (l < i) s = fmaf(fs * b.K[l][e], bd[l], s);
-        out[e] = b.Y[e] + s;
-    }
+    ld_stage_coefs(i, (float)c->dt, bd);
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (int64_t)gridDim.x * blockDim.x)
+        out[e] = ld_stage_input(b, i, bd, fs, e);
 }
 
 __global__ void __launch_bounds__(kLdThreads)
@@ -271,14 +319,28 @@ ld_ctrl_kernel(LdCtrl* c, const double* __restrict__ partial, const int nb, cons
     cudaGraphSetConditional(handle, c->done ? 0u : 1u);
 }
 
-// accepted step: dense output at the requested times inside it, then Y <- Y1, K0 <- K6 (FSAL)
+// accepted step: dense output at the requested times inside it, then Y <- Y1, K0 <- K6 (FSAL). With checkpoints
+// (ck.y != NULL) the step's start state, its seven stage values, dt and its outputs' step / abscissa go to slot n_acc-1.
 __global__ void ld_accept_kernel(const LdCtrl* __restrict__ c, const LdBufs b, const double* __restrict__ t,
-                                 float* __restrict__ xs, const int64_t n) {
+                                 float* __restrict__ xs, const int64_t n, const LdCkpt ck) {
     if (!c->accept) return;
     const float dts = c->dts_used, fs = (float)c->dir;
     const int jlo = c->jlo, jhi = c->jhi;
     const double t1 = c->t1_used, t1n = c->t1n_used, dir = c->dir;
+    const int64_t slot = (int64_t)c->n_acc - 1;
+    if (ck.y != nullptr && blockIdx.x == 0 && threadIdx.x == 0) {
+        ck.dt[slot] = dts;
+        for (int jo = jlo; jo < jhi; ++jo) {
+            ck.out_step[jo] = (int32_t)slot;
+            ck.out_x[jo] = (float)((dir * t[jo] - t1) / (t1n - t1));
+        }
+    }
     for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (int64_t)gridDim.x * blockDim.x) {
+        if (ck.y != nullptr) {
+            ck.y[slot * n + e] = b.Y[e];
+#pragma unroll
+            for (int l = 0; l < 7; ++l) ck.k[(slot * 7 + l) * n + e] = b.K[l][e];
+        }
         const float yn = b.Y1[e], kn = b.K[6][e];
         if (jhi > jlo) {
             const float y0 = b.Y[e], f0 = fs * b.K[0][e], fn = fs * kn, ymj = b.YM[e];
@@ -335,6 +397,101 @@ void ld_reap(bool all) {
     }
 }
 
+// ---- discrete adjoint (restates dopri5_impl.cuh::dopri5_bwd_kernel; kb are cotangents of the INTEGRATED stage values
+// fsign K, so the VJP of the raw field at stage i takes the cotangent fsign kb_i) ---------------------------------------
+struct LdAdj {
+    float* kb[7];  // cotangents of the seven stage values of the current step; kb[0] is kappa (FSAL) for the step before
+    float* yb0;    // cotangent of the step's start state; lambda for the step before
+    float* Yi;     // stage input of the next VJP
+    float* cot;    // fsign kb_i: cotangent of the raw field value at that stage
+    float* Yb;     // result of the VJP
+};
+
+// accepted step n as the forward saw it: Y = its start state, K = its seven raw stage values
+LdBufs ld_step_view(const LdCkpt& ck, const int64_t slot, const int64_t n) {
+    LdBufs b = {};
+    b.Y = ck.y + slot * n;
+    for (int l = 0; l < 7; ++l) b.K[l] = ck.k + (slot * 7 + l) * n;
+    return b;
+}
+
+// Step `step` begins: lambda / kappa (yb0 / kb[0] of the step after it, zero for the last one) and the cotangents of the
+// outputs interpolated inside it seed kb[0..6] and yb0 through the dense-output quartic; then stage 7's input / cotangent.
+__global__ void ld_adj_seed_kernel(const LdCkpt ck, const LdBufs sv, const int step, const int first,
+                                   const double* __restrict__ t, const int Tg, const float* __restrict__ gxs,
+                                   const LdAdj a, const int64_t n) {
+    const float dt = ck.dt[step], fs = (float)ld_dir(t, Tg);
+    int jlo = Tg, jhi = 0;   // outputs of this step: a contiguous run of the (monotone) output table
+    for (int j = 1; j < Tg; ++j)
+        if (ck.out_step[j] == step) {
+            jlo = min(jlo, j);
+            jhi = j + 1;
+        }
+    float bd[6], cm[7];   // bd: row 6 of beta times dt -- stage 7's input, which is also the step's end state y1
+    ld_stage_coefs(6, dt, bd);
+#pragma unroll
+    for (int l = 0; l < 7; ++l) cm[l] = __fmul_rn(dt, ldCMid[l]);
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (int64_t)gridDim.x * blockDim.x) {
+        float yb0 = 0.f, yb1 = first ? 0.f : a.yb0[e], ybm = 0.f, fb0 = 0.f, fb1 = first ? 0.f : a.kb[0][e];
+        for (int jo = jhi - 1; jo >= jlo; --jo) {
+            if (ck.out_step[jo] != step) continue;
+            const float x = ck.out_x[jo], x2 = x * x, x3 = x2 * x, x4 = x2 * x2;
+            const float g = gxs[(int64_t)jo * n + e];
+            yb0 = fmaf(g, 1.f - 11.f * x2 + 18.f * x3 - 8.f * x4, yb0);
+            yb1 = fmaf(g, -5.f * x2 + 14.f * x3 - 8.f * x4, yb1);
+            ybm = fmaf(g, 16.f * x2 - 32.f * x3 + 16.f * x4, ybm);
+            fb0 = fmaf(g, dt * (x - 4.f * x2 + 5.f * x3 - 2.f * x4), fb0);
+            fb1 = fmaf(g, dt * (x2 - 3.f * x3 + 2.f * x4), fb1);
+        }
+        float kb6 = 0.f;
+#pragma unroll
+        for (int l = 0; l < 7; ++l) {
+            float v = (l < 6 ? bd[l] * yb1 : 0.f) + cm[l] * ybm;
+            if (l == 0) v += fb0;
+            if (l == 6) v += fb1;
+            a.kb[l][e] = v;
+            if (l == 6) kb6 = v;
+        }
+        a.yb0[e] = yb0 + (yb1 + ybm);
+        a.Yi[e] = ld_stage_input(sv, 6, bd, fs, e);
+        a.cot[e] = fs * kb6;
+    }
+}
+
+// After the VJP of stage i (1..6): yb0 += Yb, kb_l += beta_{i-1,l} dt Yb (l < i); then the input / cotangent of stage
+// i-1, or for i == 1 of the first step the cotangent of f(y0) (the VJP at y0 itself).
+__global__ void ld_adj_stage_kernel(const LdCkpt ck, const LdBufs sv, const int step, const int i,
+                                    const double* __restrict__ t, const int Tg, const LdAdj a, const int64_t n) {
+    const float dt = ck.dt[step], fs = (float)ld_dir(t, Tg);
+    float bd[6], bn[6];
+    ld_stage_coefs(i, dt, bd);
+    if (i > 1) ld_stage_coefs(i - 1, dt, bn);
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (int64_t)gridDim.x * blockDim.x) {
+        const float yb = a.Yb[e];
+        a.yb0[e] += yb;
+        float kbn = 0.f;
+#pragma unroll
+        for (int l = 0; l < 6; ++l)
+            if (l < i) {
+                const float v = fmaf(bd[l], yb, a.kb[l][e]);
+                a.kb[l][e] = v;
+                if (l == i - 1) kbn = v;
+            }
+        if (i > 1) {
+            a.Yi[e] = ld_stage_input(sv, i - 1, bn, fs, e);
+            a.cot[e] = fs * kbn;
+        } else if (step == 0) {
+            a.cot[e] = fs * kbn;
+        }
+    }
+}
+
+// grad_x0 = lambda + grad_xs[0] (output 0 is x0 itself), lambda = yb0 + the VJP at y0
+__global__ void ld_adj_x0_kernel(const LdAdj a, const float* __restrict__ gxs, float* __restrict__ gx0, const int64_t n) {
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (int64_t)gridDim.x * blockDim.x)
+        gx0[e] = (a.yb0[e] + a.Yb[e]) + gxs[e];
+}
+
 }  // namespace
 
 // work layout (floats): Y | K0..K6 | Ys | Y1 | YM | tmp  (12 B D), then 8-byte aligned: partial sums
@@ -343,17 +500,18 @@ extern "C" int64_t gpode_dopri5_large_work_floats(int D, int64_t B) {
     return 12 * B * (int64_t)D + 2 + 2 * (2 * (int64_t)kLdMaxBlocks) + (int64_t)(sizeof(LdCtrl) + 3) / 4 + 2;
 }
 
-extern "C" int gpode_dopri5_fwd_large(const float* packed_large, const gpode_cache_t* c, const float* x0, const double* t,
-                                      int Tg, int64_t B, double rtol, double atol, float* xs, float* work,
-                                      int32_t* stats_out, int max_attempts, void* stream) {
+namespace {
+
+int ld_fwd(const float* packed_large, const gpode_cache_t* c, const float* x0, const double* t, int Tg, int64_t B,
+           double rtol, double atol, float* xs, float* work, int32_t* stats_out, int max_attempts, float* ckpt, int cap,
+           cudaStream_t st) {
     GPODE_CHECK_ARG(c != nullptr && c->D > GPODE_MAX_D && c->D <= GPODE_MAX_D_LARGE, "large-D path needs %d < D <= %d",
                     GPODE_MAX_D, GPODE_MAX_D_LARGE);
     GPODE_CHECK_ARG(Tg >= 1 && B >= 0 && max_attempts >= 1, "bad sizes Tg=%d B=%lld", Tg, (long long)B);
     GPODE_CHECK_ARG(packed_large && x0 && t && xs && work && stats_out, "NULL argument");
-    cudaStream_t st = (cudaStream_t)stream;
-    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    GPODE_CUDA(cudaStreamIsCapturing(st, &cap));
-    GPODE_CHECK_ARG(cap == cudaStreamCaptureStatusNone,
+    cudaStreamCaptureStatus capturing = cudaStreamCaptureStatusNone;
+    GPODE_CUDA(cudaStreamIsCapturing(st, &capturing));
+    GPODE_CHECK_ARG(capturing == cudaStreamCaptureStatusNone,
                     "gpode_dopri5_fwd_large builds its own CUDA graph (device-side while loop) and cannot run inside a "
                     "stream capture");
     const int D = c->D;
@@ -376,11 +534,12 @@ extern "C" int gpode_dopri5_fwd_large(const float* packed_large, const gpode_cac
     const unsigned g = ld_grid(n);
     const double n_elem = (double)n;
     const float rt = (float)rtol, at = (float)atol;
+    const LdCkpt ck = ld_ckpt(ckpt, cap, n, Tg);
 
     // ---- start: y = x0, f0, initial step (two evaluations) ----
     GPODE_CUDA(cudaMemcpyAsync(b.Y, x0, sizeof(float) * n, cudaMemcpyDeviceToDevice, st));
     GPODE_CUDA(cudaMemcpyAsync(xs, x0, sizeof(float) * n, cudaMemcpyDeviceToDevice, st));
-    ld_start_kernel<<<1, 1, 0, st>>>(ctrl, t, Tg, max_attempts);
+    ld_start_kernel<<<1, 1, 0, st>>>(ctrl, t, Tg, max_attempts, ckpt ? cap : 0, ck.out_step);
     if (int rc = gpode_vf_large_eval(packed_large, c, b.Y, b.tmp, b.K[0], B, st)) return rc;
     ld_norm01_kernel<<<g, kLdThreads, 0, st>>>(b.Y, b.K[0], rt, at, n, partial);
     ld_init1_kernel<<<1, kLdThreads, 0, st>>>(ctrl, partial, (int)g, n_elem);
@@ -418,7 +577,7 @@ extern "C" int gpode_dopri5_fwd_large(const float* packed_large, const gpode_cac
     if (rc == 0) {
         ld_err_kernel<<<g, kLdThreads, 0, cs>>>(ctrl, b, rt, at, n, partial);
         ld_ctrl_kernel<<<1, kLdThreads, 0, cs>>>(ctrl, partial, (int)g, n_elem, t, Tg, handle);
-        ld_accept_kernel<<<g, kLdThreads, 0, cs>>>(ctrl, b, t, xs, n);
+        ld_accept_kernel<<<g, kLdThreads, 0, cs>>>(ctrl, b, t, xs, n, ck);
     }
     cudaGraph_t captured = nullptr;
     cudaError_t ce = cudaStreamEndCapture(cs, &captured);
@@ -445,6 +604,66 @@ extern "C" int gpode_dopri5_fwd_large(const float* packed_large, const gpode_cac
     GPODE_CUDA(cudaEventCreateWithFlags(&pend.ev, cudaEventDisableTiming));
     GPODE_CUDA(cudaEventRecord(pend.ev, st));
     g_ld_pending.push_back(pend);
+    GPODE_LAUNCH_CHECK();
+    return 0;
+}
+
+}  // namespace
+
+extern "C" int gpode_dopri5_fwd_large(const float* packed_large, const gpode_cache_t* c, const float* x0, const double* t,
+                                      int Tg, int64_t B, double rtol, double atol, float* xs, float* work,
+                                      int32_t* stats_out, int max_attempts, void* stream) {
+    return ld_fwd(packed_large, c, x0, t, Tg, B, rtol, atol, xs, work, stats_out, max_attempts, nullptr, 0,
+                  (cudaStream_t)stream);
+}
+
+extern "C" int gpode_dopri5_fwd_large_ckpt(const float* packed_large, const gpode_cache_t* c, const float* x0,
+                                           const double* t, int Tg, int64_t B, double rtol, double atol, float* xs,
+                                           float* work, int32_t* stats_out, int max_attempts, float* ckpt, int cap,
+                                           void* stream) {
+    GPODE_CHECK_ARG(ckpt != nullptr && cap > 0, "checkpointing needs a block and cap > 0 (cap=%d)", cap);
+    return ld_fwd(packed_large, c, x0, t, Tg, B, rtol, atol, xs, work, stats_out, max_attempts, ckpt, cap,
+                  (cudaStream_t)stream);
+}
+
+// work: 11 B D floats (kb[0..6], yb0, stage input, cotangent, VJP result)
+extern "C" int gpode_dopri5_bwd_large(const float* packed_bwd, const gpode_cache_t* c, const double* t, int Tg, int64_t B,
+                                      const float* grad_xs, const float* ckpt, int cap, int n_accepted, float* grad_x0,
+                                      float* acc_large, float* work, void* stream) {
+    GPODE_CHECK_ARG(c != nullptr && c->D > GPODE_MAX_D && c->D <= GPODE_MAX_D_LARGE, "large-D path needs %d < D <= %d",
+                    GPODE_MAX_D, GPODE_MAX_D_LARGE);
+    GPODE_CHECK_ARG(Tg >= 1 && B >= 0, "bad sizes Tg=%d B=%lld", Tg, (long long)B);
+    GPODE_CHECK_ARG(cap > 0 && n_accepted >= 0 && n_accepted <= cap, "n_accepted=%d outside 0..cap=%d", n_accepted, cap);
+    if (B == 0) return 0;
+    GPODE_CHECK_ARG(packed_bwd && t && grad_xs && ckpt && grad_x0 && acc_large && work, "NULL argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    const int D = c->D, M = c->M, S = c->S;
+    const int64_t n = B * D;
+    if (Tg == 1 || n_accepted == 0) {   // no step: x0 reaches the loss only as output 0
+        GPODE_CUDA(cudaMemcpyAsync(grad_x0, grad_xs, sizeof(float) * n, cudaMemcpyDeviceToDevice, st));
+        return 0;
+    }
+    const LdCkpt ck = ld_ckpt(const_cast<float*>(ckpt), cap, n, Tg);
+    LdAdj a;
+    for (int l = 0; l < 7; ++l) a.kb[l] = work + l * n;
+    a.yb0 = work + 7 * n;
+    a.Yi = work + 8 * n;
+    a.cot = work + 9 * n;
+    a.Yb = work + 10 * n;
+    const unsigned g = ld_grid(n);
+    for (int step = n_accepted - 1; step >= 0; --step) {
+        const LdBufs sv = ld_step_view(ck, step, n);
+        ld_adj_seed_kernel<<<g, kLdThreads, 0, st>>>(ck, sv, step, step == n_accepted - 1, t, Tg, grad_xs, a, n);
+        for (int i = 6; i >= 1; --i) {
+            if (int rc = gpode_vf_bwd_large(packed_bwd, D, M, S, a.Yi, sv.K[i], a.cot, a.Yb, acc_large, B, st)) return rc;
+            ld_adj_stage_kernel<<<g, kLdThreads, 0, st>>>(ck, sv, step, i, t, Tg, a, n);
+        }
+        GPODE_LAUNCH_CHECK();
+    }
+    // the first step's k1 = f(y0) has no step before it to hand its cotangent to: one more VJP, at y0
+    const LdBufs s0 = ld_step_view(ck, 0, n);
+    if (int rc = gpode_vf_bwd_large(packed_bwd, D, M, S, s0.Y, s0.K[0], a.cot, a.Yb, acc_large, B, st)) return rc;
+    ld_adj_x0_kernel<<<g, kLdThreads, 0, st>>>(a, grad_xs, grad_x0, n);
     GPODE_LAUNCH_CHECK();
     return 0;
 }

@@ -461,7 +461,7 @@ def shooting_step(ss, t2, Z, ell, var, nu, omega, phase, w, ys, W, bias, lik_var
 
 
 MAX_D_REGISTER = 8    # GPODE_MAX_D: differentiable register-resident kernels
-MAX_D_LARGE = 64      # GPODE_MAX_D_LARGE: tcgen05 forward + FP32 VJP kernels (rk4 differentiable, dopri5 forward)
+MAX_D_LARGE = 64      # GPODE_MAX_D_LARGE: tcgen05 forward + large-D VJP kernels (rk4 and dopri5 differentiable)
 
 
 def _large_d_call(name, x, t, Z, ell, var, nu, omega, phase, w):
@@ -731,37 +731,85 @@ class _Dopri5(torch.autograd.Function):
         return gx0, None, g_Z, g_ell, g_var, g_nu.reshape(ctx.nu_shape), None, None, None, None, None, None
 
 
-def _dopri5_large_d(x0, t, Z, ell, var, nu, omega, phase, w, rtol, atol, max_attempts=100000):
-    """dopri5 for 8 < D <= 64, forward only: torchdiffeq 0.2.0's controller (whole-batch RMS norm, float64 time, Hairer
-    initial step with order 4, safety 0.9 / growth <= 10 / shrink >= 0.2, quartic dense output) ON THE DEVICE --
-    ``gpode_dopri5_fwd_large``: one attempt = six evaluations on the tcgen05 vector-field kernels + element-wise stage /
-    error kernels + a one-CTA controller kernel, looped by a CUDA-graph WHILE node whose condition the controller sets.
-    The host enqueues one graph launch and reads nothing back (the reference synchronises once per attempt)."""
-    tensors = (x0, Z, ell, var, nu)
-    if torch.is_grad_enabled() and any(a.requires_grad for a in tensors):
-        raise _lib.GpodeError("state dimension %d > %d: dopri5 is forward-only there (rk4 is differentiable)"
-                              % (Z.shape[1], MAX_D_REGISTER))
-    lib = _lib.load()
-    field = LargeField(Z, ell, var, nu, omega, phase, w)
+def _dopri5_large_setup(field, x0, t):
     xc = f32(x0, "x0")
     if xc.ndim != 2 or xc.shape[1] != field.D:
         raise _lib.GpodeError("x0 must be (B,%d), got %s" % (field.D, tuple(xc.shape)))
     B, Tg = xc.shape[0], t.shape[0]
     t64 = t.detach().to(device=xc.device, dtype=torch.float64).contiguous()
     xs = torch.empty(Tg, B, field.D, dtype=torch.float32, device=xc.device)
-    work = torch.empty(lib.gpode_dopri5_large_work_floats(field.D, B), dtype=torch.float32, device=xc.device)
+    work = torch.empty(_lib.load().gpode_dopri5_large_work_floats(field.D, B), dtype=torch.float32, device=xc.device)
     stats = torch.zeros(4, dtype=torch.int32, device=xc.device)
-    _lib.call("gpode_dopri5_fwd_large", ptr(field.packed), ctypes.byref(field.struct), ptr(xc), ptr(t64), Tg, B,
-              float(rtol), float(atol), ptr(xs), ptr(work), ptr(stats), int(max_attempts), stream_ptr())
+    return xc, t64, xs, work, stats
+
+
+def _dopri5_large_d(x0, t, Z, ell, var, nu, omega, phase, w, rtol, atol, max_attempts=100000):
+    """dopri5 for 8 < D <= 64 without gradients: torchdiffeq 0.2.0's controller (whole-batch RMS norm, float64 time,
+    Hairer initial step with order 4, safety 0.9 / growth <= 10 / shrink >= 0.2, quartic dense output) ON THE DEVICE --
+    ``gpode_dopri5_fwd_large``: one attempt = six evaluations on the tcgen05 vector-field kernels + element-wise stage /
+    error kernels + a one-CTA controller kernel, looped by a CUDA-graph WHILE node whose condition the controller sets.
+    The host enqueues one graph launch and reads nothing back (the reference synchronises once per attempt)."""
+    field = LargeField(Z, ell, var, nu, omega, phase, w)
+    xc, t64, xs, work, stats = _dopri5_large_setup(field, x0, t)
+    _lib.call("gpode_dopri5_fwd_large", ptr(field.packed), ctypes.byref(field.struct), ptr(xc), ptr(t64), t64.shape[0],
+              xc.shape[0], float(rtol), float(atol), ptr(xs), ptr(work), ptr(stats), int(max_attempts), stream_ptr())
     return xs, stats
+
+
+class _Dopri5Large(torch.autograd.Function):
+    """Differentiable dopri5 for 8 < D <= 64: ``gpode_dopri5_fwd_large_ckpt`` records the accepted steps (8 B D floats
+    each), ``gpode_dopri5_bwd_large`` runs their discrete adjoint on the large-D VJP kernels. One host read of the stats
+    per integration: the checkpoint capacity doubles until it holds every accepted step."""
+
+    @staticmethod
+    def forward(ctx, x0, t, Z, ell, var, nu, omega, phase, w, rtol, atol, max_attempts):
+        lib = _lib.load()
+        field = LargeField(Z, ell, var, nu, omega, phase, w)
+        xc, t64, xs, work, stats = _dopri5_large_setup(field, x0, t)
+        B, D, Tg = xc.shape[0], field.D, t64.shape[0]
+        cap = max(32, 4 * Tg)
+        while True:
+            ckpt = torch.empty(lib.gpode_dopri5_ckpt_floats(D, B, Tg, cap), dtype=torch.float32, device=xc.device)
+            _lib.call("gpode_dopri5_fwd_large_ckpt", ptr(field.packed), ctypes.byref(field.struct), ptr(xc), ptr(t64),
+                      Tg, B, float(rtol), float(atol), ptr(xs), ptr(work), ptr(stats), int(max_attempts), ptr(ckpt), cap,
+                      stream_ptr())
+            st = [int(v) for v in stats.cpu()]
+            if st[3] == 3:
+                cap *= 2
+                continue
+            if st[3] != 0:
+                raise _lib.GpodeError("dopri5 failed: status %d (1 = attempt limit, 2 = step-size underflow)" % st[3])
+            break
+        ctx.field, ctx.nu_shape, ctx.cap, ctx.n_acc = field, nu.shape, cap, st[1]
+        ctx.save_for_backward(t64, ckpt)
+        ctx.mark_non_differentiable(stats)
+        return xs, stats
+
+    @staticmethod
+    def backward(ctx, gxs, _gstats):
+        field = ctx.field
+        t64, ckpt = ctx.saved_tensors
+        gxs = f32(gxs, "grad_xs")
+        Tg, B, D = gxs.shape
+        gx0 = torch.empty(B, D, dtype=torch.float32, device=gxs.device)
+        acc = field.new_acc()
+        work = torch.empty(11 * B * D, dtype=torch.float32, device=gxs.device)
+        _lib.call("gpode_dopri5_bwd_large", ptr(field.packed_bwd), ctypes.byref(field.struct), ptr(t64), Tg, B,
+                  ptr(gxs), ptr(ckpt), ctx.cap, ctx.n_acc, ptr(gx0), ptr(acc), ptr(work), stream_ptr())
+        _lib.LAUNCH_COUNT["gpode_dopri5_bwd_large"] += 19 * max(ctx.n_acc - 1, 0)   # counted for one step: the others
+        g_Z, g_ell, g_var, g_nu = field.finalize(acc, B)
+        return gx0, None, g_Z, g_ell, g_var, g_nu.reshape(ctx.nu_shape), None, None, None, None, None, None
 
 
 def dopri5_integrate(x0, t, Z, ell, var, nu, omega, phase, w, rtol=1e-6, atol=1e-6):
     """Adaptive dopri5 with torchdiffeq 0.2.0's controller in one cooperative kernel. Returns ``(xs (len(t),B,D),
     stats)`` with ``stats`` a device int32 tensor [nfe, accepted, rejected, status]. Differentiable in x0, Z, ell,
     var, nu through the discrete adjoint of the accepted steps (step sizes are constants, as in torchdiffeq).
-    For 8 < D <= 64 (forward only) the same controller runs on the device inside a CUDA-graph while loop."""
+    For 8 < D <= 64 the same controller runs on the device inside a CUDA-graph while loop; without gradients that path
+    never synchronises with the host, with gradients it reads the stats once per integration."""
     if Z.shape[1] > MAX_D_REGISTER:
+        if torch.is_grad_enabled() and any(a.requires_grad for a in (x0, Z, ell, var, nu)):
+            return _Dopri5Large.apply(x0, t, Z, ell, var, nu, omega, phase, w, rtol, atol, 100000)
         return _dopri5_large_d(x0, t, Z, ell, var, nu, omega, phase, w, rtol, atol)
     return _Dopri5.apply(x0, t, Z, ell, var, nu, omega, phase, w, rtol, atol, torch.is_grad_enabled())
 

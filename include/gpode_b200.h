@@ -261,17 +261,32 @@ int gpode_rk4_bwd_large(const float* packed_bwd, const gpode_cache_t* cache, con
                         const float* xs, const float* kstages, const float* grad_xs, float* grad_x0, float* acc_large,
                         float* work, void* stream);
 
-/* Adaptive dopri5 for 8 < D <= GPODE_MAX_D_LARGE, forward only, controller on the device: torchdiffeq 0.2.0's
+/* Adaptive dopri5 for 8 < D <= GPODE_MAX_D_LARGE, controller on the device: torchdiffeq 0.2.0's
  * odeint(method='dopri5') as called from Flow.forward (src/core/flow.py:84-90). One attempt (six tcgen05 vector-field
  * evaluations, stage / error kernels, a one-CTA controller kernel, an accept kernel) is the body of a CUDA-graph WHILE
  * node; the controller sets the loop condition, so the host enqueues one graph launch and never synchronises (the
  * reference does once per attempt). t: float64 device grid (increasing or decreasing); xs [Tg,B,D]; stats_out (device,
- * 4 int32): nfe, accepted, rejected, status (0 ok, 1 attempt limit, 2 dt underflow); work:
- * gpode_dopri5_large_work_floats(D,B) floats. Cannot be called inside a stream capture (it builds its own graph). */
+ * 4 int32): nfe, accepted, rejected, status (0 ok, 1 attempt limit, 2 dt underflow, 3 checkpoint capacity); work:
+ * gpode_dopri5_large_work_floats(D,B) floats. Cannot be called inside a stream capture (it builds its own graph).
+ *   gpode_dopri5_fwd_large_ckpt: the same solve (bitwise the same xs and stats when it succeeds) that also records the
+ *     accepted steps in ckpt, gpode_dopri5_ckpt_floats(D,B,Tg,cap) floats (layout at that function; k holds the RAW
+ *     vector-field values here): 8 B D floats per accepted step. status 3 = more than `cap` accepted steps (retry with
+ *     a larger cap).
+ *   gpode_dopri5_bwd_large: the discrete adjoint of those steps (step sizes are constants, as in torchdiffeq; the two
+ *     initial-step evaluations get no cotangent): grad_xs [Tg,B,D] -> grad_x0 [B,D], six gpode_vf_bwd_large launches
+ *     per accepted step plus one at x0, all adding into acc_large (zeroed by the caller; follow with
+ *     gpode_grads_finalize_large). n_accepted = stats_out[1] of the forward; work: 11 B D floats. Bitwise
+ *     reproducible (no atomics). */
 int64_t gpode_dopri5_large_work_floats(int D, int64_t B);
 int gpode_dopri5_fwd_large(const float* packed_large, const gpode_cache_t* cache, const float* x0, const double* t, int Tg,
                            int64_t B, double rtol, double atol, float* xs, float* work, int32_t* stats_out,
                            int max_attempts, void* stream);
+int gpode_dopri5_fwd_large_ckpt(const float* packed_large, const gpode_cache_t* cache, const float* x0, const double* t,
+                                int Tg, int64_t B, double rtol, double atol, float* xs, float* work, int32_t* stats_out,
+                                int max_attempts, float* ckpt, int cap, void* stream);
+int gpode_dopri5_bwd_large(const float* packed_bwd, const gpode_cache_t* cache, const double* t, int Tg, int64_t B,
+                           const float* grad_xs, const float* ckpt, int cap, int n_accepted, float* grad_x0,
+                           float* acc_large, float* work, void* stream);
 
 /* Fused multiple-shooting ELBO step (SURVEY.md section 8f item 2). Every row (s, n, t) of the (S_mc, N, T) batch of
  * sampled states `ss` is integrated over ONE interval t2[0] -> t2[1] with the 3/8-rule RK4 step (as gpode_rk4_fwd with

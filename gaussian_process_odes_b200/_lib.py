@@ -53,8 +53,6 @@ SIGNATURES = {
     "gpode_inducing_sample_fwd": (_I, [_P, _P, _P, _I, _I, _P, _P]),
     "gpode_inducing_sample_bwd": (_I, [_P, _P, _I, _I, _P, _P]),
     "gpode_dopri5_work_floats": (_L, [_I, _L]),
-    "gpode_vf_fwd_large": (_I, [_CP, _P, _P, _L, _P]),
-    "gpode_rk4_fwd_large": (_I, [_CP, _P, _P, _I, _L, _P, _P]),
     "gpode_state_fwd": (_I, [_P, _P, _P, _I, _L, _I, _F, _P, _P, _P]),
     "gpode_state_bwd": (_I, [_P, _P, _I, _L, _I, _F, _P, _P, _P, _P, _P]),
     "gpode_loglik_sum": (_I, [_P, _P, _P, _P, _P, _I, _L, _I, _I, _P, _P, _P, _P, _P]),
@@ -63,9 +61,6 @@ SIGNATURES = {
     "gpode_set_option": (_I, [ctypes.c_char_p, _I]),
     "gpode_get_option": (_I, [ctypes.c_char_p]),
     "gpode_shoot_work_doubles": (_L, []),
-    "gpode_packed_ubwd_floats": (_L, [_I, _I]),
-    "gpode_pack_cache_ubwd": (_I, [_CP, _P, _P]),
-    "gpode_vf_bwd_umma": (_I, [_P, _P, _I, _I, _I, _P, _P, _P, _P, _P, _L, _P]),
     "gpode_packed_large_bwd_floats": (_L, [_I, _I, _I]),
     "gpode_acc_large_floats": (_L, [_I, _I]),
     "gpode_pack_cache_large_bwd": (_I, [_CP, _P, _P]),
@@ -91,7 +86,6 @@ SIGNATURES = {
     "gpode_pack_cache_large": (_I, [_CP, _P, _P]),
     "gpode_rff_fwd_large": (_I, [_P, _I, _I, _P, _P, _L, _P]),
     "gpode_vf_fwd_large_add_rbf": (_I, [_CP, _P, _P, _P, _L, _P]),
-    "gpode_vf_fwd_umma": (_I, [_P, _I, _I, _I, _P, _P, _L, _P]),
     "gpode_pack_cache_sets": (_I, [_CP, _I, _P, _P]),
     "gpode_whiten_fwd_sets": (_I, [_CP, _P, _F, _I, _P, _P, _P, _P]),
     "gpode_vf_fwd_sets": (_I, [_P, _I, _I, _I, _I, _L, _P, _P, _P]),
@@ -119,14 +113,14 @@ def load():
     for name, (res, args) in SIGNATURES.items():
         fn = getattr(lib, name)  # AttributeError here = header/library mismatch, fail loudly
         fn.restype, fn.argtypes = res, args
-    if lib.gpode_abi_version() != 1:
-        raise GpodeError("libgpode_b200.so ABI version %d, expected 1" % lib.gpode_abi_version())
+    if lib.gpode_abi_version() != 2:
+        raise GpodeError("libgpode_b200.so ABI version %d, expected 2" % lib.gpode_abi_version())
     _lib = lib
     return lib
 
 
 def set_option(name, value):
-    """Process-wide kernel-selection option (``gpode_set_option``): bwd_mma, fwd_mma, mma_parts, force_narrow, use_mma."""
+    """Process-wide kernel-selection option (``gpode_set_option``): bwd_mma, fwd_mma."""
     check(load().gpode_set_option(name.encode(), int(value)))
 
 
@@ -170,12 +164,11 @@ KERNELS_PER_CALL = {
     "gpode_pack_cache": 1, "gpode_vf_fwd": 1, "gpode_vf_bwd": 1, "gpode_rk4_fwd": 1, "gpode_rk4_bwd": 1,
     "gpode_param_grad": 1, "gpode_grads_finalize": 1, "gpode_whiten_fwd": 1, "gpode_whiten_bwd": 1,
     "gpode_kl_fwd": 1, "gpode_kl_bwd": 1, "gpode_inducing_sample_fwd": 1, "gpode_inducing_sample_bwd": 1, "gpode_dopri5_fwd": 1, "gpode_dopri5_bwd": 1, "gpode_state_fwd": 1,
-    "gpode_state_bwd": 1, "gpode_loglik_sum": 2, "gpode_constraint_sum": 2, "gpode_vf_fwd_large": 1,
-    "gpode_rk4_fwd_large": 1, "gpode_pack_cache_large": 1, "gpode_rbf_fwd_large": 1, "gpode_rff_fwd_large": 1,
-    "gpode_vf_fwd_large_add_rbf": 1, "gpode_dopri5_bwd_dev": 1, "gpode_param_grad_dev": 1, "gpode_vf_fwd_umma": 1,
+    "gpode_state_bwd": 1, "gpode_loglik_sum": 2, "gpode_constraint_sum": 2,
+    "gpode_pack_cache_large": 1, "gpode_rbf_fwd_large": 1, "gpode_rff_fwd_large": 1,
+    "gpode_vf_fwd_large_add_rbf": 1, "gpode_dopri5_bwd_dev": 1, "gpode_param_grad_dev": 1,
     "gpode_pack_cache_sets": 1, "gpode_whiten_fwd_sets": 2, "gpode_vf_fwd_sets": 1, "gpode_rk4_fwd_sets": 1,
     "gpode_dopri5_fwd_sets": 1, "gpode_shoot_fwd": 2, "gpode_shoot_bwd": 1,
-    "gpode_pack_cache_ubwd": 1, "gpode_vf_bwd_umma": 1,
     "gpode_pack_cache_large_bwd": 2, "gpode_vf_bwd_large": 2, "gpode_grads_finalize_large": 2,
     # per RK4 step: forward 4 evaluations x 2 kernels + 4 stage kernels; adjoint 4 VJPs + 8 element-wise kernels
     "gpode_rk4_fwd_large_dev": 12, "gpode_rk4_bwd_large": 16,

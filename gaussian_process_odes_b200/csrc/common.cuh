@@ -41,10 +41,9 @@ void gpode_set_error(const char* fmt, ...);
 // ------------------------------------------------------------------------------------------------------------------
 // process-wide kernel-selection options (gpode_set_option / gpode_get_option, include/gpode_b200.h): the library's only
 // mutable global state. Defaults come from the environment ONCE, when the first option is read (GPODE_BWD_MMA,
-// GPODE_FWD_MMA, GPODE_MMA_PARTS, GPODE_FORCE_NARROW, GPODE_USE_MMA, GPODE_LARGE_BWD_UMMA); after that only gpode_set_option changes them.
+// GPODE_FWD_MMA); after that only gpode_set_option changes them.
 // ------------------------------------------------------------------------------------------------------------------
-enum { GPODE_OPT_BWD_MMA = 0, GPODE_OPT_FWD_MMA, GPODE_OPT_MMA_PARTS, GPODE_OPT_FORCE_NARROW, GPODE_OPT_USE_MMA,
-       GPODE_OPT_LARGE_BWD_UMMA, GPODE_OPT_COUNT };
+enum { GPODE_OPT_BWD_MMA = 0, GPODE_OPT_FWD_MMA, GPODE_OPT_COUNT };
 int gpode_option(int which);  // pack.cu
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -65,27 +64,19 @@ int gpode_option(int which);  // pack.cu
 struct GpodeLayout {
     int D, M, S, S2, S2P, RP, KS, WP;
     int off_rff, off_kern, off_il, total;  // in floats; every offset and `total` is a multiple of 4 (16 bytes)
-    // tensor-core (mma.sync m16n8k8 tf32) operand blocks, appended after `total`, one record per (output k, tile of
-    // 8 features):  mma  : 80 floats = 64 theta-B fragment (lane-major b0,b1) | 16 (phase, phase', a, a') per quad lane
-    //               mmah : operands for mma.sync m16n8k16 f16 (vjp_mma.cuh: adjoint and forward), 152 words per (output k,
-    //                      tile of 8 features; tiles padded to an even count S8P with zero records):
-    //                        [0,64)    theta-B, lane-major (b0,b1) half2 pairs: contraction slots 0..D-1 = Omega_hi,
-    //                                  D..2D-1 = Omega_lo, 2D..3D-1 = Omega_hi (the state tile carries x_hi, x_hi, x_lo)
-    //                        [64,80)   per quad lane t: phase(2t), phase(2t+1), phase(2t), phase(2t+1)  (fp32, the MMA's C)
-    //                        [80,144)  G-B of the tile PAIR (2i, 2i+1), lane-major (b0,b1): the even record holds the hi
-    //                                  parts (tile 2i, tile 2i+1), the odd record the lo parts; one half2 =
-    //                                  (Bp[2t][g], Bp[2t+1][g]), Bp[s][j] = GPODE_MMAH_SCALE a_s Omega_{j,s,k}
-    //                        [144,152) a_s of the tile's 8 features (fp32; the forward's cosine weights)
-    int S8, off_mma, off_mmag, S8P;
-    // tcgen05 (UMMA) operand block, one record of GPODE_UMMA_REC(SU) floats per output k:
-    //   B_hi [SU x 8] | B_lo [SU x 8] | a [SU]   (SU = S rounded up to 32)   -- B = (Omega_k | phase | 0)^T, features x padded input dims, in
-    //   the canonical K-major no-swizzle shared-memory layout of the MMA (8-feature x 16-byte core matrices: feature s,
-    //   slot q at float (s/8) 64 + (q/4) 32 + (s%8) 4 + q%4), pre-split into tf32 hi / lo parts; slot D carries the
-    //   phase (the state tile carries a constant 1 there), so theta leaves the tensor core complete. D <= 7 only.
-    int SU, off_umma, total_all;
+    // tensor-core operand block, appended at `total` for D <= GPODE_MMAH_MAX_D:
+    //  mmah : operands for mma.sync m16n8k16 f16 (vjp_mma.cuh: adjoint and forward), 152 words per (output k,
+    //         tile of 8 features; tiles padded to an even count S8P with zero records):
+    //           [0,64)    theta-B, lane-major (b0,b1) half2 pairs: contraction slots 0..D-1 = Omega_hi,
+    //                     D..2D-1 = Omega_lo, 2D..3D-1 = Omega_hi (the state tile carries x_hi, x_hi, x_lo)
+    //           [64,80)   per quad lane t: phase(2t), phase(2t+1), phase(2t), phase(2t+1)  (fp32, the MMA's C)
+    //           [80,144)  G-B of the tile PAIR (2i, 2i+1), lane-major (b0,b1): the even record holds the hi
+    //                     parts (tile 2i, tile 2i+1), the odd record the lo parts; one half2 =
+    //                     (Bp[2t][g], Bp[2t+1][g]), Bp[s][j] = GPODE_MMAH_SCALE a_s Omega_{j,s,k}
+    //           [144,152) a_s of the tile's 8 features (fp32; the forward's cosine weights)
+    int S8P, off_mmah;
+    int n_packed;  // floats of the whole packed block (gpode_packed_floats)
 };
-#define GPODE_UMMA_REC(SU) (17 * (SU))
-#define GPODE_MMA_REC 80
 #define GPODE_MMAH_REC 152
 #define GPODE_MMAH_MAX_D 5  // 3 D contraction slots (x_hi, x_hi, x_lo) must fit the 16 of one m16n8k16
 #define GPODE_MMAH_SCALE 256.f  // keeps the fp16 low parts of a Omega out of the subnormal range
@@ -104,13 +95,9 @@ __host__ __device__ inline GpodeLayout gpode_layout(int D, int M, int S) {
     L.off_kern = L.off_rff + D * L.S2P * L.RP;
     L.off_il = L.off_kern + M * L.KS;
     L.total = L.off_il + D * L.WP;
-    L.S8 = (S + 7) / 8;
-    L.off_mma = L.total;
-    L.off_mmag = L.off_mma + D * L.S8 * GPODE_MMA_REC;
-    L.SU = (S + 31) & ~31;  // features padded to whole 32-column TMEM loads (zero weight)
-    L.S8P = (L.S8 + 1) & ~1;
-    L.off_umma = L.off_mmag + (D <= GPODE_MMAH_MAX_D ? D * L.S8P * GPODE_MMAH_REC : 0);
-    L.total_all = L.off_umma + (D <= 7 ? D * GPODE_UMMA_REC(L.SU) : 0);
+    L.S8P = ((S + 7) / 8 + 1) & ~1;
+    L.off_mmah = L.total;
+    L.n_packed = L.off_mmah + (D <= GPODE_MMAH_MAX_D ? D * L.S8P * GPODE_MMAH_REC : 0);
     return L;
 }
 
@@ -229,13 +216,6 @@ __device__ __forceinline__ float2 fadd2(float2 a, float2 b) {
     return gpode_unpack2(d);
 }
 
-// ---- legacy tensor-core path: mma.sync m16n8k8, tf32 operands, fp32 accumulate (SASS HMMA.1688.F32.TF32) ----------
-// tf32 operands are passed as raw fp32 bit patterns: the tensor core ignores the 13 low mantissa bits, so
-// hi = v & 0xffffe000 is exactly what it sees and lo = v - hi is exact in fp32 (error-compensated "3xTF32" split).
-__device__ __forceinline__ void gpode_split_tf32(float v, uint32_t& hi, uint32_t& lo) {
-    hi = __float_as_uint(v) & 0xffffe000u;
-    lo = __float_as_uint(v - __uint_as_float(hi));
-}
 // 3xTF32 split for the tcgen05 path, round-to-nearest: hi = tf32(v), lo = tf32(v - hi). Both parts have their 13 low
 // mantissa bits clear, so the tensor core (which truncates) sees them exactly; the residual v - hi - lo is <= 2^-24 |v|
 // and unbiased (a truncating split leaves a one-sided 2^-22 |v|, visible at D = 64 where 65 products add up).
@@ -245,13 +225,6 @@ __device__ __forceinline__ float gpode_round_tf32(float v) {
 __device__ __forceinline__ void gpode_split_tf32_rn(float v, float& hi, float& lo) {
     hi = gpode_round_tf32(v);
     lo = gpode_round_tf32(v - hi);
-}
-
-__device__ __forceinline__ void gpode_mma_tf32(float (&d)[4], const uint32_t (&a)[4], const uint32_t b0,
-                                               const uint32_t b1) {
-    asm("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-        : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-        : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
 }
 
 __device__ __forceinline__ uint32_t gpode_smem_u32(const void* p) {

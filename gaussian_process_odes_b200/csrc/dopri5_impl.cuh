@@ -442,7 +442,7 @@ int launch_dopri5_sets(const float* packed, int M, int S, int n_sets, int64_t se
     a.red = nullptr;
     a.stats = stats;
     a.set_rows = set_rows;
-    a.set_stride = L.total_all;
+    a.set_stride = L.n_packed;
     a.max_attempts = 1 << 20;
     dopri5_set_ckpt(a, n_sets == 1 ? ckpt : nullptr, cap, a.B * D, Tg);  // checkpoints: single-set (training) use only
     int warps = (int)(set_rows < kDpSetThreads / 32 ? set_rows : kDpSetThreads / 32);

@@ -10,7 +10,6 @@
 // [time][row][dim] layout torchdiffeq itself returns.
 #pragma once
 #include <stdlib.h>
-#include "vf_mma.cuh"
 #include "vjp_mma.cuh"
 #include "shoot.cuh"
 
@@ -596,50 +595,6 @@ vf_bwd_warp_kernel(const float* __restrict__ packed, const int M, const int S, c
     reduce_AV64<D>(wa, acc, slabs + kWarpsPerCta * WarpAcc64<D>::kSlabDoubles);
 }
 
-// ------------------------------------------------------------------------------------------------------------------
-// Tensor-core (quad layout) kernels: a warp owns 32 rows, see vf_mma.cuh
-// ------------------------------------------------------------------------------------------------------------------
-template <int D>
-__device__ __forceinline__ void load_rows_quad(float (&v)[4][D], const float* __restrict__ base, const int64_t row0,
-                                               const int64_t B) {
-#pragma unroll
-    for (int r = 0; r < 4; ++r) {
-        const int64_t row = row0 + 8 * r;
-#pragma unroll
-        for (int j = 0; j < D; ++j) v[r][j] = row < B ? __ldg(base + row * D + j) : 0.f;
-    }
-}
-// the four lanes of a quad hold identical values: lane t writes row slot t
-template <int D>
-__device__ __forceinline__ void store_rows_quad(const float (&v)[4][D], float* __restrict__ base, const int64_t row0,
-                                                const int64_t B, const int t) {
-#pragma unroll
-    for (int r = 0; r < 4; ++r) {
-        const int64_t row = row0 + 8 * r;
-        if (r == t && row < B) {
-#pragma unroll
-            for (int j = 0; j < D; ++j) base[row * D + j] = v[r][j];
-        }
-    }
-}
-
-template <int D>
-__global__ void __launch_bounds__(kThreads, 4)
-vf_fwd_mma_kernel(const float* __restrict__ packed, const int M, const int S, const int off_kern, const int total_all,
-                  const float* __restrict__ x, float* __restrict__ f, const int64_t B) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    const float* sp = stage_params_mma(smem_raw, packed, off_kern, total_all);
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, wpc = blockDim.x >> 5;
-    const int64_t nblocks = (B + 31) / 32;
-    for (int64_t blk = (int64_t)blockIdx.x * wpc + warp; blk < nblocks; blk += (int64_t)gridDim.x * wpc) {
-        const int64_t row0 = blk * 32 + (lane >> 2);
-        float xr[4][D], fr[4][D];
-        load_rows_quad<D>(xr, x, row0, B);
-        vf_eval_mma<D>(sp, M, S, xr, fr, lane);
-        store_rows_quad<D>(fr, f, row0, B, lane & 3);
-    }
-}
-
 // ---- tensor-core adjoint kernels (vjp_mma.cuh) -------------------------------------------------------------------
 // One CTA of kHWarps warps per SM (the f16 operand records take ~92 KB at D = 5, S = 256, so they are staged once per
 // SM); a warp owns 32 rows, lane = row.
@@ -652,8 +607,6 @@ constexpr int kHThreads = kHWarps * 32;
 
 struct HParams {
     int M, S8P, off_kern, n_small, off_mmah, n_mmah;
-    int parts;  // tuning (GPODE_MMA_PARTS): bit 0 = RFF part, bit 1 = RBF part of the adjoint; bits 2-3 = schedule of the
-                // forward evaluation (0 fused stream, 1 two parts, 2 two parts staggered across warps); default 3
 };
 
 template <int D>
@@ -698,7 +651,7 @@ vf_bwd_mma_kernel(const float* __restrict__ packed, const HParams p, const float
         load_rows<D, 1>(xr, x, row, B, 0);
         load_rows<D, 1>(fr, f, row, B, 0);
         load_rows<D, 1>(kb, gf, row, B, 0);
-        vf_vjp_h<D>(sm.small, sm.mmah, sm.stage, p.M, p.S8P, xr, kb, fr, xb, qa, lane, p.parts);
+        vf_vjp_h<D>(sm.small, sm.mmah, sm.stage, p.M, p.S8P, xr, kb, fr, xb, qa, lane);
         store_rows<D, 1>(xb, gx, row, B, 0);
     }
     hacc_reduce<D>(qa, sm.small, p.M, acc, sm.red);
@@ -720,7 +673,7 @@ vf_fwd_h_kernel(const float* __restrict__ packed, const HParams p, const float* 
         const int64_t row = blk * 32 + lane;
         float xr[1][D], fr[1][D];
         load_rows<D, 1>(xr, x, row, B, 0);
-        vf_eval_h<D>(sm.small, sm.mmah, sm.stage, p.M, p.S8P, xr, fr, lane, (p.parts >> 2) & 3);
+        vf_eval_h<D>(sm.small, sm.mmah, sm.stage, p.M, p.S8P, xr, fr, lane);
         store_rows<D, 1>(fr, f, row, B, 0);
     }
 }
@@ -756,7 +709,7 @@ rk4_fwd_h_kernel(const float* __restrict__ packed, const HParams p, const float*
             }
 #pragma unroll 1
             for (int st = 1; st <= 4; ++st) {
-                vf_eval_h<D>(sm.small, sm.mmah, sm.stage, p.M, p.S8P, ys, kk, lane, (p.parts >> 2) & 3);
+                vf_eval_h<D>(sm.small, sm.mmah, sm.stage, p.M, p.S8P, ys, kk, lane);
                 if (kst != nullptr) store_rows<D, R>(kk, kst + ((int64_t)i * 4 + (st - 1)) * plane, row0, B, 0);
                 if (st == 1) {
 #pragma unroll
@@ -876,7 +829,7 @@ rk4_bwd_mma_kernel(const float* __restrict__ packed, const HParams p, const floa
                 }
                 store_rows<D, R>(ys, vyi + (int64_t)(st - 1) * plane, row0, B, 0);
                 store_rows<D, R>(kbar, vki + (int64_t)(st - 1) * plane, row0, B, 0);
-                vf_vjp_h<D>(sm.small, sm.mmah, sm.stage, p.M, p.S8P, ys, kbar, ks, yb, qa, lane, p.parts);
+                vf_vjp_h<D>(sm.small, sm.mmah, sm.stage, p.M, p.S8P, ys, kbar, ks, yb, qa, lane);
                 float lam[R][D];
                 get(F_LAM, lam);
                 if (st == 4) {
@@ -997,8 +950,7 @@ inline int warp_shape_for(K kernel, int64_t B, size_t smem, LaunchShape* out) {
 
 template <int D, int R>
 inline bool use_wide(int64_t B) {
-    const bool force_narrow = gpode_option(GPODE_OPT_FORCE_NARROW) != 0;  // tuning knob: one row per thread
-    return !force_narrow && R > 1 && B >= (int64_t)num_sms() * 2 * kThreads * R;
+    return R > 1 && B >= (int64_t)num_sms() * 2 * kThreads * R;
 }
 
 
@@ -1019,8 +971,7 @@ inline HParams h_params(const GpodeLayout& L) {
     HParams p;
     p.M = L.M; p.S8P = L.S8P;
     p.off_kern = L.off_kern; p.n_small = L.total - L.off_kern;
-    p.off_mmah = L.off_mmag; p.n_mmah = D * L.S8P * GPODE_MMAH_REC;
-    p.parts = gpode_option(GPODE_OPT_MMA_PARTS);
+    p.off_mmah = L.off_mmah; p.n_mmah = D * L.S8P * GPODE_MMAH_REC;
     return p;
 }
 template <int D>
@@ -1046,11 +997,10 @@ int launch_vf_fwd(const float* packed, int M, int S, const float* x, float* f, i
     const size_t smem = 16 + (size_t)L.total * 4;
     LaunchShape ls;
     constexpr int RW = RowsFwd<D>::value;
-    const bool use_mma = gpode_option(GPODE_OPT_USE_MMA) != 0;
     if constexpr (kMmaBwd<D>) {
         const HParams hp = h_params<D>(L);
         const size_t hs = h_smem<D>(hp, false, kHFWarps);
-        if (!use_mma && use_mma_fwd(B) && hs <= 227 * 1024) {
+        if (use_mma_fwd(B) && hs <= 227 * 1024) {
             int grid = 0;
             if (int rc = h_grid(vf_fwd_h_kernel<D>, B, hs, &grid, kHFThreads)) return rc;
             vf_fwd_h_kernel<D><<<grid, kHFThreads, hs, st>>>(packed, hp, x, f, B);
@@ -1058,19 +1008,7 @@ int launch_vf_fwd(const float* packed, int M, int S, const float* x, float* f, i
             return 0;
         }
     }
-    if (use_mma && B > kWarpPathMaxRows) {
-        const size_t smem_mma = 16 + (size_t)(L.off_mmag - L.off_kern) * 4;  // forward: no G fragments
-        GPODE_CUDA(cudaFuncSetAttribute(vf_fwd_mma_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_mma));
-        int occ = 0;
-        GPODE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, vf_fwd_mma_kernel<D>, kThreads, smem_mma));
-        if (occ < 1) {
-            gpode_set_error("mma kernel does not fit on an SM (smem %zu bytes)", smem_mma);
-            return -2;
-        }
-        const int64_t want = (B + 127) / 128, cap = (int64_t)num_sms() * occ;
-        vf_fwd_mma_kernel<D><<<(unsigned)(want < cap ? want : cap), kThreads, smem_mma, st>>>(
-            packed, M, S, L.off_kern, L.off_mmag, x, f, B);
-    } else if (B <= kWarpPathMaxRows) {
+    if (B <= kWarpPathMaxRows) {
         if (int rc = warp_shape_for(vf_fwd_warp_kernel<D>, B, smem, &ls)) return rc;
         vf_fwd_warp_kernel<D><<<ls.grid, ls.threads, ls.smem, st>>>(packed, M, S, L.total, x, f, B);
     } else if (use_wide<D, RW>(B)) {
@@ -1139,10 +1077,10 @@ int launch_fwd_sets(const float* packed, int M, int S, int n_sets, int64_t set_r
     const dim3 grid((unsigned)want, (unsigned)n_sets);
     if (t == nullptr) {
         GPODE_CUDA(cudaFuncSetAttribute(vf_fwd_sets_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        vf_fwd_sets_kernel<D><<<grid, threads, smem, st>>>(packed, M, S, L.total, L.total_all, set_rows, x0, out);
+        vf_fwd_sets_kernel<D><<<grid, threads, smem, st>>>(packed, M, S, L.total, L.n_packed, set_rows, x0, out);
     } else {
         GPODE_CUDA(cudaFuncSetAttribute(rk4_fwd_sets_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        rk4_fwd_sets_kernel<D><<<grid, threads, smem, st>>>(packed, M, S, L.total, L.total_all, set_rows, x0, t, Tg,
+        rk4_fwd_sets_kernel<D><<<grid, threads, smem, st>>>(packed, M, S, L.total, L.n_packed, set_rows, x0, t, Tg,
                                                             out);
     }
     GPODE_LAUNCH_CHECK();

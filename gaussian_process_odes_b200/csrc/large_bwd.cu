@@ -10,11 +10,9 @@
 //     for the stage algebra; step sizes are read from the device-side grid, nothing returns to the host;
 //   * gpode_grads_finalize_large: per-CTA partial rows -> parameter gradients in float64, fixed order (no atomics).
 //
+// The RFF part of the VJP runs first, on the tcgen05 tensor cores (large_rffb.cu): it writes its share of the row
+// cotangent to gx and its lengthscale partial sums to accumulator rows of its own. The kernels here add the RBF part.
 // VJP mapping (FP32 CUDA cores). CTA = 128 threads = one tile of 128 rows, THREAD = ROW for everything that is per row:
-//   RFF part, per output k: theta_s = phase_sk + sum_j x_j Omega_jsk, g_s = a_sk sin(theta_s), G_j = sum_s g_s Omega_jsk
-//     with x, G in registers and the (k, 64-feature) chunk of Omega -- 16 KB, j contiguous -- staged in shared memory by
-//     the bulk-copy engine (cp.async.bulk + mbarrier, double-buffered one chunk ahead) and read by broadcast LDS.128:
-//     4 features per trip = 4 independent FMA chains;  xb_j -= kb_k G_j;  A[k][j] -= sum_rows kb_k x_j G_j.
 //   RBF part, per inducing point m (CTA-uniform loop): dd_j = (x_j - Z_mj)^2 in registers; per k: e = sum_j dd_j w_kj,
 //     K = 2^-e, p = kb_k K, t_j += 2 ln2 c_km p w_kj;  xb_j -= d_j t_j.
 //   The sums over ROWS -- T[k][m] = sum_r p, A2[k][j] = sum_r p dd_j, Zb[m][j] = sum_r d_j t_j -- are taken by
@@ -28,7 +26,6 @@ int gpode_vf_large_eval(const float* packed_large, const gpode_cache_t* c, const
 // large_rffb.cu: the RFF part of the VJP on the tcgen05 tensor cores (both projections as 3xTF32 GEMMs)
 int64_t gpode_rv_packed_floats(int D, int S);
 int64_t gpode_rv_acc_floats(int D);
-bool gpode_rv_supported(int D);
 int gpode_rv_grid(int64_t B);
 int gpode_rv_dn(int D);
 int gpode_rv_pack(const gpode_cache_t* c, float* out, cudaStream_t st);
@@ -37,44 +34,29 @@ int gpode_rv_launch(const float* packed, int D, int S, const float* x, const flo
 
 namespace {
 
-constexpr int kLbRows = 128, kLbThreads = 128, kLbSC = 64;  // tile rows, threads, features per staged Omega chunk
+constexpr int kLbRows = 128, kLbThreads = 128;  // tile rows, threads
 constexpr int kLbMaxCtas = 148 * 4;
 
 __host__ __device__ inline int lb_dp(int D) { return D <= 16 ? 16 : (D <= 32 ? 32 : 64); }
 
 struct LbLayout {
-    int D, DP, M, S, SU, NCH;
-    int64_t off_om, off_ph, off_aw, off_w, off_z, off_c, total;  // floats
+    int D, DP, M;
+    int64_t off_w, off_z, off_c, total;  // floats
 };
-__host__ __device__ inline LbLayout lb_layout(int D, int M, int S) {
+__host__ __device__ inline LbLayout lb_layout(int D, int M) {
     LbLayout L;
-    L.D = D; L.DP = lb_dp(D); L.M = M; L.S = S;
-    L.SU = (S + kLbSC - 1) / kLbSC * kLbSC;
-    L.NCH = L.SU / kLbSC;
-    L.off_om = 0;                                     // [k < D][chunk][feature in chunk][DP]  Omega_jsk, j contiguous
-    L.off_ph = L.off_om + (int64_t)D * L.SU * L.DP;   // [k][SU] phase
-    L.off_aw = L.off_ph + (int64_t)D * L.SU;          // [k][SU] a_sk = w_sk sqrt(var_k / S)  (0 for padded features)
-    L.off_w = L.off_aw + (int64_t)D * L.SU;           // [DP][DP] w_kj = 0.5 log2(e) / ell_kj^2
+    L.D = D; L.DP = lb_dp(D); L.M = M;
+    L.off_w = 0;                                      // [DP][DP] w_kj = 0.5 log2(e) / ell_kj^2
     L.off_z = L.off_w + (int64_t)L.DP * L.DP;         // [M][DP] Z
     L.off_c = L.off_z + (int64_t)M * L.DP;            // [M][DP] c_km = var_k nu_km, k contiguous
     L.total = L.off_c + (int64_t)M * L.DP;
     return L;
 }
 
-__global__ void pack_lb_kernel(const LbLayout L, const float* __restrict__ omega, const float* __restrict__ phase,
-                               const float* __restrict__ w, const float* __restrict__ Z, const float* __restrict__ nu,
+__global__ void pack_lb_kernel(const LbLayout L, const float* __restrict__ Z, const float* __restrict__ nu,
                                const float* __restrict__ ell, const float* __restrict__ var, float* __restrict__ out) {
-    const int D = L.D, DP = L.DP, S = L.S, SU = L.SU, M = L.M;
+    const int D = L.D, DP = L.DP, M = L.M;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x, i0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    for (int64_t i = i0; i < (int64_t)D * SU * DP; i += stride) {
-        const int j = (int)(i % DP), s = (int)((i / DP) % SU), k = (int)(i / ((int64_t)DP * SU));
-        out[L.off_om + i] = (s < S && j < D) ? omega[((size_t)j * S + s) * D + k] : 0.f;
-    }
-    for (int64_t i = i0; i < (int64_t)D * SU; i += stride) {
-        const int s = (int)(i % SU), k = (int)(i / SU);
-        out[L.off_ph + i] = s < S ? phase[s * D + k] : 0.f;
-        out[L.off_aw + i] = s < S ? w[s * D + k] * sqrtf(var[k] / (float)S) : 0.f;
-    }
     for (int64_t i = i0; i < (int64_t)DP * DP; i += stride) {
         const int j = (int)(i % DP), k = (int)(i / DP);
         float v = 0.f;
@@ -92,23 +74,22 @@ __global__ void pack_lb_kernel(const LbLayout L, const float* __restrict__ omega
 }
 
 // shared memory (floats): xs | kbs | stA | stB | xbs (each [128][DP + 4]; xbs = the running row cotangent: kept out of
-// the register file, which holds x / G resp. dd / t) | Ws [DP][DP] | As [DP][DP] | red [4][DP] | V1 [DP],
-// then two mbarriers. The two Omega chunk buffers (64 x DP floats each) alias stA and stB during the RFF part.
+// the register file, which holds dd / t) | Ws [DP][DP] | As [DP][DP] | red [4][DP] | V1 [DP]
 template <int DP>
 struct LbSmem {
     static constexpr int LD = DP + 4;
     static constexpr int tile = kLbRows * LD;
     static constexpr int floats = 5 * tile + 2 * DP * DP + 4 * DP + DP;
-    static constexpr size_t bytes = (size_t)floats * 4 + 16;
+    static constexpr size_t bytes = (size_t)floats * 4;
 };
 
+// RBF half of the VJP at DP = 16, 32 (DP = 64: rbf_vjp_large_kernel). gx holds the RFF half on entry (large_rffb.cu);
+// this kernel adds the RBF half to it and writes the RBF and variance partial sums.
 template <int DP>
-__global__ void __launch_bounds__(kLbThreads, DP >= 64 ? 1 : 2)
+__global__ void __launch_bounds__(kLbThreads, 2)
 vjp_large_kernel(const float* __restrict__ pk, const LbLayout L, const float* __restrict__ x,
                  const float* __restrict__ f, const float* __restrict__ kb, float* __restrict__ gx, const int64_t B,
-                 float* __restrict__ accA, float* __restrict__ accT, float* __restrict__ accZ, const int rff_done) {
-    // rff_done != 0: the tensor-core kernel of large_rffb.cu has already written the RFF part of the row cotangent to gx
-    // (and its lengthscale partial sums to its own rows): this kernel adds the RBF part and the variance sums.
+                 float* __restrict__ accA, float* __restrict__ accT, float* __restrict__ accZ) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     constexpr int LD = LbSmem<DP>::LD, TILE = LbSmem<DP>::tile;
     float* xs = reinterpret_cast<float*>(smem_raw);
@@ -120,28 +101,17 @@ vjp_large_kernel(const float* __restrict__ pk, const LbLayout L, const float* __
     float* As = Ws + DP * DP;
     float* red = As + DP * DP;
     float* V1 = red + 4 * DP;
-    uint64_t* mbar = reinterpret_cast<uint64_t*>(V1 + DP);
-    float* obuf[2] = {stA, stB};
-    const int D = L.D, M = L.M, SU = L.SU, NCH = L.NCH;
+    const int D = L.D, M = L.M;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const float* __restrict__ om_g = pk + L.off_om;
-    const float* __restrict__ ph_g = pk + L.off_ph;
-    const float* __restrict__ aw_g = pk + L.off_aw;
     const float* __restrict__ z_g = pk + L.off_z;
     const float* __restrict__ c_g = pk + L.off_c;
-    constexpr uint32_t kChunkBytes = kLbSC * DP * 4;
 
     for (int i = tid; i < DP * DP; i += kLbThreads) {
         Ws[i] = pk[L.off_w + i];
         As[i] = 0.f;
     }
     for (int i = tid; i < DP; i += kLbThreads) V1[i] = 0.f;
-    if (tid == 0) {
-        gpode_mbar_init(mbar, 1);
-        gpode_mbar_init(mbar + 1, 1);
-    }
     __syncthreads();
-    uint32_t it = 0;  // running count of staged chunks (buffer = it & 1, parity = (it >> 1) & 1)
     float* __restrict__ Tg = accT + (size_t)blockIdx.x * D * M;
     float* __restrict__ Zg = accZ + (size_t)blockIdx.x * M * DP;
 
@@ -156,27 +126,12 @@ vjp_large_kernel(const float* __restrict__ pk, const LbLayout L, const float* __
             xs[r * LD + j] = ok ? __ldg(x + (r0 + r) * D + j) : 0.f;
             kbs[r * LD + j] = ok ? __ldg(kb + (r0 + r) * D + j) : 0.f;
         }
-        // first Omega chunk of this tile; the generic-proxy writes of the previous tile's RBF part to stA / stB are
-        // ordered before the async-proxy copy by the barrier at the end of that tile + this fence
-        if (tid == 0 && !rff_done) {
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            gpode_bulk_g2s(obuf[it & 1], om_g, kChunkBytes, mbar + (it & 1));
-        }
         __syncthreads();
-        // At DP = 64 the state row stays in shared memory (one extra LDS.128 per four input dimensions): x, G and the
-        // four feature chains together exceed the register file (ptxas: 4 KB of spills, 140 ms per 1e5-row VJP).
-        constexpr bool kXReg = DP < 64;
-        float xr[kXReg ? DP : 4];
-        const float* __restrict__ xrow = xs + tid * LD;
         float* __restrict__ xbr = xbs + tid * LD;   // this row's cotangent (only its own thread touches it)
 #pragma unroll
         for (int j4 = 0; j4 < DP / 4; ++j4) {
-            if constexpr (kXReg) {
-                const float4 v = *reinterpret_cast<const float4*>(xrow + 4 * j4);
-                xr[4 * j4] = v.x; xr[4 * j4 + 1] = v.y; xr[4 * j4 + 2] = v.z; xr[4 * j4 + 3] = v.w;
-            }
             float4 init = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (rff_done && tid < n) {
+            if (tid < n) {
                 const float* __restrict__ gr = gx + (r0 + tid) * D;
                 init.x = 4 * j4 < D ? gr[4 * j4] : 0.f;
                 init.y = 4 * j4 + 1 < D ? gr[4 * j4 + 1] : 0.f;
@@ -194,87 +149,14 @@ vjp_large_kernel(const float* __restrict__ pk, const LbLayout L, const float* __
         __syncthreads();
         for (int k = tid; k < D; k += kLbThreads) V1[k] += (red[k] + red[DP + k]) + (red[2 * DP + k] + red[3 * DP + k]);
 
-        // ================= RFF part =================
-        for (int k = 0; k < (rff_done ? 0 : D); ++k) {
-            float G[DP];
-#pragma unroll
-            for (int j = 0; j < DP; ++j) G[j] = 0.f;
-            for (int ch = 0; ch < NCH; ++ch, ++it) {
-                // stage the next chunk (of this k, or the first of k + 1) into the other buffer: its last readers
-                // finished before the barrier that closed the previous trip
-                const bool more = !(k == D - 1 && ch == NCH - 1);
-                if (tid == 0 && more) {
-                    const int kn = ch + 1 < NCH ? k : k + 1, cn = ch + 1 < NCH ? ch + 1 : 0;
-                    gpode_bulk_g2s(obuf[(it + 1) & 1], om_g + ((size_t)kn * NCH + cn) * kLbSC * DP, kChunkBytes,
-                                   mbar + ((it + 1) & 1));
-                }
-                gpode_mbar_wait(mbar + (it & 1), (it >> 1) & 1);
-                const float* __restrict__ ob = obuf[it & 1];
-                const float* __restrict__ php = ph_g + (size_t)k * SU + ch * kLbSC;
-                const float* __restrict__ awp = aw_g + (size_t)k * SU + ch * kLbSC;
-#pragma unroll 1
-                for (int s = 0; s < kLbSC; s += 4) {
-                    const float4 ph4 = __ldg(reinterpret_cast<const float4*>(php + s));
-                    const float4 a4 = __ldg(reinterpret_cast<const float4*>(awp + s));
-                    float th0 = ph4.x, th1 = ph4.y, th2 = ph4.z, th3 = ph4.w;
-                    const float* __restrict__ o = ob + s * DP;
-#pragma unroll
-                    for (int j4 = 0; j4 < DP / 4; ++j4) {
-                        const float4 o0 = *reinterpret_cast<const float4*>(o + 4 * j4);
-                        const float4 o1 = *reinterpret_cast<const float4*>(o + DP + 4 * j4);
-                        const float4 o2 = *reinterpret_cast<const float4*>(o + 2 * DP + 4 * j4);
-                        const float4 o3 = *reinterpret_cast<const float4*>(o + 3 * DP + 4 * j4);
-                        float4 xv;
-                        if constexpr (kXReg) xv = make_float4(xr[4 * j4], xr[4 * j4 + 1], xr[4 * j4 + 2], xr[4 * j4 + 3]);
-                        else xv = *reinterpret_cast<const float4*>(xrow + 4 * j4);
-                        th0 = fmaf(xv.x, o0.x, th0); th1 = fmaf(xv.x, o1.x, th1);
-                        th2 = fmaf(xv.x, o2.x, th2); th3 = fmaf(xv.x, o3.x, th3);
-                        th0 = fmaf(xv.y, o0.y, th0); th1 = fmaf(xv.y, o1.y, th1);
-                        th2 = fmaf(xv.y, o2.y, th2); th3 = fmaf(xv.y, o3.y, th3);
-                        th0 = fmaf(xv.z, o0.z, th0); th1 = fmaf(xv.z, o1.z, th1);
-                        th2 = fmaf(xv.z, o2.z, th2); th3 = fmaf(xv.z, o3.z, th3);
-                        th0 = fmaf(xv.w, o0.w, th0); th1 = fmaf(xv.w, o1.w, th1);
-                        th2 = fmaf(xv.w, o2.w, th2); th3 = fmaf(xv.w, o3.w, th3);
-                    }
-                    const float g0 = a4.x * gpode_sin_red(th0), g1 = a4.y * gpode_sin_red(th1), g2 = a4.z * gpode_sin_red(th2),
-                                g3 = a4.w * gpode_sin_red(th3);
-#pragma unroll
-                    for (int j4 = 0; j4 < DP / 4; ++j4) {
-                        const float4 o0 = *reinterpret_cast<const float4*>(o + 4 * j4);
-                        const float4 o1 = *reinterpret_cast<const float4*>(o + DP + 4 * j4);
-                        const float4 o2 = *reinterpret_cast<const float4*>(o + 2 * DP + 4 * j4);
-                        const float4 o3 = *reinterpret_cast<const float4*>(o + 3 * DP + 4 * j4);
-                        G[4 * j4] = fmaf(g0, o0.x, fmaf(g1, o1.x, fmaf(g2, o2.x, fmaf(g3, o3.x, G[4 * j4]))));
-                        G[4 * j4 + 1] = fmaf(g0, o0.y, fmaf(g1, o1.y, fmaf(g2, o2.y, fmaf(g3, o3.y, G[4 * j4 + 1]))));
-                        G[4 * j4 + 2] = fmaf(g0, o0.z, fmaf(g1, o1.z, fmaf(g2, o2.z, fmaf(g3, o3.z, G[4 * j4 + 2]))));
-                        G[4 * j4 + 3] = fmaf(g0, o0.w, fmaf(g1, o1.w, fmaf(g2, o2.w, fmaf(g3, o3.w, G[4 * j4 + 3]))));
-                    }
-                }
-                __syncthreads();  // everyone is done with this buffer before it is refilled two trips later
-            }
-            // xb_j -= kb_k G_j;  A[k][j] -= sum_rows kb_k x_j G_j  (rows by warp shuffle, warps in warp order)
-            const float nkb = -kbs[tid * LD + k];
-#pragma unroll
-            for (int j = 0; j < DP; ++j) {
-                const float gj = nkb * G[j];
-                xbr[j] += gj;
-                const float v = gpode_warp_sum((kXReg ? xr[j < (kXReg ? DP : 4) ? j : 0] : xrow[j]) * gj);
-                if (lane == 0) red[warp * DP + j] = v;
-            }
-            __syncthreads();
-            for (int j = tid; j < DP; j += kLbThreads)
-                As[k * DP + j] += (red[j] + red[DP + j]) + (red[2 * DP + j] + red[3 * DP + j]);
-            __syncthreads();
-        }
-
         // ================= RBF part =================
         constexpr int TK = DP / 16, TJ = DP / 8;   // row-contraction tile per thread: 16 x 8 tiles cover [DP][DP]
-        static_assert(kLbThreads == 128 && (DP == 16 || DP == 32 || DP == 64), "tile mapping assumes 128 threads");
+        static_assert(kLbThreads == 128 && (DP == 16 || DP == 32), "tile mapping assumes 128 threads");
         const int ck0 = (tid >> 3) * TK, cj0 = (tid & 7) * TJ;
         constexpr bool kTwoRows = DP >= 32;   // two rows x half the inputs per thread in the exponent / t phases
         constexpr int NC2 = DP / 8;           // float4 chunks of a lane's half row
         const int h2 = tid & 1, rA = tid >> 1, rB = rA + kLbRows / 2;
-        auto off2 = [&](const int c) { return h2 * (DP / 2) + 4 * ((c + (DP == 64 ? h2 * (NC2 / 2) : 0)) & (NC2 - 1)); };
+        auto off2 = [&](const int c) { return h2 * (DP / 2) + 4 * c; };
         for (int m = 0; m < M; ++m) {
             const float* __restrict__ zm = z_g + (size_t)m * DP;
             const float* __restrict__ cm = c_g + (size_t)m * DP;
@@ -283,9 +165,8 @@ vjp_large_kernel(const float* __restrict__ pk, const LbLayout L, const float* __
             // Register tile: a thread owns TWO rows (rA, rB = rA + 64) x HALF of the input dimensions, so every W element
             // fetched from shared memory feeds both rows -- the one-row form below issues two broadcast LDS.128 (four
             // wavefronts each) per four packed FMAs and is bound by shared-memory wavefronts at DP >= 32. Chunk c of a
-            // lane is floats off(c) .. off(c)+3 of the row: the upper-half lane walks its chunks rotated by half a
-            // turn at DP = 64 so that the two lanes of a row pair never hit the same banks. The exponent halves of the
-            // two lanes are added by one shuffle (a + b in both lanes: bitwise the same value).
+            // lane is floats off(c) .. off(c)+3 of the row. The exponent halves of the two lanes are added by one
+            // shuffle (a + b in both lanes: bitwise the same value).
 #pragma unroll
             for (int c = 0; c < NC2; ++c) {
                 const int o = off2(c);
@@ -411,10 +292,7 @@ vjp_large_kernel(const float* __restrict__ pk, const LbLayout L, const float* __
                 for (int r = 0; r < kLbRows; ++r) {
                     float pv[TK];
                     float2 dv[TJ / 2];
-                    if constexpr (TK == 4) {
-                        const float4 p4 = *reinterpret_cast<const float4*>(stA + r * LD + ck0);
-                        pv[0] = p4.x; pv[1] = p4.y; pv[2] = p4.z; pv[3] = p4.w;
-                    } else if constexpr (TK == 2) {
+                    if constexpr (TK == 2) {
                         const float2 p2 = *reinterpret_cast<const float2*>(stA + r * LD + ck0);
                         pv[0] = p2.x; pv[1] = p2.y;
                     } else {
@@ -513,7 +391,7 @@ vjp_large_kernel(const float* __restrict__ pk, const LbLayout L, const float* __
     for (int i = tid; i < DP; i += kLbThreads) Ag[DP * DP + i] += V1[i];
 }
 
-// ---- RBF half of the VJP on EIGHT warps (used when the tcgen05 kernel has already done the RFF half) ---------------------
+// ---- RBF half of the VJP at DP = 64, on EIGHT warps ----------------------------------------------------------------
 // Same tiles, arithmetic and accumulator rows as the RBF part of vjp_large_kernel, but two warpgroups share the 128-row
 // tile, so every scheduler has two warps to interleave (ncu on the four-warp form at DP = 64: FMA pipe 24 %, issue 34 %,
 // shared-memory wavefronts 59 % -- latency with one warp per scheduler). Both warpgroups build the same dd registers
@@ -894,27 +772,16 @@ int lb_check(const gpode_cache_t* c) {
     return 0;
 }
 
-// persistent grid: SMs x resident CTAs of the VJP kernel for this DP (the accumulator rows are per CTA: every launch
-// of one backward pass and the finalize kernel must agree on this number)
+// persistent grid: SMs x the CTAs per SM the launch bounds ask for -- two of vjp_large_kernel (DP = 16, 32), one of
+// rbf_vjp_large_kernel (DP = 64). The accumulator rows are per CTA: every launch of one backward pass and the finalize
+// kernel must agree on this number, and it fixes the order in which the parameter-gradient sums are added, so it is a
+// constant rather than an occupancy query that would follow the compiler's register allocation.
 int lb_grid(int64_t B, int DP) {
-    static int occ_cache[3] = {0, 0, 0};
     int sms = 148, dev = 0;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const int slot = DP == 16 ? 0 : (DP == 32 ? 1 : 2);
-    if (occ_cache[slot] == 0) {
-        int occ = 1;
-        if (DP == 16) {
-            cudaFuncSetAttribute(vjp_large_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LbSmem<16>::bytes);
-            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, vjp_large_kernel<16>, kLbThreads, LbSmem<16>::bytes);
-        } else if (DP == 32) {
-            cudaFuncSetAttribute(vjp_large_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LbSmem<32>::bytes);
-            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, vjp_large_kernel<32>, kLbThreads, LbSmem<32>::bytes);
-        }
-        occ_cache[slot] = occ < 1 ? 1 : (occ > 4 ? 4 : occ);
-    }
     const int64_t tiles = (B + kLbRows - 1) / kLbRows;
-    int64_t g = (int64_t)sms * occ_cache[slot];
+    int64_t g = (int64_t)sms * (DP == 64 ? 1 : 2);
     if (g > tiles) g = tiles;
     if (g > kLbMaxCtas) g = kLbMaxCtas;
     return (int)(g < 1 ? 1 : g);
@@ -922,34 +789,30 @@ int lb_grid(int64_t B, int DP) {
 
 template <int DP>
 int launch_vjp(const float* pk, const LbLayout& L, const float* x, const float* f, const float* kb, float* gx,
-               int64_t B, float* acc, cudaStream_t st, int rff_done) {
+               int64_t B, float* acc, cudaStream_t st) {
     const size_t smem = LbSmem<DP>::bytes;
     GPODE_CUDA(cudaFuncSetAttribute(vjp_large_kernel<DP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     float* accA = acc;
     float* accT = accA + (size_t)kLbMaxCtas * (DP * DP + DP);
     float* accZ = accT + (size_t)kLbMaxCtas * L.D * L.M;
-    vjp_large_kernel<DP><<<lb_grid(B, DP), kLbThreads, smem, st>>>(pk, L, x, f, kb, gx, B, accA, accT, accZ, rff_done);
+    vjp_large_kernel<DP><<<lb_grid(B, DP), kLbThreads, smem, st>>>(pk, L, x, f, kb, gx, B, accA, accT, accZ);
     GPODE_LAUNCH_CHECK();
     return 0;
 }
 
-// floats of the FP32 kernel's accumulator rows (the tensor-core RFF rows follow them in acc_large)
+// floats of the RBF kernels' accumulator rows (the tensor-core RFF rows follow them in acc_large)
 int64_t lb_acc_floats(int D, int M) {
     const int DP = lb_dp(D);
     return (int64_t)kLbMaxCtas * ((int64_t)DP * DP + DP + (int64_t)D * M + (int64_t)M * DP);
 }
-// the RFF part on the tcgen05 kernel of large_rffb.cu unless the option large_bwd_umma is 0 (or it does not fit)
-bool use_rv(int D) { return gpode_option(GPODE_OPT_LARGE_BWD_UMMA) != 0 && gpode_rv_supported(D); }
-
+// the RFF half on the tcgen05 kernel of large_rffb.cu, then the RBF half on the CUDA cores
 int vjp_dispatch(const float* pk, int D, int M, int S, const float* x, const float* f, const float* kb, float* gx,
                  int64_t B, float* acc, cudaStream_t st) {
-    const LbLayout L = lb_layout(D, M, S);
-    int rff_done = 0;
-    if (use_rv(D)) {
-        if (int rc = gpode_rv_launch(pk + L.total, D, S, x, kb, gx, B, acc + lb_acc_floats(D, M), st)) return rc;
-        rff_done = 1;
-    }
-    if (rff_done && L.DP == 64 && gpode_option(GPODE_OPT_LARGE_BWD_UMMA) == 1) {   // option value 2: the four-warp RBF half
+    const LbLayout L = lb_layout(D, M);
+    if (int rc = gpode_rv_launch(pk + L.total, D, S, x, kb, gx, B, acc + lb_acc_floats(D, M), st)) return rc;
+    if (L.DP == 16) return launch_vjp<16>(pk, L, x, f, kb, gx, B, acc, st);
+    if (L.DP == 32) return launch_vjp<32>(pk, L, x, f, kb, gx, B, acc, st);
+    {
         constexpr int DP = 64;
         GPODE_CUDA(cudaFuncSetAttribute(rbf_vjp_large_kernel<DP>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                         (int)Rb2Smem<DP>::bytes));
@@ -960,9 +823,6 @@ int vjp_dispatch(const float* pk, int D, int M, int S, const float* x, const flo
         GPODE_LAUNCH_CHECK();
         return 0;
     }
-    if (L.DP == 16) return launch_vjp<16>(pk, L, x, f, kb, gx, B, acc, st, rff_done);
-    if (L.DP == 32) return launch_vjp<32>(pk, L, x, f, kb, gx, B, acc, st, rff_done);
-    return launch_vjp<64>(pk, L, x, f, kb, gx, B, acc, st, rff_done);
 }
 
 inline unsigned ew_grid(int64_t n) {
@@ -974,7 +834,7 @@ inline unsigned ew_grid(int64_t n) {
 
 extern "C" int64_t gpode_packed_large_bwd_floats(int D, int M, int S) {
     if (D <= GPODE_MAX_D || D > GPODE_MAX_D_LARGE || S < 1 || M < 1) return -1;
-    return lb_layout(D, M, S).total + gpode_rv_packed_floats(D, S);   // FP32 kernel's block | tensor-core RFF operands
+    return lb_layout(D, M).total + gpode_rv_packed_floats(D, S);   // RBF operands | tensor-core RFF operands
 }
 
 extern "C" int64_t gpode_acc_large_floats(int D, int M) {
@@ -985,9 +845,8 @@ extern "C" int64_t gpode_acc_large_floats(int D, int M) {
 extern "C" int gpode_pack_cache_large_bwd(const gpode_cache_t* c, float* packed_bwd, void* stream) {
     if (int rc = lb_check(c)) return rc;
     GPODE_CHECK_ARG(packed_bwd != nullptr, "packed_bwd is NULL");
-    const LbLayout L = lb_layout(c->D, c->M, c->S);
-    pack_lb_kernel<<<592, 256, 0, (cudaStream_t)stream>>>(L, c->omega, c->phase, c->w, c->Z, c->nu, c->ell, c->var,
-                                                         packed_bwd);
+    const LbLayout L = lb_layout(c->D, c->M);
+    pack_lb_kernel<<<592, 256, 0, (cudaStream_t)stream>>>(L, c->Z, c->nu, c->ell, c->var, packed_bwd);
     GPODE_LAUNCH_CHECK();
     return gpode_rv_pack(c, packed_bwd + L.total, (cudaStream_t)stream);
 }
@@ -1011,7 +870,7 @@ extern "C" int gpode_grads_finalize_large(const gpode_cache_t* c, const float* a
     const float* accZ = accT + (size_t)kLbMaxCtas * D * M;
     const int n_out = D * D + 2 * D * M;
     const float* accR = acc_large + lb_acc_floats(D, M);
-    const int n_rows_r = use_rv(D) ? gpode_rv_grid(B) * 4 : 0;
+    const int n_rows_r = gpode_rv_grid(B) * 4;
     finalize_large_kernel<<<(n_out + 31) / 32, 256, 0, (cudaStream_t)stream>>>(
         D, DP, M, lb_grid(B, DP), accA, accT, accZ, accR, n_rows_r, gpode_rv_dn(D), c->ell, c->var, grad_ell, grad_Z,
         grad_nu);

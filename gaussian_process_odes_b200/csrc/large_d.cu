@@ -1,15 +1,11 @@
-// Vector field and fixed-grid RK4 for 8 < D <= 64 (forward only) -- the upper half of the scaling sweep
-// (BASELINE.json configs[4]: state dim 2-64). At these sizes neither a row's state (6 D floats through an RK4 step)
-// nor the sampled function (D*S*D floats of Omega: 262 KB at D=16, 4 MB at D=64) fits the register / shared-memory
-// budget of the row-per-thread kernels, so the mapping changes:
-//   * a CTA owns a tile of TR = 32 rows whose state and stage derivatives live in shared memory;
-//   * thread = (output dim k, group of 8 rows): for every Fourier feature it streams the column Omega[:, s, k] from
-//     global memory (L2-resident, coalesced over k, every value reused for 8 rows from registers) against the tile's
-//     x in shared memory -- a register-blocked GEMV batch, FP32 FMA as in the small-D kernels (a 3xTF32 tensor-core
-//     projection is the planned next step for these shapes);
-//   * the RBF term uses the same mapping with Z and nu read through the read-only cache.
-// Arithmetic replaced: DSVGP_Layer.forward (reference src/core/dsvgp.py:172-197) inside torchdiffeq's rk4 step
-// (restated in oracle/torchdiffeq_shim). Takes the RAW cache tensors (no repacking needed).
+// RBF term of the vector field for 8 < D <= 64 on the FP32 CUDA cores, added to a Fourier-feature term computed by the
+// tensor-core kernel (gpode_rff_fwd_large, large_umma.cu): f = f_rff + sum_m var_k nu_km exp(-0.5 r_km^2). This is the
+// fallback of gpode_rbf_fwd_large when the inducing points do not fit its shared-memory copy of Z. Mapping:
+//   * a CTA owns a tile of TR = 32 rows whose state lives in shared memory;
+//   * thread = (output dim k, group of 8 rows): for every inducing point it reads Z through the read-only cache against
+//     the tile's x in shared memory, every value reused for 8 rows from registers.
+// Arithmetic replaced: the RBF half of DSVGP_Layer.forward (reference src/core/dsvgp.py:172-197). Takes the RAW cache
+// tensors (no repacking needed).
 #include "common.cuh"
 
 namespace {
@@ -19,50 +15,25 @@ constexpr int kRG = 8;    // rows per thread (register block)
 constexpr int kNG = kTR / kRG;
 
 struct LdArgs {
-    int D, M, S;
-    const float* omega;  // [D,S,D] (j,s,k)
-    const float* phase;  // [S,D]
-    const float* w;      // [S,D]
+    int D, M;
     const float* Z;      // [M,D]
     const float* nu;     // [D,M]
     const float* ell;    // [D,D] (k,j)
     const float* var;    // [D]
 };
 
-// f[r][k] for the tile; xs, fs: shared, TRANSPOSED [D][kTR] (a thread's 8 rows are two LDS.128);
-// thread (k = tid % D, g = tid / D) handles rows g*8 .. g*8+7
-// frff != nullptr: the Fourier-feature term was computed by the tensor-core kernel (large_umma.cu) and is read from
-// global memory [B,D]; only the RBF term is evaluated here.
+// f[r][k] = frff[r][k] + RBF term for the tile; xs, fs: shared, TRANSPOSED [D][kTR] (a thread's 8 rows are two
+// LDS.128); thread (k = tid % D, g = tid / D) handles rows g*8 .. g*8+7
 __device__ void eval_tile(const LdArgs& a, const float* __restrict__ xs, float* __restrict__ fs, const float* wl,
-                          const int k, const int g, const bool active, const float* __restrict__ frff = nullptr,
-                          const int64_t row0 = 0, const int64_t B = 0) {
-    const int D = a.D, S = a.S, M = a.M;
+                          const int k, const int g, const bool active, const float* __restrict__ frff,
+                          const int64_t row0, const int64_t B) {
+    const int D = a.D, M = a.M;
     if (active) {
         float acc[kRG];
 #pragma unroll
         for (int r = 0; r < kRG; ++r) {
             const int64_t row = row0 + g * kRG + r;
-            acc[r] = (frff != nullptr && row < B) ? __ldg(frff + row * D + k) : 0.f;
-        }
-        const float ak = sqrtf(__ldg(a.var + k) / (float)S);
-        for (int s = 0; frff == nullptr && s < S; ++s) {
-            float th[kRG];
-            const float ph = __ldg(a.phase + s * D + k);
-#pragma unroll
-            for (int r = 0; r < kRG; ++r) th[r] = ph;
-            const float* om = a.omega + (size_t)s * D + k;
-            for (int j = 0; j < D; ++j) {
-                const float o = __ldg(om + (size_t)j * S * D);
-                const float4 xa = *reinterpret_cast<const float4*>(xs + j * kTR + g * kRG);
-                const float4 xb = *reinterpret_cast<const float4*>(xs + j * kTR + g * kRG + 4);
-                th[0] = fmaf(xa.x, o, th[0]); th[1] = fmaf(xa.y, o, th[1]);
-                th[2] = fmaf(xa.z, o, th[2]); th[3] = fmaf(xa.w, o, th[3]);
-                th[4] = fmaf(xb.x, o, th[4]); th[5] = fmaf(xb.y, o, th[5]);
-                th[6] = fmaf(xb.z, o, th[6]); th[7] = fmaf(xb.w, o, th[7]);
-            }
-            const float as = __ldg(a.w + s * D + k) * ak;
-#pragma unroll
-            for (int r = 0; r < kRG; ++r) acc[r] = fmaf(as, __cosf(th[r]), acc[r]);
+            acc[r] = row < B ? __ldg(frff + row * D + k) : 0.f;
         }
         const float vk = __ldg(a.var + k);
         for (int m = 0; m < M; ++m) {
@@ -91,122 +62,66 @@ __device__ void eval_tile(const LdArgs& a, const float* __restrict__ xs, float* 
     __syncthreads();
 }
 
-#define GPODE_THIRD_LD 0.3333333432674407958984375f
-
-// smem: wl[D*D] | y[kTR*D] | ys | k1 | k2 | k3 | k4
-__global__ void large_d_kernel(const LdArgs a, const float* __restrict__ x0, const float* __restrict__ ts,
-                               const int Tg, const int64_t B, float* __restrict__ xs_out, const int vf_only,
-                               const float* __restrict__ frff) {
+// smem: wl[D*D] | y[kTR*D] | f[kTR*D]
+__global__ void large_d_rbf_kernel(const LdArgs a, const float* __restrict__ x, const int64_t B,
+                                   const float* __restrict__ frff, float* __restrict__ out) {
     extern __shared__ __align__(16) float sm[];
     const int D = a.D;
     float* wl = sm;
     float* y = wl + ((D * D + 3) & ~3);  // keep the tiles 16-byte aligned for the float4 reads
-    float* ys = y + kTR * D;
-    float* k1 = ys + kTR * D;
-    float* k2 = k1 + kTR * D;
-    float* k3 = k2 + kTR * D;
-    float* k4 = k3 + kTR * D;
+    float* fs = y + kTR * D;
     for (int i = threadIdx.x; i < D * D; i += blockDim.x) {
         const float l = __ldg(a.ell + i);
         wl[i] = GPODE_HALF_LOG2E / (l * l);
     }
     const int k = threadIdx.x % D, g = threadIdx.x / D;
     const bool active = g < kNG;
-    const int64_t plane = B * D;
     const int64_t ntiles = (B + kTR - 1) / kTR;
     for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
         const int64_t row0 = tile * kTR;
         __syncthreads();
         for (int i = threadIdx.x; i < kTR * D; i += blockDim.x) {
             const int r = i / D, j = i - r * D;
-            y[j * kTR + r] = row0 + r < B ? __ldg(x0 + row0 * D + i) : 0.f;
+            y[j * kTR + r] = row0 + r < B ? __ldg(x + row0 * D + i) : 0.f;
         }
         __syncthreads();
-        if (vf_only) {
-            eval_tile(a, y, k1, wl, k, g, active, frff, row0, B);
-            for (int i = threadIdx.x; i < kTR * D; i += blockDim.x) {
-                const int r = i / D, j = i - r * D;
-                if (row0 + r < B) xs_out[row0 * D + i] = k1[j * kTR + r];
-            }
-            continue;
-        }
+        eval_tile(a, y, fs, wl, k, g, active, frff, row0, B);
         for (int i = threadIdx.x; i < kTR * D; i += blockDim.x) {
             const int r = i / D, j = i - r * D;
-            if (row0 + r < B) xs_out[row0 * D + i] = y[j * kTR + r];
-        }
-        for (int step = 0; step + 1 < Tg; ++step) {
-            const float dt = __fsub_rn(__ldg(ts + step + 1), __ldg(ts + step));
-            eval_tile(a, y, k1, wl, k, g, active);
-            for (int i = threadIdx.x; i < kTR * D; i += blockDim.x)
-                ys[i] = __fadd_rn(y[i], __fmul_rn(__fmul_rn(dt, k1[i]), GPODE_THIRD_LD));
-            __syncthreads();
-            eval_tile(a, ys, k2, wl, k, g, active);
-            for (int i = threadIdx.x; i < kTR * D; i += blockDim.x)
-                ys[i] = __fadd_rn(y[i], __fmul_rn(dt, __fsub_rn(k2[i], __fmul_rn(k1[i], GPODE_THIRD_LD))));
-            __syncthreads();
-            eval_tile(a, ys, k3, wl, k, g, active);
-            for (int i = threadIdx.x; i < kTR * D; i += blockDim.x)
-                ys[i] = __fadd_rn(y[i], __fmul_rn(dt, __fadd_rn(__fsub_rn(k1[i], k2[i]), k3[i])));
-            __syncthreads();
-            eval_tile(a, ys, k4, wl, k, g, active);
-            for (int i = threadIdx.x; i < kTR * D; i += blockDim.x) {
-                const float sum = __fadd_rn(__fadd_rn(k1[i], __fmul_rn(3.0f, __fadd_rn(k2[i], k3[i]))), k4[i]);
-                y[i] = __fadd_rn(y[i], __fmul_rn(__fmul_rn(sum, dt), 0.125f));
-            }
-            __syncthreads();
-            for (int i = threadIdx.x; i < kTR * D; i += blockDim.x) {
-                const int r = i / D, j = i - r * D;
-                if (row0 + r < B) xs_out[(int64_t)(step + 1) * plane + row0 * D + i] = y[j * kTR + r];
-            }
+            if (row0 + r < B) out[row0 * D + i] = fs[j * kTR + r];
         }
     }
 }
 
-int launch_large(const gpode_cache_t* c, const float* x0, const float* ts, int Tg, int64_t B, float* out, int vf_only,
-                 cudaStream_t st, const float* frff = nullptr) {
+}  // namespace
+
+extern "C" int gpode_vf_fwd_large_add_rbf(const gpode_cache_t* c, const float* x, const float* f_rff, float* f,
+                                          int64_t B, void* stream) {
     GPODE_CHECK_ARG(c != nullptr, "cache is NULL");
     GPODE_CHECK_ARG(c->D > GPODE_MAX_D && c->D <= GPODE_MAX_D_LARGE, "large-D path needs %d < D <= %d, got %d",
                     GPODE_MAX_D, GPODE_MAX_D_LARGE, c->D);
     GPODE_CHECK_ARG(c->M >= 1 && c->S >= 1 && B >= 0, "bad sizes");
     GPODE_CHECK_ARG(c->Z && c->nu && c->ell && c->var, "cache tensor is NULL");
-    GPODE_CHECK_ARG(frff != nullptr || (c->omega && c->phase && c->w), "cache tensor is NULL");
+    GPODE_CHECK_ARG(f_rff != nullptr, "f_rff is NULL");
     if (B == 0) return 0;
-    GPODE_CHECK_ARG(x0 && out, "NULL argument");
-    LdArgs a{c->D, c->M, c->S, c->omega, c->phase, c->w, c->Z, c->nu, c->ell, c->var};
+    GPODE_CHECK_ARG(x && f, "NULL argument");
+    const LdArgs a{c->D, c->M, c->Z, c->nu, c->ell, c->var};
     const int D = c->D;
     const int threads = ((kNG * D + 31) / 32) * 32;  // D=16 -> 64, D=32 -> 128, D=64 -> 256
-    const size_t smem = sizeof(float) * ((size_t)((D * D + 3) & ~3) + 6 * (size_t)kTR * D);
-    GPODE_CUDA(cudaFuncSetAttribute(large_d_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const size_t smem = sizeof(float) * ((size_t)((D * D + 3) & ~3) + 2 * (size_t)kTR * D);
+    GPODE_CUDA(cudaFuncSetAttribute(large_d_rbf_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int occ = 0, sms = 148, dev = 0;
     GPODE_CUDA(cudaGetDevice(&dev));
     GPODE_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    GPODE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, large_d_kernel, threads, smem));
+    GPODE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, large_d_rbf_kernel, threads, smem));
     if (occ < 1) {
         gpode_set_error("large-D kernel does not fit on an SM (smem %zu bytes)", smem);
         return -2;
     }
     const int64_t ntiles = (B + kTR - 1) / kTR;
     const int64_t cap = (int64_t)sms * occ;
-    large_d_kernel<<<(unsigned)(ntiles < cap ? ntiles : cap), threads, smem, st>>>(a, x0, ts, Tg, B, out, vf_only,
-                                                                                            frff);
+    large_d_rbf_kernel<<<(unsigned)(ntiles < cap ? ntiles : cap), threads, smem, (cudaStream_t)stream>>>(a, x, B, f_rff,
+                                                                                                         f);
     GPODE_LAUNCH_CHECK();
     return 0;
-}
-
-}  // namespace
-
-extern "C" int gpode_vf_fwd_large(const gpode_cache_t* cache, const float* x, float* f, int64_t B, void* stream) {
-    return launch_large(cache, x, nullptr, 1, B, f, 1, (cudaStream_t)stream);
-}
-
-extern "C" int gpode_vf_fwd_large_add_rbf(const gpode_cache_t* cache, const float* x, const float* f_rff, float* f,
-                                          int64_t B, void* stream) {
-    GPODE_CHECK_ARG(f_rff != nullptr, "f_rff is NULL");
-    return launch_large(cache, x, nullptr, 1, B, f, 1, (cudaStream_t)stream, f_rff);
-}
-
-extern "C" int gpode_rk4_fwd_large(const gpode_cache_t* cache, const float* x0, const float* t, int Tg, int64_t B,
-                                   float* xs, void* stream) {
-    GPODE_CHECK_ARG(Tg >= 1 && (Tg == 1 || t != nullptr), "bad time grid");
-    return launch_large(cache, x0, t, Tg, B, xs, 0, (cudaStream_t)stream);
 }

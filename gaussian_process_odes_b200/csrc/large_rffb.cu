@@ -13,7 +13,7 @@
 //   GEMM 2  TS form: A = p, WRITTEN BACK TO TENSOR MEMORY by the row threads (tcgen05.st, hi and lo column blocks), B =
 //           the same chunk of Omega_k re-tiled with the input dimension as N and the feature as K; the accumulator G_k
 //           collects all chunks of output k.
-// The FP32 CUDA-core kernel this replaces (large_bwd.cu, RFF part of vjp_large_kernel) spends 4 S D^2 FMAs per row on
+// The FP32 CUDA-core loop this replaced (formerly the RFF part of vjp_large_kernel) spent 4 S D^2 FMAs per row on
 // the two projections: the whole VJP took 80 ms per 1e5 rows at D = 64 (register spills); this kernel 5.7 ms (ncu: tensor
 // pipe 26 % busy, bound by the L2 operand stream -- 14 GB per 1e5 rows, two tilings of Omega -- and by the single row
 // warp per scheduler), the whole VJP 21.5 ms (profiles/r02_summary.md section 4).
@@ -410,7 +410,6 @@ int64_t gpode_rv_packed_floats(int D, int S) {
     return (int64_t)D * NCH * (rv_b1(D) + rv_b2(D)) + (int64_t)D * rv_su(S);
 }
 int64_t gpode_rv_acc_floats(int D) { return (int64_t)kRvMaxCtas * 4 * rv_dn(D) * rv_dn(D); }
-bool gpode_rv_supported(int D) { return rv_smem(D) <= 227u * 1024u; }
 int gpode_rv_grid(int64_t B) {
     int sms = 148, dev = 0;
     cudaGetDevice(&dev);
@@ -432,6 +431,7 @@ int gpode_rv_pack(const gpode_cache_t* c, float* out, cudaStream_t st) {
 int gpode_rv_launch(const float* packed, int D, int S, const float* x, const float* kb, float* gx, int64_t B, float* acc,
                     cudaStream_t st) {
     const size_t smem = rv_smem(D);
+    GPODE_CHECK_ARG(smem <= 227u * 1024u, "large-D tensor-core VJP needs %zu bytes of shared memory at D=%d", smem, D);
     const int grid = gpode_rv_grid(B);
     const int DN = rv_dn(D);
 #define GPODE_RV_CASE(DN_)                                                                                              \

@@ -13,7 +13,7 @@
 // "slot free" for the next copy; the rows' 128 arrivals -> "TMEM buffer free".
 //
 // Arithmetic replaced: DSVGP_Layer.rff_forward (reference src/core/dsvgp.py:124-137) for the upper sweep points of
-// BASELINE.json configs[4]. Output: f_rff [B, D]; gpode_vf_fwd_large adds the RBF term.
+// BASELINE.json configs[4]. Output: f_rff [B, D]; gpode_rbf_fwd_large (or gpode_vf_fwd_large_add_rbf) adds the RBF term.
 #include "umma.cuh"
 
 namespace {

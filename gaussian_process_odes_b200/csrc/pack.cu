@@ -17,7 +17,7 @@ extern "C" int gpode_abi_version(void) { return GPODE_B200_ABI_VERSION; }
 
 extern "C" int64_t gpode_packed_floats(int D, int M, int S) {
     if (D < 1 || M < 1 || S < 1) return -1;
-    return gpode_layout(D, M, S).total_all;
+    return gpode_layout(D, M, S).n_packed;
 }
 
 namespace {
@@ -25,7 +25,7 @@ namespace {
 // One thread per packed record. Source layouts are the reference's cache tensors (src/core/dsvgp.py:100-103,122):
 // omega (j,s,k), phase (s,k), w (s,k), Z (m,j), nu (k,m), ell (k,j), var (k).
 // blockIdx.y = parameter set (batched Monte-Carlo prediction): omega / phase / w / nu carry a leading set dimension,
-// Z / ell / var are shared; the packed blocks follow each other at stride L.total_all.
+// Z / ell / var are shared; the packed blocks follow each other at stride L.n_packed.
 __global__ void pack_kernel(const GpodeLayout L, const float* __restrict__ omega, const float* __restrict__ phase,
                             const float* __restrict__ w, const float* __restrict__ Z, const float* __restrict__ nu,
                             const float* __restrict__ ell, const float* __restrict__ var, float* __restrict__ out) {
@@ -36,20 +36,19 @@ __global__ void pack_kernel(const GpodeLayout L, const float* __restrict__ omega
         phase += set * S * D;
         w += set * S * D;
         if (nu) nu += set * D * M;
-        out += set * L.total_all;
+        out += set * L.n_packed;
     }
-    const int n_rff = D * S2, n_kern = M, n_il = D, n_mma = D * L.S8 * 32;
-    const int n_umma = D <= 7 ? D * L.SU : 0;
+    const int n_rff = D * S2, n_kern = M, n_il = D;
     const int n_mmah = D <= GPODE_MMAH_MAX_D ? D * L.S8P * 32 : 0;
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n_rff + n_kern + n_il + n_mma + n_umma + n_mmah;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n_rff + n_kern + n_il + n_mmah;
          i += gridDim.x * blockDim.x) {
-        if (i >= n_rff + n_kern + n_il + n_mma + n_umma) {
+        if (i >= n_rff + n_kern + n_il) {
             // f16 tensor-core operands of the adjoint (see GpodeLayout::mmah) for one lane of one (k, feature tile)
-            const int q = i - (n_rff + n_kern + n_il + n_mma + n_umma);
+            const int q = i - (n_rff + n_kern + n_il);
             const int lane = q & 31, rec = q >> 5;          // rec = k * S8P + ft
             const int k = rec / L.S8P, ft = rec - k * L.S8P;
             const int g = lane >> 2, t = lane & 3;
-            uint32_t* o = reinterpret_cast<uint32_t*>(out + L.off_mmag + (size_t)rec * GPODE_MMAH_REC);
+            uint32_t* o = reinterpret_cast<uint32_t*>(out + L.off_mmah + (size_t)rec * GPODE_MMAH_REC);
             auto om = [&](int j, int sidx) -> float {
                 return (j < D && sidx < S) ? omega[((size_t)j * S + sidx) * D + k] : 0.f;
             };
@@ -106,50 +105,11 @@ __global__ void pack_kernel(const GpodeLayout L, const float* __restrict__ omega
             float* o = out + L.off_kern + (size_t)m * L.KS;
             for (int j = 0; j < D; ++j) o[j] = Z[m * D + j];
             for (int k = 0; k < L.KS - D; ++k) o[D + k] = (nu && k < D) ? var[k] * nu[k * M + m] : 0.f;
-        } else if (i < n_rff + n_kern + n_il) {
+        } else {
             const int j = i - n_rff - n_kern;
             float* o = out + L.off_il + (size_t)j * L.WP;
             for (int k = 0; k < L.WP; ++k)
                 o[k] = k < D ? -GPODE_HALF_LOG2E / (ell[k * D + j] * ell[k * D + j]) : 0.f;
-        } else if (i >= n_rff + n_kern + n_il + n_mma) {
-            // tcgen05 operand rows: one feature s of output k (see GpodeLayout)
-            const int q = i - n_rff - n_kern - n_il - n_mma;
-            const int k = q / L.SU, sidx = q - k * L.SU;
-            float* rec = out + L.off_umma + (size_t)k * GPODE_UMMA_REC(L.SU);
-            float* bh = rec + (sidx >> 3) * 64 + (sidx & 7) * 4;
-            float* bl = bh + 8 * L.SU;
-            const bool ok = sidx < S;
-            for (int slot = 0; slot < 8; ++slot) {
-                float v = 0.f;
-                if (ok && slot < D) v = omega[((size_t)slot * S + sidx) * D + k];
-                else if (ok && slot == D) v = phase[sidx * D + k];
-                float hi, lo;
-                gpode_split_tf32_rn(v, hi, lo);
-                bh[(slot >> 2) * 32 + (slot & 3)] = hi;
-                bl[(slot >> 2) * 32 + (slot & 3)] = lo;
-            }
-            rec[16 * L.SU + sidx] = ok ? w[sidx * D + k] * sqrtf(var[k] / (float)S) : 0.f;
-        } else {
-            // tensor-core operand fragments of one (k, feature tile) for one lane (g = lane / 4, t = lane % 4)
-            const int q = i - n_rff - n_kern - n_il;
-            const int lane = q & 31, rec = q >> 5;          // rec = k * S8 + ft
-            const int k = rec / L.S8, ft = rec - k * L.S8;
-            const int g = lane >> 2, t = lane & 3;
-            float* o = out + L.off_mma + (size_t)rec * GPODE_MMA_REC;
-            auto om = [&](int j, int sidx) -> float {
-                return (j < D && sidx < S) ? omega[((size_t)j * S + sidx) * D + k] : 0.f;
-            };
-            // theta = x Omega: B is (j x feature), b0 = B[t][g], b1 = B[t+4][g]
-            o[lane * 2 + 0] = om(t, 8 * ft + g);
-            o[lane * 2 + 1] = om(t + 4, 8 * ft + g);
-            if (g == 0) {
-                const float ak = sqrtf(var[k] / (float)S);
-                for (int h = 0; h < 2; ++h) {
-                    const int sidx = 8 * ft + 2 * t + h;
-                    o[64 + t * 4 + h] = sidx < S ? phase[sidx * D + k] : 0.f;
-                    o[64 + t * 4 + 2 + h] = sidx < S ? w[sidx * D + k] * ak : 0.f;
-                }
-            }
         }
     }
 }
@@ -163,8 +123,7 @@ static int pack_sets(const gpode_cache_t* c, int n_sets, float* packed, void* st
     GPODE_CHECK_ARG(c->M >= 1 && c->S >= 1, "M=%d and S=%d must be positive", c->M, c->S);
     GPODE_CHECK_ARG(c->omega && c->phase && c->w && c->Z && c->ell && c->var, "cache tensor is NULL");
     const GpodeLayout L = gpode_layout(c->D, c->M, c->S);
-    const int n = c->D * L.S2 + c->M + c->D + c->D * L.S8 * 32 + (c->D <= 7 ? c->D * L.SU : 0) +
-                  (c->D <= GPODE_MMAH_MAX_D ? c->D * L.S8P * 32 : 0);
+    const int n = c->D * L.S2 + c->M + c->D + (c->D <= GPODE_MMAH_MAX_D ? c->D * L.S8P * 32 : 0);
     pack_kernel<<<dim3((n + 127) / 128, n_sets), 128, 0, (cudaStream_t)stream>>>(L, c->omega, c->phase, c->w, c->Z,
                                                                                  c->nu, c->ell, c->var, packed);
     GPODE_LAUNCH_CHECK();
@@ -187,8 +146,7 @@ extern "C" int gpode_pack_cache_sets(const gpode_cache_t* c, int n_sets, float* 
 namespace {
 std::atomic<int> g_opt[GPODE_OPT_COUNT];
 std::once_flag g_opt_once;
-const char* const kOptNames[GPODE_OPT_COUNT] = {"bwd_mma", "fwd_mma", "mma_parts", "force_narrow", "use_mma",
-                                                  "large_bwd_umma"};
+const char* const kOptNames[GPODE_OPT_COUNT] = {"bwd_mma", "fwd_mma"};
 void opt_init() {
     auto env_int = [](const char* n, int dflt) {
         const char* e = getenv(n);
@@ -196,10 +154,6 @@ void opt_init() {
     };
     g_opt[GPODE_OPT_BWD_MMA] = env_int("GPODE_BWD_MMA", 1);
     g_opt[GPODE_OPT_FWD_MMA] = env_int("GPODE_FWD_MMA", 1);
-    g_opt[GPODE_OPT_MMA_PARTS] = env_int("GPODE_MMA_PARTS", 3);
-    g_opt[GPODE_OPT_FORCE_NARROW] = getenv("GPODE_FORCE_NARROW") != nullptr;
-    g_opt[GPODE_OPT_USE_MMA] = getenv("GPODE_USE_MMA") != nullptr;
-    g_opt[GPODE_OPT_LARGE_BWD_UMMA] = env_int("GPODE_LARGE_BWD_UMMA", 1);
 }
 }  // namespace
 int gpode_option(int which) {
@@ -214,7 +168,7 @@ extern "C" int gpode_set_option(const char* name, int value) {
             g_opt[i].store(value, std::memory_order_relaxed);
             return 0;
         }
-    gpode_set_error("unknown option %s (bwd_mma, fwd_mma, mma_parts, force_narrow, use_mma, large_bwd_umma)", name);
+    gpode_set_error("unknown option %s (bwd_mma, fwd_mma)", name);
     return -1;
 }
 extern "C" int gpode_get_option(const char* name) {

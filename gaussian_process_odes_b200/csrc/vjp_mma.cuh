@@ -3,7 +3,7 @@
 // mma.sync m16n8k16 (SASS HMMA.16816.F32); sin, the RBF term, the stage algebra and every parameter-gradient partial
 // sum stay FP32. Why the adjoint and not the forward kernel: ncu (profiles/r01_summary.md) shows the FFMA2 adjoint
 // FMA-pipe bound (72 % busy, MUFU 36 %), and 10 of its 13 FMA-pipe cycles per (feature, output) are exactly these two
-// projections; the forward kernel is MUFU-bound and gains nothing (measured, vf_mma.cuh / vf_umma.cu).
+// projections; the forward kernel is MUFU-bound and gains nothing (measured with the 3xTF32 and tcgen05 forward experiments, DESIGN.md).
 //
 // Arithmetic replaced: autograd through DSVGP_Layer.forward (reference src/core/dsvgp.py:172-197, rff_forward
 // :124-137, RBF.K src/core/kernels.py:53-99); formulas in SURVEY.md section 8(a) row A7.
@@ -100,7 +100,7 @@ template <int D>
 __device__ __forceinline__ void vf_vjp_h(const float* __restrict__ small, const uint32_t* __restrict__ mmah,
                                          float* __restrict__ stage, const int M, const int S8P, const float (&x)[1][D],
                                          const float (&kb)[1][D], const float (&fst)[1][D], float (&xb)[1][D],
-                                         HAcc<D>& acc, const int lane, const int parts = 3) {
+                                         HAcc<D>& acc, const int lane) {
     static_assert(D <= GPODE_MMAH_MAX_D, "x_hi | x_hi | x_lo must fit the 16 contraction slots");
     constexpr int KS = VfShape<D>::KS, WP = VfShape<D>::WP, SXS = HShape<D>::SXS;
     const float* __restrict__ kern = small;
@@ -290,49 +290,9 @@ __device__ __forceinline__ void vf_vjp_h(const float* __restrict__ small, const 
         for (int j = 0; j < D; ++j) xbp[j] = fmaf(d[j], (tq[j].x + tq[j].y) + tl[j], xbp[j]);
     };
 
-#ifdef GPODE_VJP_FUSED_EXPERIMENT
-    if ((parts & 16) && (parts & 3) == 3) {
-        // FUSED stream (experiment, compiled only with -DGPODE_VJP_FUSED_EXPERIMENT; mma_parts bit 4): two inducing
-        // points of the RBF part ride in every feature-tile-pair trip of the RFF loop; same sums in the same order, so
-        // the results are bit-identical. MEASURED (B200, D = 5, M = 100, 1e6 rows, tools/time_bwd_modes.py, whole
-        // backward pass): 12 warps 5.40 ms against 5.06 ms for the two-part form (168 registers, 100 bytes of spills);
-        // 8 warps / 248 registers 5.07 ms against 5.21 ms. Unlike the forward evaluation (vf_eval_h mode 2, -5 %) the
-        // adjoint gains nothing: it is bound by instruction dispatch (10 issue slots per sine), not by a pipe that the
-        // other part leaves idle.
-        rff_begin();
-        rbf_begin();
-        int m = 0;
-#pragma unroll 1
-        for (int k = 0; k < D; ++k) {
-            float Ga[2][4], Gb[2][4], Gl[2][4];
-#pragma unroll
-            for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-                for (int i = 0; i < 4; ++i) Ga[mt][i] = Gb[mt][i] = Gl[mt][i] = 0.f;
-            const uint32_t* __restrict__ rec = mmah + (size_t)k * S8P * GPODE_MMAH_REC;
-            const int n_pairs = S8P >> 1;
-            const int n_fused = ((M - m) >> 1) < n_pairs ? ((M - m) >> 1) : n_pairs;
-            int fp = 0;
-#pragma unroll 1
-            for (; fp < n_fused; ++fp, rec += 2 * GPODE_MMAH_REC, m += 2) {
-                rff_pair(rec, Ga, Gb, Gl);
-                rbf_step(m);
-                rbf_step(m + 1);
-            }
-#pragma unroll 1
-            for (; fp < n_pairs; ++fp, rec += 2 * GPODE_MMAH_REC) rff_pair(rec, Ga, Gb, Gl);
-            rff_output_done(k, Ga, Gb, Gl);
-        }
-        rff_end();
-#pragma unroll 1
-        for (; m < M; ++m) rbf_step(m);
-    } else
-#endif
-    {
 #pragma unroll 1
     for (int part = 0; part < 2; ++part) {
         if ((part == 0) != rbf_first) {
-        if (parts & 1) {
             rff_begin();
 #pragma unroll 1   // one copy of the feature loop: the instruction cache is the scarce resource with 12 warps per SM
             for (int k = 0; k < D; ++k) {
@@ -348,13 +308,11 @@ __device__ __forceinline__ void vf_vjp_h(const float* __restrict__ small, const 
                 rff_output_done(k, Ga, Gb, Gl);
             }
             rff_end();
-        }
-        } else if (parts & 2) {
+        } else {
             rbf_begin();
 #pragma unroll 2
             for (int m = 0; m < M; ++m) rbf_step(m);
         }
-    }
     }
     __syncwarp();
     const float cG = 1.f / (GPODE_NEG_2LN2 * GPODE_MMAH_SCALE);
@@ -369,7 +327,7 @@ __device__ __forceinline__ void vf_vjp_h(const float* __restrict__ small, const 
 template <int D>
 __device__ __forceinline__ void vf_eval_h(const float* __restrict__ small, const uint32_t* __restrict__ mmah,
                                           float* __restrict__ stage, const int M, const int S8P, const float (&x)[1][D],
-                                          float (&f)[1][D], const int lane, const int mode = 0) {
+                                          float (&f)[1][D], const int lane) {
     static_assert(D <= GPODE_MMAH_MAX_D, "x_hi | x_hi | x_lo must fit the 16 contraction slots");
     constexpr int KS = VfShape<D>::KS, WP = VfShape<D>::WP, SXS = HShape<D>::SXS;
     const float* __restrict__ kern = small;
@@ -397,17 +355,13 @@ __device__ __forceinline__ void vf_eval_h(const float* __restrict__ small, const
     float fl = 0.f;
 #pragma unroll
     for (int kp = 0; kp < KF; ++kp) fu[kp] = make_float2(0.f, 0.f);
-    // The RFF part is bound by the MUFU pipe (cos), the RBF part by FMA dispatch: half of the warps of every scheduler
-    // take them in the opposite order so that the two kinds of work meet on the SM at the same time.
-    // mode 0 (default): FUSED -- one inducing point of the RBF term rides in every feature-tile trip of the RFF loop;
-    // mode 1: the two parts one after the other; mode 2: one after the other, half of the warps in the opposite order
-    // (the round-1 / early round-2 form). Why fused: the RFF loop alone saturates the MUFU pipe (ncu source view: 16
-    // cosines per 129.7 cycles of a sub-partition = 99 %), the RBF loop alone needs the FP32 pipe and the MUFU pipe for
-    // 40 cycles each per inducing point and reaches 65 % of either, and a warp issues in order -- only a stream that
-    // carries MUFU work everywhere keeps that pipe fed (tools/pipe_probe.cu: FFMA2 and MUFU do overlap when both are on
-    // offer). Measured, D = 5, M = 100, 1e6 rows: evaluation 0.528 -> 0.516 ms, RK4 step 2.123 -> 2.021 ms, bit-identical
+    // One inducing point of the RBF term rides in every feature-tile trip of the RFF loop (a fused stream). Why fused:
+    // the RFF loop alone saturates the MUFU pipe (ncu source view: 16 cosines per 129.7 cycles of a sub-partition =
+    // 99 %), the RBF loop alone needs the FP32 pipe and the MUFU pipe for 40 cycles each per inducing point and reaches
+    // 65 % of either, and a warp issues in order -- only a stream that carries MUFU work everywhere keeps that pipe fed
+    // (tools/pipe_probe.cu: FFMA2 and MUFU do overlap when both are on offer). Measured against the two parts one after
+    // the other, D = 5, M = 100, 1e6 rows: evaluation 0.528 -> 0.516 ms, RK4 step 2.123 -> 2.021 ms, bit-identical
     // results (the sums run in the same order); XU pipe 83 % of the active cycles (profiles/r02_summary.md).
-    const bool stagger = mode == 2;
     auto rbf_compute = [&](const float (&kp_)[KS]) {
         float dd[D];
 #pragma unroll
@@ -435,131 +389,71 @@ __device__ __forceinline__ void vf_eval_h(const float* __restrict__ small, const
         lds_vec<KS>(kp_, kern + m * KS);
         rbf_compute(kp_);
     };
-    if (mode == 0) {
-        uint32_t ax[2][4];
-        auto slotA = [&](const int row, const int s) -> float {  // x_hi | x_hi | x_lo | 0
-            const int kind = s / D, j = s - kind * D;
-            const float v = kind < 3 ? sx[row * SXS + j] : 0.f;
-            const float hi = gpode_trunc11(v);
-            return kind == 2 ? v - hi : hi;
-        };
+    uint32_t ax[2][4];
+    auto slotA = [&](const int row, const int s) -> float {  // x_hi | x_hi | x_lo | 0
+        const int kind = s / D, j = s - kind * D;
+        const float v = kind < 3 ? sx[row * SXS + j] : 0.f;
+        const float hi = gpode_trunc11(v);
+        return kind == 2 ? v - hi : hi;
+    };
 #pragma unroll
-        for (int mt = 0; mt < 2; ++mt) {
-            const int r0 = 16 * mt + g, r1 = r0 + 8;
-            ax[mt][0] = gpode_pack_h2(slotA(r0, 2 * t), slotA(r0, 2 * t + 1));
-            ax[mt][1] = gpode_pack_h2(slotA(r1, 2 * t), slotA(r1, 2 * t + 1));
-            ax[mt][2] = gpode_pack_h2(slotA(r0, 2 * t + 8), slotA(r0, 2 * t + 9));
-            ax[mt][3] = gpode_pack_h2(slotA(r1, 2 * t + 8), slotA(r1, 2 * t + 9));
-        }
-        int m = 0;
+    for (int mt = 0; mt < 2; ++mt) {
+        const int r0 = 16 * mt + g, r1 = r0 + 8;
+        ax[mt][0] = gpode_pack_h2(slotA(r0, 2 * t), slotA(r0, 2 * t + 1));
+        ax[mt][1] = gpode_pack_h2(slotA(r1, 2 * t), slotA(r1, 2 * t + 1));
+        ax[mt][2] = gpode_pack_h2(slotA(r0, 2 * t + 8), slotA(r0, 2 * t + 9));
+        ax[mt][3] = gpode_pack_h2(slotA(r1, 2 * t + 8), slotA(r1, 2 * t + 9));
+    }
+    int m = 0;
 #pragma unroll 1
-        for (int k = 0; k < D; ++k) {
-            float fk[4] = {0.f, 0.f, 0.f, 0.f};
-            const uint32_t* __restrict__ rc = mmah + (size_t)k * S8P * GPODE_MMAH_REC;
-            const int n_fused = M - m < S8P ? M - m : S8P;   // tiles of this output that carry an inducing point
-            int ft = 0;
+    for (int k = 0; k < D; ++k) {
+        float fk[4] = {0.f, 0.f, 0.f, 0.f};
+        const uint32_t* __restrict__ rc = mmah + (size_t)k * S8P * GPODE_MMAH_REC;
+        const int n_fused = M - m < S8P ? M - m : S8P;   // tiles of this output that carry an inducing point
+        int ft = 0;
 #pragma unroll 2
-            for (; ft < n_fused; ++ft, rc += GPODE_MMAH_REC, ++m) {   // branch-free body: one scheduling region
-                const uint2 b = *reinterpret_cast<const uint2*>(rc + lane * 2);
-                const float4 ph = *reinterpret_cast<const float4*>(rc + 64 + t * 4);
-                const float2 a2 = *reinterpret_cast<const float2*>(rc + 144 + t * 2);
-                float c[2][4];
-                gpode_mma_f16(c[0], ax[0], b.x, b.y, ph);
-                gpode_mma_f16(c[1], ax[1], b.x, b.y, ph);
-                rbf_step(m);
-#pragma unroll
-                for (int mt = 0; mt < 2; ++mt) {
-                    fk[2 * mt] = fmaf(a2.x, __cosf(c[mt][0]), fk[2 * mt]);
-                    fk[2 * mt] = fmaf(a2.y, __cosf(c[mt][1]), fk[2 * mt]);
-                    fk[2 * mt + 1] = fmaf(a2.x, __cosf(c[mt][2]), fk[2 * mt + 1]);
-                    fk[2 * mt + 1] = fmaf(a2.y, __cosf(c[mt][3]), fk[2 * mt + 1]);
-                }
-            }
-#pragma unroll 2
-            for (; ft < S8P; ++ft, rc += GPODE_MMAH_REC) {
-                const uint2 b = *reinterpret_cast<const uint2*>(rc + lane * 2);
-                const float4 ph = *reinterpret_cast<const float4*>(rc + 64 + t * 4);
-                const float2 a2 = *reinterpret_cast<const float2*>(rc + 144 + t * 2);
-                float c[2][4];
-                gpode_mma_f16(c[0], ax[0], b.x, b.y, ph);
-                gpode_mma_f16(c[1], ax[1], b.x, b.y, ph);
-#pragma unroll
-                for (int mt = 0; mt < 2; ++mt) {
-                    fk[2 * mt] = fmaf(a2.x, __cosf(c[mt][0]), fk[2 * mt]);
-                    fk[2 * mt] = fmaf(a2.y, __cosf(c[mt][1]), fk[2 * mt]);
-                    fk[2 * mt + 1] = fmaf(a2.x, __cosf(c[mt][2]), fk[2 * mt + 1]);
-                    fk[2 * mt + 1] = fmaf(a2.y, __cosf(c[mt][3]), fk[2 * mt + 1]);
-                }
-            }
-#pragma unroll
-            for (int r = 0; r < 4; ++r) {
-                float v = fk[r];
-                v += __shfl_xor_sync(0xffffffffu, v, 1);
-                v += __shfl_xor_sync(0xffffffffu, v, 2);
-                if (r == t) sxb[(g + 8 * r) * 8 + k] = v;
-            }
-        }
-#pragma unroll 1
-        for (; m < M; ++m) rbf_step(m);   // more inducing points than feature tiles
-    } else {
-    const int warp_id = threadIdx.x >> 5;
-    const bool rbf_first = stagger && ((warp_id ^ (warp_id >> 2)) & 1) != 0;
-#pragma unroll 1
-    for (int part = 0; part < 2; ++part) {
-        if ((part == 0) != rbf_first) {
-        {
-            uint32_t ax[2][4];
-            auto slotA = [&](const int row, const int s) -> float {  // x_hi | x_hi | x_lo | 0
-                const int kind = s / D, j = s - kind * D;
-                const float v = kind < 3 ? sx[row * SXS + j] : 0.f;
-                const float hi = gpode_trunc11(v);
-                return kind == 2 ? v - hi : hi;
-            };
+        for (; ft < n_fused; ++ft, rc += GPODE_MMAH_REC, ++m) {   // branch-free body: one scheduling region
+            const uint2 b = *reinterpret_cast<const uint2*>(rc + lane * 2);
+            const float4 ph = *reinterpret_cast<const float4*>(rc + 64 + t * 4);
+            const float2 a2 = *reinterpret_cast<const float2*>(rc + 144 + t * 2);
+            float c[2][4];
+            gpode_mma_f16(c[0], ax[0], b.x, b.y, ph);
+            gpode_mma_f16(c[1], ax[1], b.x, b.y, ph);
+            rbf_step(m);
 #pragma unroll
             for (int mt = 0; mt < 2; ++mt) {
-                const int r0 = 16 * mt + g, r1 = r0 + 8;
-                ax[mt][0] = gpode_pack_h2(slotA(r0, 2 * t), slotA(r0, 2 * t + 1));
-                ax[mt][1] = gpode_pack_h2(slotA(r1, 2 * t), slotA(r1, 2 * t + 1));
-                ax[mt][2] = gpode_pack_h2(slotA(r0, 2 * t + 8), slotA(r0, 2 * t + 9));
-                ax[mt][3] = gpode_pack_h2(slotA(r1, 2 * t + 8), slotA(r1, 2 * t + 9));
+                fk[2 * mt] = fmaf(a2.x, __cosf(c[mt][0]), fk[2 * mt]);
+                fk[2 * mt] = fmaf(a2.y, __cosf(c[mt][1]), fk[2 * mt]);
+                fk[2 * mt + 1] = fmaf(a2.x, __cosf(c[mt][2]), fk[2 * mt + 1]);
+                fk[2 * mt + 1] = fmaf(a2.y, __cosf(c[mt][3]), fk[2 * mt + 1]);
             }
+        }
+#pragma unroll 2
+        for (; ft < S8P; ++ft, rc += GPODE_MMAH_REC) {
+            const uint2 b = *reinterpret_cast<const uint2*>(rc + lane * 2);
+            const float4 ph = *reinterpret_cast<const float4*>(rc + 64 + t * 4);
+            const float2 a2 = *reinterpret_cast<const float2*>(rc + 144 + t * 2);
+            float c[2][4];
+            gpode_mma_f16(c[0], ax[0], b.x, b.y, ph);
+            gpode_mma_f16(c[1], ax[1], b.x, b.y, ph);
+#pragma unroll
+            for (int mt = 0; mt < 2; ++mt) {
+                fk[2 * mt] = fmaf(a2.x, __cosf(c[mt][0]), fk[2 * mt]);
+                fk[2 * mt] = fmaf(a2.y, __cosf(c[mt][1]), fk[2 * mt]);
+                fk[2 * mt + 1] = fmaf(a2.x, __cosf(c[mt][2]), fk[2 * mt + 1]);
+                fk[2 * mt + 1] = fmaf(a2.y, __cosf(c[mt][3]), fk[2 * mt + 1]);
+            }
+        }
+#pragma unroll
+        for (int r = 0; r < 4; ++r) {
+            float v = fk[r];
+            v += __shfl_xor_sync(0xffffffffu, v, 1);
+            v += __shfl_xor_sync(0xffffffffu, v, 2);
+            if (r == t) sxb[(g + 8 * r) * 8 + k] = v;
+        }
+    }
 #pragma unroll 1
-            for (int k = 0; k < D; ++k) {
-                float fk[4] = {0.f, 0.f, 0.f, 0.f};  // rows g, g+8, g+16, g+24; this lane's features 2t, 2t+1 of every tile
-                const uint32_t* __restrict__ rc = mmah + (size_t)k * S8P * GPODE_MMAH_REC;
-#pragma unroll 2
-                for (int ft = 0; ft < S8P; ++ft, rc += GPODE_MMAH_REC) {
-                    const uint2 b = *reinterpret_cast<const uint2*>(rc + lane * 2);
-                    const float4 ph = *reinterpret_cast<const float4*>(rc + 64 + t * 4);
-                    const float2 a2 = *reinterpret_cast<const float2*>(rc + 144 + t * 2);
-                    float c[2][4];
-                    gpode_mma_f16(c[0], ax[0], b.x, b.y, ph);
-                    gpode_mma_f16(c[1], ax[1], b.x, b.y, ph);
-#pragma unroll
-                    for (int mt = 0; mt < 2; ++mt) {
-                        fk[2 * mt] = fmaf(a2.x, __cosf(c[mt][0]), fk[2 * mt]);
-                        fk[2 * mt] = fmaf(a2.y, __cosf(c[mt][1]), fk[2 * mt]);
-                        fk[2 * mt + 1] = fmaf(a2.x, __cosf(c[mt][2]), fk[2 * mt + 1]);
-                        fk[2 * mt + 1] = fmaf(a2.y, __cosf(c[mt][3]), fk[2 * mt + 1]);
-                    }
-                }
-#pragma unroll
-                for (int r = 0; r < 4; ++r) {
-                    float v = fk[r];
-                    v += __shfl_xor_sync(0xffffffffu, v, 1);
-                    v += __shfl_xor_sync(0xffffffffu, v, 2);
-                    if (r == t) sxb[(g + 8 * r) * 8 + k] = v;
-                }
-            }
-        }
-        } else {
-        {
-#pragma unroll 2
-        for (int m = 0; m < M; ++m) rbf_step(m);
-        }
-        }
-    }
-    }
+    for (; m < M; ++m) rbf_step(m);   // more inducing points than feature tiles
     __syncwarp();
 #pragma unroll
     for (int k = 0; k < D; ++k) {

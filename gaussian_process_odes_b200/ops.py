@@ -464,31 +464,6 @@ MAX_D_REGISTER = 8    # GPODE_MAX_D: differentiable register-resident kernels
 MAX_D_LARGE = 64      # GPODE_MAX_D_LARGE: tcgen05 forward + large-D VJP kernels (rk4 and dopri5 differentiable)
 
 
-def _large_d_call(name, x, t, Z, ell, var, nu, omega, phase, w):
-    """Forward-only evaluation / integration for 8 < D <= 64 on the raw cache tensors."""
-    tensors = (x, Z, ell, var, nu)
-    if torch.is_grad_enabled() and any(a.requires_grad for a in tensors):
-        raise _lib.GpodeError("state dimension %d > %d: only the forward (no_grad) path exists for large D"
-                              % (Z.shape[1], MAX_D_REGISTER))
-    Zc, ec, vc, oc, wc, xc = f32(Z, "Z"), f32(ell, "ell"), f32(var, "var"), f32(omega, "omega"), f32(w, "w"), f32(x, "x")
-    M, D = Zc.shape
-    S = wc.shape[0]
-    pc_, nc = f32(phase, "phase").reshape(S, D), f32(nu, "nu").reshape(D, M)
-    st = _cache_struct(D, M, S, oc, pc_, wc, Zc, nc, ec, vc)
-    B = xc.shape[0]
-    if name == "gpode_vf_fwd_large":
-        out = torch.empty_like(xc)
-        _lib.call(name, ctypes.byref(st), ptr(xc), ptr(out), B, stream_ptr())
-    else:
-        tc = f32(t, "t")
-        out = torch.empty(tc.shape[0], B, D, dtype=torch.float32, device=xc.device)
-        _lib.call(name, ctypes.byref(st), ptr(xc), ptr(tc), tc.shape[0], B, ptr(out), stream_ptr())
-    return out
-
-
-LARGE_RBF_TENSOR_CORES = True   # False: RBF term in the FP32 tiled kernel (gpode_vf_fwd_large_add_rbf)
-
-
 class LargeField:
     """One sampled GP function for 8 < D <= 64: the Fourier-feature term runs on the tcgen05 tensor cores
     (``gpode_rff_fwd_large`` over the pre-tiled 3xTF32 operand chunks of ``gpode_pack_cache_large``), the RBF term as
@@ -543,7 +518,7 @@ class LargeField:
         f_rff = torch.empty_like(xc)
         _lib.call("gpode_rff_fwd_large", ptr(self.packed), self.D, self.S, ptr(xc), ptr(f_rff), B, stream_ptr())
         f = torch.empty_like(xc)
-        if LARGE_RBF_TENSOR_CORES and self.rbf_on_tensor_cores:
+        if self.rbf_on_tensor_cores:
             try:
                 _lib.call("gpode_rbf_fwd_large", ptr(self.packed), self.D, self.M, self.S, ptr(self.keep[0]), ptr(xc),
                           ptr(f_rff), ptr(f), B, stream_ptr())
@@ -945,14 +920,3 @@ def integrate_sets(x0, t, Z, ell, var, nu, omega, phase, w, method="dopri5", rto
         raise _lib.GpodeError("integrate_sets: method %r has no fused CUDA integrator (rk4, dopri5)" % (method,))
     return xs.view(Tg, pcs.n, N, pcs.D).permute(1, 2, 0, 3), stats
 
-
-def vector_field_umma(x, Z, ell, var, nu, omega, phase, w):
-    """EXPERIMENTAL, forward only, 2 <= D <= 7: ``vector_field`` with the Fourier-feature projection on the tcgen05
-    tensor cores (``gpode_vf_fwd_umma``: 3xTF32 in TMEM accumulators)."""
-    pc = PackedCache(Z, ell, var, nu, omega, phase, w)
-    xc = f32(x, "x")
-    if xc.ndim != 2 or xc.shape[1] != pc.D:
-        raise _lib.GpodeError("x must be (B,%d), got %s" % (pc.D, tuple(xc.shape)))
-    f = torch.empty_like(xc)
-    _lib.call("gpode_vf_fwd_umma", ptr(pc.packed), pc.D, pc.M, pc.S, ptr(xc), ptr(f), xc.shape[0], stream_ptr())
-    return f

@@ -26,9 +26,9 @@
 extern "C" {
 #endif
 
-#define GPODE_B200_ABI_VERSION 1
+#define GPODE_B200_ABI_VERSION 2
 #define GPODE_MAX_D 8          /* register-resident state kernels are instantiated for 1 <= D <= 8 */
-#define GPODE_MAX_D_LARGE 64   /* forward-only shared-memory-tile kernels cover 8 < D <= 64 */
+#define GPODE_MAX_D_LARGE 64   /* the large-D kernels (tcgen05 forward, large-D VJP) cover 8 < D <= 64 */
 #define GPODE_MAX_M_F64 112    /* whitening backward keeps two MxM float64 tiles in shared memory */
 #define GPODE_MAX_M 160        /* ... and falls back to float32 tiles up to this M */
 
@@ -162,15 +162,11 @@ int gpode_param_grad_dev(const float* packed, int D, int M, int S, const float* 
                          int64_t n_rows_max, const int32_t* stats_dev, int64_t rows_per_step, float* acc,
                          void* stream);
 
-/* Forward-only paths for 8 < D <= GPODE_MAX_D_LARGE (the upper half of the scaling sweep): same arithmetic as
- * gpode_vf_fwd / gpode_rk4_fwd, state tiles in shared memory, Omega streamed from L2; they take the RAW cache. */
-int gpode_vf_fwd_large(const gpode_cache_t* cache, const float* x, float* f, int64_t B, void* stream);
-int gpode_rk4_fwd_large(const gpode_cache_t* cache, const float* x0, const float* t, int Tg, int64_t B, float* xs,
-                        void* stream);
-
-/* Tensor-core route for the same sizes: the Fourier-feature term as tcgen05 kind::tf32 GEMMs (3xTF32, TMEM
- * accumulators) over operand chunks pre-tiled by gpode_pack_cache_large (gpode_packed_large_floats(D,M,S) floats) and
- * streamed from L2 through a shared-memory ring; gpode_vf_fwd_large_add_rbf adds the RBF term: f = f_rff + K(x,Z) nu. */
+/* Vector field for 8 < D <= GPODE_MAX_D_LARGE (the upper half of the scaling sweep): the Fourier-feature term as
+ * tcgen05 kind::tf32 GEMMs (3xTF32, TMEM accumulators) over operand chunks pre-tiled by gpode_pack_cache_large
+ * (gpode_packed_large_floats(D,M,S) floats) and streamed from L2 through a shared-memory ring;
+ * gpode_vf_fwd_large_add_rbf adds the RBF term on the FP32 CUDA cores (state tiles in shared memory, RAW cache):
+ * f = f_rff + K(x,Z) nu. */
 int64_t gpode_packed_large_floats(int D, int M, int S);
 int gpode_pack_cache_large(const gpode_cache_t* cache, float* packed_large, void* stream);
 int gpode_rff_fwd_large(const float* packed_large, int D, int S, const float* x, float* f_rff, int64_t B, void* stream);
@@ -237,10 +233,11 @@ int gpode_constraint_sum(const float* ss, const float* pred, const float* scale,
 
 /* Differentiable path for 8 < D <= GPODE_MAX_D_LARGE (autograd through src/core/dsvgp.py:172-197 at the upper sweep
  * dimensions; round 1 was forward-only there). Everything is stream-ordered on the device -- no host loop reads a value.
- *   gpode_pack_cache_large_bwd: Omega re-tiled per (output k, 64-feature chunk) with the input dimension contiguous, plus
- *     w_kj = 0.5 log2(e)/ell_kj^2, Z and c_km = var_k nu_km, padded to DP = 16 / 32 / 64
- *     (gpode_packed_large_bwd_floats(D,M,S) floats).
- *   gpode_vf_bwd_large: grad_x = J(x)^T grad_f and the partial sums of every shared-parameter gradient, ADDED to the
+ *   gpode_pack_cache_large_bwd: w_kj = 0.5 log2(e)/ell_kj^2, Z and c_km = var_k nu_km, padded to DP = 16 / 32 / 64,
+ *     then the 3xTF32 operand chunks of the tensor-core Fourier-feature half (gpode_packed_large_bwd_floats(D,M,S)
+ *     floats).
+ *   gpode_vf_bwd_large: grad_x = J(x)^T grad_f (Fourier-feature half on the tcgen05 tensor cores, RBF half on the
+ *     FP32 CUDA cores) and the partial sums of every shared-parameter gradient, ADDED to the
  *     calling launch's per-CTA rows of acc_large (gpode_acc_large_floats(D,M) floats, zeroed by the caller before the
  *     first launch of a backward pass; all launches of one pass must use the same B). f = the forward value at x.
  *   gpode_grads_finalize_large: rows -> grad_ell [D,D], grad_var [D], grad_Z [M,D], grad_nu [D,M] (float64, row order).
@@ -326,28 +323,14 @@ int gpode_shoot_bwd(const float* packed, int D, int M, int S, const gpode_shoot_
                     const float* kstages, const float* seeds, const float* g_ll, const float* g_cons, float* grad_ss,
                     float* vrows, float* acc, void* stream);
 
-/* Kernel-selection options (tuning / ablation; the library's only process-wide mutable state). Defaults are read from
- * the environment once (GPODE_BWD_MMA, GPODE_FWD_MMA, GPODE_MMA_PARTS, GPODE_FORCE_NARROW, GPODE_USE_MMA); names:
+/* Kernel-selection options (the library's only process-wide mutable state). Defaults are read from the environment
+ * once (GPODE_BWD_MMA, GPODE_FWD_MMA); names:
  *   "bwd_mma" / "fwd_mma" (1): tensor-core adjoint / forward at D = 4, 5 and B >= SMs x 384 rows; 0 = FFMA2 kernels.
  *       Domain of the split-fp16 operands: |x_j|, |Omega| < 65504 -- beyond it the kernels return NaN (fp16 overflow),
  *       never silently wrong numbers; a float32 angle of that size carries no phase information anyway.
- *   "mma_parts" (3): ablation mask of the tensor-core adjoint (anything else gives wrong gradients; timing only)
- *   "force_narrow" (0): FFMA2 kernels with one row per thread;  "use_mma" (0): the 3xTF32 forward experiment. */
+ * Any other name is an error (-1). */
 int gpode_set_option(const char* name, int value);
 int gpode_get_option(const char* name);
-
-/* gpode_vf_bwd with both Fourier projections of the VJP on the tcgen05 tensor cores (D = 4, 5): theta as a kind::f16
- * split GEMM from shared memory, sin(theta) written back to tensor memory as the A operand of the second GEMM
- * (G = sin(theta) (a Omega)^T, kind::tf32, TS form); csrc/vjp_umma.cu. packed_ubwd: its operand block
- * (gpode_packed_ubwd_floats(D,S) floats, gpode_pack_cache_ubwd). Same outputs as gpode_vf_bwd. */
-int64_t gpode_packed_ubwd_floats(int D, int S);
-int gpode_pack_cache_ubwd(const gpode_cache_t* cache, float* packed_ubwd, void* stream);
-int gpode_vf_bwd_umma(const float* packed, const float* packed_ubwd, int D, int M, int S, const float* x, const float* f,
-                      const float* grad_f, float* grad_x, float* acc, int64_t B, void* stream);
-
-/* EXPERIMENTAL (2 <= D <= 7): gpode_vf_fwd with the Fourier-feature projection on the 5th-generation tensor cores
- * (tcgen05.mma kind::tf32, 3xTF32 error compensation, accumulators in TMEM); same arguments and results. */
-int gpode_vf_fwd_umma(const float* packed, int D, int M, int S, const float* x, float* f, int64_t B, void* stream);
 
 /* Measurement utility (no reference counterpart): sustained FP32 FMA throughput of the current device in TFLOP/s
  * (best of 5 launches of a register-only FMA loop; synchronises the stream). scratch: >= 1 float (device). */

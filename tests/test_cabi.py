@@ -23,19 +23,18 @@ def test_library_builds_loads_and_exports_header_symbols():
         assert hasattr(lib, n), "libgpode_b200.so does not export %s" % n
     # the ctypes binding covers exactly the header
     assert sorted(_lib.SIGNATURES) == names
-    assert _lib.load().gpode_abi_version() == 1
+    assert _lib.load().gpode_abi_version() == 2
 
 
 def test_pure_host_entry_points():
     from gaussian_process_odes_b200 import _lib
     lib = _lib.load()
     # layout arithmetic only: rff D*roundup32(S/2)*roundup4(2D+4) + kern M*roundup4(D+2*ceil(D/2)) + w D*roundup4(2*ceil(D/2))
-    # + mma.sync tf32 operand blocks D*ceil(S/8)*80 + f16 adjoint operand blocks D*roundup2(ceil(S/8))*152 (D <= 5)
-    # + tcgen05 operand blocks D*17*roundup32(S) (D <= 7)
-    assert lib.gpode_packed_floats(2, 16, 256) == 2 * 128 * 8 + 16 * 4 + 2 * 4 + 2 * 32 * (80 + 152) + 2 * 17 * 256
-    assert lib.gpode_packed_floats(5, 100, 256) == 5 * 128 * 16 + 100 * 12 + 5 * 8 + 5 * 32 * (80 + 152) + 5 * 17 * 256
-    assert lib.gpode_packed_floats(3, 24, 64) == 3 * 32 * 12 + 24 * 8 + 3 * 4 + 3 * 8 * (80 + 152) + 3 * 17 * 64
-    assert lib.gpode_packed_floats(8, 10, 40) == 8 * 32 * 20 + 10 * 16 + 8 * 8 + 8 * 5 * 80
+    # + f16 tensor-core operand blocks D*roundup2(ceil(S/8))*152 (D <= 5)
+    assert lib.gpode_packed_floats(2, 16, 256) == 2 * 128 * 8 + 16 * 4 + 2 * 4 + 2 * 32 * 152
+    assert lib.gpode_packed_floats(5, 100, 256) == 5 * 128 * 16 + 100 * 12 + 5 * 8 + 5 * 32 * 152
+    assert lib.gpode_packed_floats(3, 24, 64) == 3 * 32 * 12 + 24 * 8 + 3 * 4 + 3 * 8 * 152
+    assert lib.gpode_packed_floats(8, 10, 40) == 8 * 32 * 20 + 10 * 16 + 8 * 8
     assert lib.gpode_packed_floats(0, 1, 1) == -1
     # header | 4096 adjoint-CTA rows of A[D,D] | V[D] | 1024 param-grad-CTA rows of M x {T[k], W[j,k]}
     assert lib.gpode_acc_header_floats() == 4
@@ -48,6 +47,9 @@ def test_pure_host_entry_points():
     assert rc < 0 and b"NULL" in lib.gpode_last_error()
     rc = lib.gpode_rk4_fwd(ctypes.c_void_p(16), 9, 16, 256, None, None, 2, 4, None, None, None)
     assert rc < 0 and b"dimension" in lib.gpode_last_error()
+    # the kernel-selection options are bwd_mma and fwd_mma; any other name is rejected
+    assert lib.gpode_set_option(b"use_mma", 1) == -1 and b"unknown option" in lib.gpode_last_error()
+    assert lib.gpode_get_option(b"bwd_mma") in (0, 1) and lib.gpode_get_option(b"fwd_mma") in (0, 1)
 
 
 def test_kernels_have_no_register_spills_on_the_config_shapes():

@@ -176,22 +176,17 @@ def test_rk4_forward(D, M, S, B, Tg, h):
                                       (24, 7, 33, 64), (64, 150, 64, 130), (41, 30, 200, 257)])
 def test_large_state_dimension_forward(D, M, S, B):
     """8 < D <= 64 (upper half of the scaling sweep): tensor-core forward kernels, same parity bars."""
-    from gaussian_process_odes_b200 import ops, _lib
+    from gaussian_process_odes_b200 import ops
     gp32, c32, gp64, c64, x = _setup(D, M, S, B, seed=D, nu_scale=0.1)
     args = _cuda_args(gp32, c32)
     with torch.no_grad():
         f = ops.vector_field(x.cuda(), *args).cpu()
         ts = _grid(4, 0.02, 2)
         xs = ops.rk4_integrate(x.cuda(), ts.cuda(), *args).cpu()
-        # the all-FP32 tiled kernels (the tensor-core route's predecessor, still exported)
-        f_fma = ops._large_d_call("gpode_vf_fwd_large", x.cuda(), None, *args).cpu()
-        xs_fma = ops._large_d_call("gpode_rk4_fwd_large", x.cuda(), ts.cuda(), *args).cpu()
     f32 = O.vf_forward(x, gp32['Z'], gp32['ell'], gp32['var'], c32)
     c64n = dict(c64, nu=c32['nu'].double())
     f64 = O.vf_forward(x.double(), gp64['Z'], gp64['ell'], gp64['var'], c64n)
     assert_parity("large-D vf", f, f32, f64, TOL_VF)
-    assert_parity("large-D vf (fp32 tiles)", f_fma, f32, f64, TOL_VF)
-    assert relerr(xs_fma, xs) <= TOL_TRAJ
     ref32 = O.odeint(lambda t, y: O.vf_forward(y, gp32['Z'], gp32['ell'], gp32['var'], c32), x, ts, method='rk4')
     assert relerr(xs, ref32) <= TOL_TRAJ
 
@@ -247,30 +242,6 @@ def test_large_state_dimension_backward(D, M, S, B):
     ops.rk4_integrate(xc2, ts.cuda(), *args2).backward(cot3.cuda())
     assert torch.equal(xc2.grad, xc.grad) and torch.equal(args2[0].grad, args[0].grad)
     assert torch.equal(args2[1].grad, args[1].grad) and torch.equal(args2[3].grad, args[3].grad)
-
-
-@pytest.mark.parametrize("D,M,S,B", [(16, 100, 256, 1000), (41, 30, 200, 257), (64, 30, 64, 130)])
-def test_large_state_dimension_vjp_tensor_core_vs_fp32(D, M, S, B):
-    """The Fourier half of the large-D VJP on tcgen05 (csrc/large_rffb.cu, default) against the FP32 CUDA-core form
-    (option large_bwd_umma = 0): same row cotangent and parameter gradients to the 3xTF32 split's accuracy (2^-21 per
-    product, measured 2.6e-6 on the row cotangent; the gradient gate itself is 1e-4); ragged sizes (rows not a multiple
-    of 128, S not a multiple of 64, D not a multiple of 16)."""
-    from gaussian_process_odes_b200 import ops, _lib
-    gp32, c32, gp64, c64, x = _setup(D, M, S, B, seed=D + 3, nu_scale=0.1)
-    cot = torch.tensor(np.random.default_rng(9).normal(size=(B, D)), dtype=torch.float32)
-    res = {}
-    try:
-        for u in (1, 0, 2):   # 2: tcgen05 RFF half + the four-warp form of the RBF half (1 runs it on eight warps at D > 32)
-            _lib.set_option("large_bwd_umma", u)
-            args = [a.detach().clone().requires_grad_(i < 4) for i, a in enumerate(_cuda_args(gp32, c32))]
-            xc = x.cuda().requires_grad_(True)
-            ops.vector_field(xc, *args).backward(cot.cuda())
-            res[u] = dict(x=xc.grad, Z=args[0].grad, ell=args[1].grad, var=args[2].grad, nu=args[3].grad)
-    finally:
-        _lib.set_option("large_bwd_umma", 1)
-    for k in res[1]:
-        assert relerr(res[1][k].cpu(), res[0][k].cpu()) <= 1e-5, (k, relerr(res[1][k].cpu(), res[0][k].cpu()))
-        assert relerr(res[1][k].cpu(), res[2][k].cpu()) <= 2e-6, (k, relerr(res[1][k].cpu(), res[2][k].cpu()))
 
 
 @pytest.mark.parametrize("D,M,S,B", [(16, 100, 256, 300), (33, 20, 64, 40)])
@@ -498,15 +469,6 @@ def test_forward_tensor_core_path(D, M, S, B, monkeypatch):
     assert relerr(f1, f0) <= TOL_VF and relerr(f1, f32) <= TOL_VF
     assert relerr(xs1, xs0) <= TOL_TRAJ and relerr(xs1, out) <= TOL_TRAJ
     assert torch.equal(xs1[0], x)
-    # the schedule variants of the tensor-core evaluation (mma_parts bits 2-3: fused stream = default, two parts, two
-    # parts staggered across warps) run the same sums in the same order: bit-identical results
-    try:
-        for parts in (7, 11):
-            _lib.set_option("mma_parts", parts)
-            fv, xsv = run("1")
-            assert torch.equal(fv, f1) and torch.equal(xsv, xs1), parts
-    finally:
-        _lib.set_option("mma_parts", 3)
     # outside the split-fp16 domain (|x| >= 65504) the tensor-core kernels answer NaN, never a wrong finite number
     if D == 5 and B == 60000:
         xbad = x.clone()

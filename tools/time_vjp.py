@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Time one vector-field VJP (B = 1e6) for the adjoint variants (tuning helper)."""
+"""Time one vector-field VJP (B = 1e6) with the tensor-core and the FFMA2 adjoint (tuning helper)."""
 import json
 import os
 import sys
@@ -27,10 +27,8 @@ pc = ops.PackedCache(*args)
 f = ops.vector_field(x, *args)
 gx = torch.empty_like(x)
 ptr = ops.ptr
-VARIANTS = [v.split(":") for v in os.environ.get("TV_VARIANTS", "0:3,1:3,1:1,1:2,1:0").split(",")]
-for mode, parts in VARIANTS:
+for mode in os.environ.get("TV_VARIANTS", "0,1").split(","):
     _lib.set_option("bwd_mma", int(mode))
-    _lib.set_option("mma_parts", int(parts))
     acc = pc.new_acc()
     def run():
         _lib.call("gpode_vf_bwd", ptr(pc.packed), pc.D, pc.M, pc.S, ptr(x), ptr(f), ptr(gf), ptr(gx), ptr(acc),
@@ -44,4 +42,4 @@ for mode, parts in VARIANTS:
         run()
     e1.record()
     torch.cuda.synchronize()
-    print(json.dumps(dict(D=D, mma=mode, parts=parts, vjp_ms=round(e0.elapsed_time(e1) / 10, 4))), flush=True)
+    print(json.dumps(dict(D=D, mma=mode, vjp_ms=round(e0.elapsed_time(e1) / 10, 4))), flush=True)

@@ -91,6 +91,11 @@ SIGNATURES = {
     "gpode_vf_fwd_sets": (_I, [_P, _I, _I, _I, _I, _L, _P, _P, _P]),
     "gpode_rk4_fwd_sets": (_I, [_P, _I, _I, _I, _I, _L, _P, _P, _I, _P, _P]),
     "gpode_dopri5_fwd_sets": (_I, [_P, _I, _I, _I, _I, _L, _P, _P, _I, _D, _D, _P, _P, _P, _P]),
+    "gpode_pack_cache_large_sets": (_I, [_CP, _I, _P, _P]),
+    "gpode_vf_fwd_large_sets": (_I, [_P, _CP, _I, _L, _P, _P, _P, _P]),
+    "gpode_rk4_fwd_large_sets": (_I, [_P, _CP, _I, _L, _P, _P, _I, _P, _P, _P]),
+    "gpode_dopri5_large_sets_work_floats": (_L, [_I, _I, _L]),
+    "gpode_dopri5_fwd_large_sets": (_I, [_P, _CP, _I, _L, _P, _P, _I, _D, _D, _P, _P, _P, _I, _P]),
 }
 
 _lib = None
@@ -174,6 +179,9 @@ KERNELS_PER_CALL = {
     "gpode_rk4_fwd_large_dev": 12, "gpode_rk4_bwd_large": 16,
     # start: 2 evaluations (2 kernels each) + 6 small kernels; every attempt of the device-side loop launches 21 more
     "gpode_dopri5_fwd_large": 10 + 21, "gpode_dopri5_fwd_large_ckpt": 10 + 21,
+    # batched prediction above D = 8: the same counts, all draws in each launch; dopri5 adds the "any draw left" kernel
+    "gpode_pack_cache_large_sets": 1, "gpode_vf_fwd_large_sets": 2, "gpode_rk4_fwd_large_sets": 12,
+    "gpode_dopri5_fwd_large_sets": 10 + 22,
     # per accepted step: 6 VJPs (2 kernels each) + 7 element-wise kernels; once: the VJP at x0 + the grad_x0 kernel
     "gpode_dopri5_bwd_large": 19 + 3,
 }

@@ -47,6 +47,21 @@ enum { GPODE_OPT_BWD_MMA = 0, GPODE_OPT_FWD_MMA, GPODE_OPT_COUNT };
 int gpode_option(int which);  // pack.cu
 
 // ------------------------------------------------------------------------------------------------------------------
+// draw indexing of the large-D vector field (8 < D <= 64; batched Monte-Carlo prediction). n draws of `rows` rows each,
+// laid out [n * rows, D]; draw q's packed block starts at packed + q * stride and its nu at nu + q * D * M. A tile never
+// straddles two draws: draw q owns tiles [q * ceil(rows / TR), (q + 1) * ceil(rows / TR)) and its first tile starts at
+// its row 0. done: NULL, or a per-draw flag (done[q * done_stride] != 0) read at the start of each tile -- a finished
+// draw's tiles are skipped. One draw without flags ({1, B, 0, NULL, 0}) is the single-function evaluation.
+// ------------------------------------------------------------------------------------------------------------------
+struct GpodeDraws {
+    int n;
+    int64_t rows, stride;
+    const int* done;
+    int done_stride;
+};
+inline GpodeDraws gpode_one_draw(int64_t B) { return GpodeDraws{1, B, 0, nullptr, 0}; }
+
+// ------------------------------------------------------------------------------------------------------------------
 // packed parameter block (what every integrator CTA stages into shared memory with one bulk copy). Records are laid
 // out for the packed dual-FP32 FMA of sm_100 (SASS FFMA2, PTX fma.rn.f32x2): two Fourier features / two output
 // dimensions sit side by side so that one 64-bit register pair feeds one FFMA2.

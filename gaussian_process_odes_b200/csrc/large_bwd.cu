@@ -22,7 +22,7 @@
 #include "../../include/gpode_b200.h"
 
 int gpode_vf_large_eval(const float* packed_large, const gpode_cache_t* c, const float* x, float* tmp, float* f,
-                        int64_t B, cudaStream_t st);  // large_umma.cu: f = vf(x) on the tcgen05 tensor cores
+                        const GpodeDraws& dr, cudaStream_t st);  // large_umma.cu: f = vf(x) on the tcgen05 tensor cores
 // large_rffb.cu: the RFF part of the VJP on the tcgen05 tensor cores (both projections as 3xTF32 GEMMs)
 int64_t gpode_rv_packed_floats(int D, int S);
 int64_t gpode_rv_acc_floats(int D);
@@ -880,15 +880,12 @@ extern "C" int gpode_grads_finalize_large(const gpode_cache_t* c, const float* a
     return 0;
 }
 
-// xs [Tg,B,D] (xs[0] = x0), kstages [Tg-1,4,B,D] or NULL; tmp: 2 B D floats (6 B D when kstages is NULL)
-extern "C" int gpode_rk4_fwd_large_dev(const float* packed_large, const gpode_cache_t* c, const float* x0, const float* t,
-                                       int Tg, int64_t B, float* xs, float* kstages, float* tmp, void* stream) {
-    if (int rc = lb_check(c)) return rc;
-    GPODE_CHECK_ARG(Tg >= 1 && B >= 0, "bad sizes Tg=%d B=%lld", Tg, (long long)B);
-    if (B == 0) return 0;
+// xs [Tg,B,D] (xs[0] = x0), kstages [Tg-1,4,B,D] or NULL; tmp: 2 B D floats (6 B D when kstages is NULL);
+// B = dr.n * dr.rows rows, draw q of the field integrating its own dr.rows of them
+static int rk4_fwd_large(const float* packed_large, const gpode_cache_t* c, const float* x0, const float* t, int Tg,
+                         float* xs, float* kstages, float* tmp, const GpodeDraws& dr, cudaStream_t st) {
     GPODE_CHECK_ARG(packed_large && x0 && t && xs && tmp, "NULL argument");
-    cudaStream_t st = (cudaStream_t)stream;
-    const int64_t n = B * c->D;
+    const int64_t n = dr.n * dr.rows * c->D;
     GPODE_CUDA(cudaMemcpyAsync(xs, x0, sizeof(float) * n, cudaMemcpyDeviceToDevice, st));
     float* ys = tmp;
     float* frff = tmp + n;
@@ -898,17 +895,37 @@ extern "C" int gpode_rk4_fwd_large_dev(const float* packed_large, const gpode_ca
         const float* y = xs + (int64_t)i * n;
         float* k = kstages ? kstages + (int64_t)i * 4 * n : kloc;
         float *k1 = k, *k2 = k + n, *k3 = k + 2 * n, *k4 = k + 3 * n;
-        if (int rc = gpode_vf_large_eval(packed_large, c, y, frff, k1, B, st)) return rc;
+        if (int rc = gpode_vf_large_eval(packed_large, c, y, frff, k1, dr, st)) return rc;
         rk4_stage_large_kernel<<<g, 256, 0, st>>>(2, t, i, y, k1, k2, k3, k4, ys, n);
-        if (int rc = gpode_vf_large_eval(packed_large, c, ys, frff, k2, B, st)) return rc;
+        if (int rc = gpode_vf_large_eval(packed_large, c, ys, frff, k2, dr, st)) return rc;
         rk4_stage_large_kernel<<<g, 256, 0, st>>>(3, t, i, y, k1, k2, k3, k4, ys, n);
-        if (int rc = gpode_vf_large_eval(packed_large, c, ys, frff, k3, B, st)) return rc;
+        if (int rc = gpode_vf_large_eval(packed_large, c, ys, frff, k3, dr, st)) return rc;
         rk4_stage_large_kernel<<<g, 256, 0, st>>>(4, t, i, y, k1, k2, k3, k4, ys, n);
-        if (int rc = gpode_vf_large_eval(packed_large, c, ys, frff, k4, B, st)) return rc;
+        if (int rc = gpode_vf_large_eval(packed_large, c, ys, frff, k4, dr, st)) return rc;
         rk4_stage_large_kernel<<<g, 256, 0, st>>>(5, t, i, y, k1, k2, k3, k4, xs + (int64_t)(i + 1) * n, n);
         GPODE_LAUNCH_CHECK();
     }
     return 0;
+}
+
+extern "C" int gpode_rk4_fwd_large_dev(const float* packed_large, const gpode_cache_t* c, const float* x0, const float* t,
+                                       int Tg, int64_t B, float* xs, float* kstages, float* tmp, void* stream) {
+    if (int rc = lb_check(c)) return rc;
+    GPODE_CHECK_ARG(Tg >= 1 && B >= 0, "bad sizes Tg=%d B=%lld", Tg, (long long)B);
+    if (B == 0) return 0;
+    return rk4_fwd_large(packed_large, c, x0, t, Tg, xs, kstages, tmp, gpode_one_draw(B), (cudaStream_t)stream);
+}
+
+// n_sets draws of the "sets" cache (packed by gpode_pack_cache_large_sets), each integrating its own set_rows rows;
+// xs [Tg, n_sets set_rows, D], tmp 6 n_sets set_rows D floats
+extern "C" int gpode_rk4_fwd_large_sets(const float* packed_large, const gpode_cache_t* c, int n_sets, int64_t set_rows,
+                                        const float* x0, const float* t, int Tg, float* xs, float* tmp, void* stream) {
+    if (int rc = lb_check(c)) return rc;
+    GPODE_CHECK_ARG(n_sets >= 1 && n_sets <= 65535 && set_rows >= 0 && Tg >= 1, "bad sizes n_sets=%d Tg=%d", n_sets,
+                    Tg);
+    if (set_rows == 0) return 0;
+    const GpodeDraws dr{n_sets, set_rows, gpode_packed_large_floats(c->D, c->M, c->S), nullptr, 0};
+    return rk4_fwd_large(packed_large, c, x0, t, Tg, xs, nullptr, tmp, dr, (cudaStream_t)stream);
 }
 
 // Discrete adjoint of the above. work: 7 B D floats (lambda, stage input, cotangent, yb4, yb3, yb2, yb1).

@@ -62,8 +62,8 @@ __device__ void eval_tile(const LdArgs& a, const float* __restrict__ xs, float* 
     __syncthreads();
 }
 
-// smem: wl[D*D] | y[kTR*D] | f[kTR*D]
-__global__ void large_d_rbf_kernel(const LdArgs a, const float* __restrict__ x, const int64_t B,
+// smem: wl[D*D] | y[kTR*D] | f[kTR*D]. Draw q (GpodeDraws, common.cuh) owns ceil(rows / kTR) tiles and reads nu of draw q.
+__global__ void large_d_rbf_kernel(LdArgs a, const float* __restrict__ x, const GpodeDraws dr,
                                    const float* __restrict__ frff, float* __restrict__ out) {
     extern __shared__ __align__(16) float sm[];
     const int D = a.D;
@@ -76,9 +76,15 @@ __global__ void large_d_rbf_kernel(const LdArgs a, const float* __restrict__ x, 
     }
     const int k = threadIdx.x % D, g = threadIdx.x / D;
     const bool active = g < kNG;
-    const int64_t ntiles = (B + kTR - 1) / kTR;
+    const float* nu0 = a.nu;
+    const int64_t tpd = (dr.rows + kTR - 1) / kTR;
+    const int64_t ntiles = tpd * dr.n;
     for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
-        const int64_t row0 = tile * kTR;
+        const int64_t q = tile / tpd;
+        if (dr.done != nullptr && dr.done[q * dr.done_stride] != 0) continue;
+        // rows of the tile past the draw's last row are out of range, as rows past B are for one draw
+        const int64_t base = q * dr.rows, row0 = base + (tile - q * tpd) * kTR, B = base + dr.rows;
+        a.nu = nu0 + q * D * a.M;
         __syncthreads();
         for (int i = threadIdx.x; i < kTR * D; i += blockDim.x) {
             const int r = i / D, j = i - r * D;
@@ -95,16 +101,8 @@ __global__ void large_d_rbf_kernel(const LdArgs a, const float* __restrict__ x, 
 
 }  // namespace
 
-extern "C" int gpode_vf_fwd_large_add_rbf(const gpode_cache_t* c, const float* x, const float* f_rff, float* f,
-                                          int64_t B, void* stream) {
-    GPODE_CHECK_ARG(c != nullptr, "cache is NULL");
-    GPODE_CHECK_ARG(c->D > GPODE_MAX_D && c->D <= GPODE_MAX_D_LARGE, "large-D path needs %d < D <= %d, got %d",
-                    GPODE_MAX_D, GPODE_MAX_D_LARGE, c->D);
-    GPODE_CHECK_ARG(c->M >= 1 && c->S >= 1 && B >= 0, "bad sizes");
-    GPODE_CHECK_ARG(c->Z && c->nu && c->ell && c->var, "cache tensor is NULL");
-    GPODE_CHECK_ARG(f_rff != nullptr, "f_rff is NULL");
-    if (B == 0) return 0;
-    GPODE_CHECK_ARG(x && f, "NULL argument");
+int gpode_vf_large_add_rbf_draws(const gpode_cache_t* c, const float* x, const float* f_rff, float* f,
+                                 const GpodeDraws& dr, cudaStream_t st) {
     const LdArgs a{c->D, c->M, c->Z, c->nu, c->ell, c->var};
     const int D = c->D;
     const int threads = ((kNG * D + 31) / 32) * 32;  // D=16 -> 64, D=32 -> 128, D=64 -> 256
@@ -118,10 +116,22 @@ extern "C" int gpode_vf_fwd_large_add_rbf(const gpode_cache_t* c, const float* x
         gpode_set_error("large-D kernel does not fit on an SM (smem %zu bytes)", smem);
         return -2;
     }
-    const int64_t ntiles = (B + kTR - 1) / kTR;
+    const int64_t ntiles = (dr.rows + kTR - 1) / kTR * dr.n;
     const int64_t cap = (int64_t)sms * occ;
-    large_d_rbf_kernel<<<(unsigned)(ntiles < cap ? ntiles : cap), threads, smem, (cudaStream_t)stream>>>(a, x, B, f_rff,
-                                                                                                         f);
+    large_d_rbf_kernel<<<(unsigned)(ntiles < cap ? ntiles : cap), threads, smem, st>>>(a, x, dr, f_rff, f);
     GPODE_LAUNCH_CHECK();
     return 0;
+}
+
+extern "C" int gpode_vf_fwd_large_add_rbf(const gpode_cache_t* c, const float* x, const float* f_rff, float* f,
+                                          int64_t B, void* stream) {
+    GPODE_CHECK_ARG(c != nullptr, "cache is NULL");
+    GPODE_CHECK_ARG(c->D > GPODE_MAX_D && c->D <= GPODE_MAX_D_LARGE, "large-D path needs %d < D <= %d, got %d",
+                    GPODE_MAX_D, GPODE_MAX_D_LARGE, c->D);
+    GPODE_CHECK_ARG(c->M >= 1 && c->S >= 1 && B >= 0, "bad sizes");
+    GPODE_CHECK_ARG(c->Z && c->nu && c->ell && c->var, "cache tensor is NULL");
+    GPODE_CHECK_ARG(f_rff != nullptr, "f_rff is NULL");
+    if (B == 0) return 0;
+    GPODE_CHECK_ARG(x && f, "NULL argument");
+    return gpode_vf_large_add_rbf_draws(c, x, f_rff, f, gpode_one_draw(B), (cudaStream_t)stream);
 }

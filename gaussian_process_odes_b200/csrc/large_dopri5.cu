@@ -19,11 +19,12 @@
 // runs on a detached error ratio, so the two initial-step evaluations get no cotangent.
 #include "common.cuh"
 #include "../../include/gpode_b200.h"
+#include <cstddef>
 #include <deque>
 #include <mutex>
 
 int gpode_vf_large_eval(const float* packed_large, const gpode_cache_t* c, const float* x, float* tmp, float* f,
-                        int64_t B, cudaStream_t st);  // large_umma.cu
+                        const GpodeDraws& dr, cudaStream_t st);  // large_umma.cu
 
 namespace {
 
@@ -129,8 +130,12 @@ __device__ __forceinline__ double ld_dir(const double* __restrict__ t, const int
     return (Tg > 1 && t[Tg - 1] < t[0]) ? -1.0 : 1.0;
 }
 
+// Batched prediction (n_sets draws, gpode_dopri5_fwd_large_sets): one LdCtrl per draw. The kernels with one CTA per
+// draw index it by blockIdx.x; the element-wise kernels run on a (blocks, draws) grid, see the offsets of draw
+// blockIdx.y into every [n_sets][n] buffer, and sum into their draw's slice of 2 gridDim.x partials.
 __global__ void ld_start_kernel(LdCtrl* c, const double* __restrict__ t, const int Tg, const int max_attempts,
                                 const int cap, int32_t* __restrict__ out_step) {
+    c += blockIdx.x;
     const double dir = ld_dir(t, Tg);
     c->dir = dir;
     c->t1 = dir * t[0];
@@ -146,6 +151,8 @@ __global__ void ld_start_kernel(LdCtrl* c, const double* __restrict__ t, const i
 __global__ void __launch_bounds__(kLdThreads)
 ld_norm01_kernel(const float* __restrict__ y, const float* __restrict__ f, const float rtol, const float atol,
                  const int64_t n, double* __restrict__ partial) {
+    y += blockIdx.y * n;
+    f += blockIdx.y * n;
     double s0 = 0.0, s1 = 0.0;
     for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (int64_t)gridDim.x * blockDim.x) {
         const float sc = atol + fabsf(y[e]) * rtol;
@@ -153,11 +160,13 @@ ld_norm01_kernel(const float* __restrict__ y, const float* __restrict__ f, const
         s0 += (double)(q0 * q0);
         s1 += (double)(q1 * q1);
     }
-    ld_block_sums(s0, s1, partial, true);
+    ld_block_sums(s0, s1, partial + (size_t)blockIdx.y * 2 * gridDim.x, true);
 }
 
 __global__ void __launch_bounds__(kLdThreads)
 ld_init1_kernel(LdCtrl* c, const double* __restrict__ partial, const int nb, const double n_elem) {
+    c += blockIdx.x;
+    partial += (size_t)blockIdx.x * 2 * nb;
     const double t0 = ld_total(partial, nb), t1 = ld_total(partial + nb, nb);
     if (threadIdx.x == 0) {
         const float d0 = (float)sqrt(t0 / n_elem), d1 = (float)sqrt(t1 / n_elem);
@@ -169,6 +178,10 @@ ld_init1_kernel(LdCtrl* c, const double* __restrict__ partial, const int nb, con
 // out = y + h0 * fsign * f
 __global__ void ld_euler_kernel(const LdCtrl* __restrict__ c, const float* __restrict__ y, const float* __restrict__ f,
                                 float* __restrict__ out, const int64_t n) {
+    c += blockIdx.y;
+    y += blockIdx.y * n;
+    f += blockIdx.y * n;
+    out += blockIdx.y * n;
     const float h0 = c->h0, fs = (float)c->dir;
     for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (int64_t)gridDim.x * blockDim.x)
         out[e] = y[e] + h0 * (fs * f[e]);
@@ -177,6 +190,10 @@ __global__ void ld_euler_kernel(const LdCtrl* __restrict__ c, const float* __res
 __global__ void __launch_bounds__(kLdThreads)
 ld_norm2_kernel(const float* __restrict__ y, const float* __restrict__ f0, const float* __restrict__ f1, const float rtol,
                 const float atol, const int64_t n, double* __restrict__ partial) {
+    y += blockIdx.y * n;
+    f0 += blockIdx.y * n;
+    f1 += blockIdx.y * n;
+    partial += (size_t)blockIdx.y * 2 * gridDim.x;
     double s2 = 0.0;
     for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (int64_t)gridDim.x * blockDim.x) {
         const float sc = atol + fabsf(y[e]) * rtol;
@@ -203,6 +220,8 @@ __device__ void ld_loop_head(LdCtrl* c, const double* __restrict__ t, const int 
 __global__ void __launch_bounds__(kLdThreads)
 ld_init2_kernel(LdCtrl* c, const double* __restrict__ partial, const int nb, const double n_elem,
                 const double* __restrict__ t, const int Tg) {
+    c += blockIdx.x;
+    partial += (size_t)blockIdx.x * 2 * nb;
     const double t2 = ld_total(partial, nb);
     if (threadIdx.x == 0) {
         const float h0 = c->h0, d1 = c->d1;
@@ -239,9 +258,24 @@ __device__ __forceinline__ float ld_stage_input(const LdBufs& b, const int i, co
     return b.Y[e] + s;
 }
 
-__global__ void ld_stage_kernel(const LdCtrl* __restrict__ c, const int i, const LdBufs b, float* __restrict__ out,
+// the buffers of draw q: every [n_sets][n] buffer advanced by q n
+__device__ __forceinline__ LdBufs ld_bufs_at(LdBufs b, const int64_t o) {
+    b.Y += o;
+#pragma unroll
+    for (int l = 0; l < 7; ++l) b.K[l] += o;
+    b.Ys += o;
+    b.Y1 += o;
+    b.YM += o;
+    b.tmp += o;
+    return b;
+}
+
+__global__ void ld_stage_kernel(const LdCtrl* __restrict__ c, const int i, LdBufs b, float* __restrict__ out,
                                 const int64_t n) {
+    c += blockIdx.y;
     if (c->done) return;
+    b = ld_bufs_at(b, blockIdx.y * n);
+    out += blockIdx.y * n;
     const float fs = (float)c->dir;
     float bd[6];
     ld_stage_coefs(i, (float)c->dt, bd);
@@ -250,31 +284,33 @@ __global__ void ld_stage_kernel(const LdCtrl* __restrict__ c, const int i, const
 }
 
 __global__ void __launch_bounds__(kLdThreads)
-ld_err_kernel(const LdCtrl* __restrict__ c, const LdBufs b, const float rtol, const float atol, const int64_t n,
+ld_err_kernel(const LdCtrl* __restrict__ c, LdBufs b, const float rtol, const float atol, const int64_t n,
               double* __restrict__ partial) {
+    c += blockIdx.y;
+    if (c->done) return;   // the controller does not read the partial sums of a finished draw
+    b = ld_bufs_at(b, blockIdx.y * n);
+    partial += (size_t)blockIdx.y * 2 * gridDim.x;
     double se = 0.0;
-    if (!c->done) {
-        const float dts = (float)c->dt, fs = (float)c->dir;
-        float ce[7], cm[7];
+    const float dts = (float)c->dt, fs = (float)c->dir;
+    float ce[7], cm[7];
+#pragma unroll
+    for (int l = 0; l < 7; ++l) {
+        ce[l] = __fmul_rn(dts, ldCErr[l]);
+        cm[l] = __fmul_rn(dts, ldCMid[l]);
+    }
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (int64_t)gridDim.x * blockDim.x) {
+        float er = 0.f, m = 0.f;
 #pragma unroll
         for (int l = 0; l < 7; ++l) {
-            ce[l] = __fmul_rn(dts, ldCErr[l]);
-            cm[l] = __fmul_rn(dts, ldCMid[l]);
+            const float k = fs * b.K[l][e];
+            er = fmaf(k, ce[l], er);
+            m = fmaf(k, cm[l], m);
         }
-        for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (int64_t)gridDim.x * blockDim.x) {
-            float er = 0.f, m = 0.f;
-#pragma unroll
-            for (int l = 0; l < 7; ++l) {
-                const float k = fs * b.K[l][e];
-                er = fmaf(k, ce[l], er);
-                m = fmaf(k, cm[l], m);
-            }
-            const float y = b.Y[e];
-            b.YM[e] = y + m;
-            const float tol = atol + rtol * fmaxf(fabsf(y), fabsf(b.Y1[e]));
-            const float q = er / tol;
-            se += (double)(q * q);
-        }
+        const float y = b.Y[e];
+        b.YM[e] = y + m;
+        const float tol = atol + rtol * fmaxf(fabsf(y), fabsf(b.Y1[e]));
+        const float q = er / tol;
+        se += (double)(q * q);
     }
     ld_block_sums(se, 0.0, partial, false);
 }
@@ -282,7 +318,9 @@ ld_err_kernel(const LdCtrl* __restrict__ c, const LdBufs b, const float rtol, co
 // accept / reject, step-size update (_optimal_step_size: safety 0.9, ifactor 10, dfactor 0.2, order 5), loop condition
 __global__ void __launch_bounds__(kLdThreads)
 ld_ctrl_kernel(LdCtrl* c, const double* __restrict__ partial, const int nb, const double n_elem,
-               const double* __restrict__ t, const int Tg, const cudaGraphConditionalHandle handle) {
+               const double* __restrict__ t, const int Tg, const cudaGraphConditionalHandle handle, const int set_cond) {
+    c += blockIdx.x;
+    partial += (size_t)blockIdx.x * 2 * nb;
     const double tot = ld_total(partial, nb);
     if (threadIdx.x != 0) return;
     if (!c->done) {
@@ -316,14 +354,30 @@ ld_ctrl_kernel(LdCtrl* c, const double* __restrict__ partial, const int nb, cons
     } else {
         c->accept = 0;
     }
-    cudaGraphSetConditional(handle, c->done ? 0u : 1u);
+    if (set_cond) cudaGraphSetConditional(handle, c->done ? 0u : 1u);
+}
+
+// several draws: the loop goes on while any draw is not done
+__global__ void __launch_bounds__(kLdThreads)
+ld_any_kernel(const LdCtrl* __restrict__ c, const int n_sets, const cudaGraphConditionalHandle handle) {
+    __shared__ int any;
+    if (threadIdx.x == 0) any = 0;
+    __syncthreads();
+    for (int q = threadIdx.x; q < n_sets; q += kLdThreads)
+        if (!c[q].done) any = 1;
+    __syncthreads();
+    if (threadIdx.x == 0) cudaGraphSetConditional(handle, any ? 1u : 0u);
 }
 
 // accepted step: dense output at the requested times inside it, then Y <- Y1, K0 <- K6 (FSAL). With checkpoints
 // (ck.y != NULL) the step's start state, its seven stage values, dt and its outputs' step / abscissa go to slot n_acc-1.
-__global__ void ld_accept_kernel(const LdCtrl* __restrict__ c, const LdBufs b, const double* __restrict__ t,
+__global__ void ld_accept_kernel(const LdCtrl* __restrict__ c, LdBufs b, const double* __restrict__ t,
                                  float* __restrict__ xs, const int64_t n, const LdCkpt ck) {
+    c += blockIdx.y;
     if (!c->accept) return;
+    b = ld_bufs_at(b, blockIdx.y * n);
+    xs += blockIdx.y * n;
+    const int64_t xs_stride = n * gridDim.y;   // xs [Tg][n_sets][n]
     const float dts = c->dts_used, fs = (float)c->dir;
     const int jlo = c->jlo, jhi = c->jhi;
     const double t1 = c->t1_used, t1n = c->t1n_used, dir = c->dir;
@@ -357,7 +411,7 @@ __global__ void ld_accept_kernel(const LdCtrl* __restrict__ c, const LdBufs b, c
                 total = total + xp * cb;
                 xp = xp * x;
                 total = total + xp * ca;
-                xs[(int64_t)jo * n + e] = total;
+                xs[(int64_t)jo * xs_stride + e] = total;
             }
         }
         b.Y[e] = yn;
@@ -366,6 +420,8 @@ __global__ void ld_accept_kernel(const LdCtrl* __restrict__ c, const LdBufs b, c
 }
 
 __global__ void ld_stats_kernel(const LdCtrl* __restrict__ c, int32_t* __restrict__ stats) {
+    c += blockIdx.x;
+    stats += 4 * blockIdx.x;
     stats[0] = c->nfe;
     stats[1] = c->n_acc;
     stats[2] = c->n_rej;
@@ -494,17 +550,25 @@ __global__ void ld_adj_x0_kernel(const LdAdj a, const float* __restrict__ gxs, f
 
 }  // namespace
 
-// work layout (floats): Y | K0..K6 | Ys | Y1 | YM | tmp  (12 B D), then 8-byte aligned: partial sums
-// (2 * kLdMaxBlocks float64) and the controller block
-extern "C" int64_t gpode_dopri5_large_work_floats(int D, int64_t B) {
-    return 12 * B * (int64_t)D + 2 + 2 * (2 * (int64_t)kLdMaxBlocks) + (int64_t)(sizeof(LdCtrl) + 3) / 4 + 2;
+// work layout (floats): Y | K0..K6 | Ys | Y1 | YM | tmp  (12 n_sets B D; draw q at q B D inside each), then 8-byte
+// aligned: partial sums (2 * kLdMaxBlocks float64 per draw) and the controller blocks (one per draw)
+static int64_t ld_work_floats(int D, int n_sets, int64_t B) {
+    return 12 * n_sets * B * (int64_t)D + 2 + n_sets * (2 * (2 * (int64_t)kLdMaxBlocks) + (int64_t)(sizeof(LdCtrl) + 3) / 4) +
+           2;
+}
+
+extern "C" int64_t gpode_dopri5_large_work_floats(int D, int64_t B) { return ld_work_floats(D, 1, B); }
+
+extern "C" int64_t gpode_dopri5_large_sets_work_floats(int D, int n_sets, int64_t set_rows) {
+    return ld_work_floats(D, n_sets, set_rows);
 }
 
 namespace {
 
-int ld_fwd(const float* packed_large, const gpode_cache_t* c, const float* x0, const double* t, int Tg, int64_t B,
-           double rtol, double atol, float* xs, float* work, int32_t* stats_out, int max_attempts, float* ckpt, int cap,
-           cudaStream_t st) {
+// n_sets draws of B rows each (draw q: rows [q B, (q + 1) B) of x0 / xs, packed block q), one controller per draw
+int ld_fwd(const float* packed_large, const gpode_cache_t* c, const float* x0, const double* t, int Tg, int n_sets,
+           int64_t B, double rtol, double atol, float* xs, float* work, int32_t* stats_out, int max_attempts, float* ckpt,
+           int cap, cudaStream_t st) {
     GPODE_CHECK_ARG(c != nullptr && c->D > GPODE_MAX_D && c->D <= GPODE_MAX_D_LARGE, "large-D path needs %d < D <= %d",
                     GPODE_MAX_D, GPODE_MAX_D_LARGE);
     GPODE_CHECK_ARG(Tg >= 1 && B >= 0 && max_attempts >= 1, "bad sizes Tg=%d B=%lld", Tg, (long long)B);
@@ -515,41 +579,52 @@ int ld_fwd(const float* packed_large, const gpode_cache_t* c, const float* x0, c
                     "gpode_dopri5_fwd_large builds its own CUDA graph (device-side while loop) and cannot run inside a "
                     "stream capture");
     const int D = c->D;
-    const int64_t n = B * D;
+    const int64_t n = B * D;          // elements of one draw
+    const int64_t na = n * n_sets;    // ... of all draws
     if (B == 0) {
-        GPODE_CUDA(cudaMemsetAsync(stats_out, 0, 4 * sizeof(int32_t), st));
+        GPODE_CUDA(cudaMemsetAsync(stats_out, 0, 4 * sizeof(int32_t) * n_sets, st));
         return 0;
     }
     LdBufs b;
     b.Y = work;
-    for (int l = 0; l < 7; ++l) b.K[l] = work + (1 + l) * n;
-    b.Ys = work + 8 * n;
-    b.Y1 = work + 9 * n;
-    b.YM = work + 10 * n;
-    b.tmp = work + 11 * n;
-    uintptr_t p = reinterpret_cast<uintptr_t>(work + 12 * n);
+    for (int l = 0; l < 7; ++l) b.K[l] = work + (1 + l) * na;
+    b.Ys = work + 8 * na;
+    b.Y1 = work + 9 * na;
+    b.YM = work + 10 * na;
+    b.tmp = work + 11 * na;
+    uintptr_t p = reinterpret_cast<uintptr_t>(work + 12 * na);
     p = (p + 7) & ~(uintptr_t)7;
     double* partial = reinterpret_cast<double*>(p);
-    LdCtrl* ctrl = reinterpret_cast<LdCtrl*>(partial + 2 * kLdMaxBlocks);
+    LdCtrl* ctrl = reinterpret_cast<LdCtrl*>(partial + 2 * kLdMaxBlocks * n_sets);
     const unsigned g = ld_grid(n);
+    const dim3 grid(g, (unsigned)n_sets);
     const double n_elem = (double)n;
     const float rt = (float)rtol, at = (float)atol;
     const LdCkpt ck = ld_ckpt(ckpt, cap, n, Tg);
+    const int64_t stride = gpode_packed_large_floats(D, c->M, c->S);
+    // the start evaluates every draw; inside the loop the tiles of the draws that are done are skipped
+    const GpodeDraws all{n_sets, B, stride, nullptr, 0};
+    const GpodeDraws live{n_sets, B, stride,
+                          n_sets > 1 ? reinterpret_cast<const int*>(reinterpret_cast<const char*>(ctrl) +
+                                                                    offsetof(LdCtrl, done))
+                                     : nullptr,
+                          (int)(sizeof(LdCtrl) / sizeof(int))};
 
     // ---- start: y = x0, f0, initial step (two evaluations) ----
-    GPODE_CUDA(cudaMemcpyAsync(b.Y, x0, sizeof(float) * n, cudaMemcpyDeviceToDevice, st));
-    GPODE_CUDA(cudaMemcpyAsync(xs, x0, sizeof(float) * n, cudaMemcpyDeviceToDevice, st));
-    ld_start_kernel<<<1, 1, 0, st>>>(ctrl, t, Tg, max_attempts, ckpt ? cap : 0, ck.out_step);
-    if (int rc = gpode_vf_large_eval(packed_large, c, b.Y, b.tmp, b.K[0], B, st)) return rc;
-    ld_norm01_kernel<<<g, kLdThreads, 0, st>>>(b.Y, b.K[0], rt, at, n, partial);
-    ld_init1_kernel<<<1, kLdThreads, 0, st>>>(ctrl, partial, (int)g, n_elem);
-    ld_euler_kernel<<<g, kLdThreads, 0, st>>>(ctrl, b.Y, b.K[0], b.Ys, n);
-    if (int rc = gpode_vf_large_eval(packed_large, c, b.Ys, b.tmp, b.K[1], B, st)) return rc;
-    ld_norm2_kernel<<<g, kLdThreads, 0, st>>>(b.Y, b.K[0], b.K[1], rt, at, n, partial);
-    ld_init2_kernel<<<1, kLdThreads, 0, st>>>(ctrl, partial, (int)g, n_elem, t, Tg);
+    GPODE_CUDA(cudaMemcpyAsync(b.Y, x0, sizeof(float) * na, cudaMemcpyDeviceToDevice, st));
+    GPODE_CUDA(cudaMemcpyAsync(xs, x0, sizeof(float) * na, cudaMemcpyDeviceToDevice, st));
+    ld_start_kernel<<<n_sets, 1, 0, st>>>(ctrl, t, Tg, max_attempts, ckpt ? cap : 0, ck.out_step);
+    if (int rc = gpode_vf_large_eval(packed_large, c, b.Y, b.tmp, b.K[0], all, st)) return rc;
+    ld_norm01_kernel<<<grid, kLdThreads, 0, st>>>(b.Y, b.K[0], rt, at, n, partial);
+    ld_init1_kernel<<<n_sets, kLdThreads, 0, st>>>(ctrl, partial, (int)g, n_elem);
+    ld_euler_kernel<<<grid, kLdThreads, 0, st>>>(ctrl, b.Y, b.K[0], b.Ys, n);
+    if (int rc = gpode_vf_large_eval(packed_large, c, b.Ys, b.tmp, b.K[1], all, st)) return rc;
+    ld_norm2_kernel<<<grid, kLdThreads, 0, st>>>(b.Y, b.K[0], b.K[1], rt, at, n, partial);
+    ld_init2_kernel<<<n_sets, kLdThreads, 0, st>>>(ctrl, partial, (int)g, n_elem, t, Tg);
     GPODE_LAUNCH_CHECK();
 
-    // ---- the attempt loop as a WHILE node (condition: "not done", set by the controller kernel) ----
+    // ---- the attempt loop as a WHILE node (condition: "not done", set by the controller kernel; with several draws
+    // "any draw not done", set by ld_any_kernel) ----
     std::lock_guard<std::mutex> lock(g_ld_mutex);
     ld_reap(false);
     if (g_ld_capture_stream == nullptr) GPODE_CUDA(cudaStreamCreateWithFlags(&g_ld_capture_stream, cudaStreamNonBlocking));
@@ -571,13 +646,14 @@ int ld_fwd(const float* packed_large, const gpode_cache_t* c, const float* x0, c
     int rc = 0;
     for (int i = 1; i <= 6 && rc == 0; ++i) {
         float* out = i == 6 ? b.Y1 : b.Ys;
-        ld_stage_kernel<<<g, kLdThreads, 0, cs>>>(ctrl, i, b, out, n);
-        rc = gpode_vf_large_eval(packed_large, c, out, b.tmp, b.K[i], B, cs);
+        ld_stage_kernel<<<grid, kLdThreads, 0, cs>>>(ctrl, i, b, out, n);
+        rc = gpode_vf_large_eval(packed_large, c, out, b.tmp, b.K[i], live, cs);
     }
     if (rc == 0) {
-        ld_err_kernel<<<g, kLdThreads, 0, cs>>>(ctrl, b, rt, at, n, partial);
-        ld_ctrl_kernel<<<1, kLdThreads, 0, cs>>>(ctrl, partial, (int)g, n_elem, t, Tg, handle);
-        ld_accept_kernel<<<g, kLdThreads, 0, cs>>>(ctrl, b, t, xs, n, ck);
+        ld_err_kernel<<<grid, kLdThreads, 0, cs>>>(ctrl, b, rt, at, n, partial);
+        ld_ctrl_kernel<<<n_sets, kLdThreads, 0, cs>>>(ctrl, partial, (int)g, n_elem, t, Tg, handle, n_sets == 1);
+        if (n_sets > 1) ld_any_kernel<<<1, kLdThreads, 0, cs>>>(ctrl, n_sets, handle);
+        ld_accept_kernel<<<grid, kLdThreads, 0, cs>>>(ctrl, b, t, xs, n, ck);
     }
     cudaGraph_t captured = nullptr;
     cudaError_t ce = cudaStreamEndCapture(cs, &captured);
@@ -597,7 +673,7 @@ int ld_fwd(const float* packed_large, const gpode_cache_t* c, const float* x0, c
         return (int)ce;
     }
     GPODE_CUDA(cudaGraphLaunch(exec, st));
-    ld_stats_kernel<<<1, 1, 0, st>>>(ctrl, stats_out);
+    ld_stats_kernel<<<n_sets, 1, 0, st>>>(ctrl, stats_out);
     LdPending pend;
     pend.exec = exec;
     pend.graph = graph;
@@ -613,7 +689,7 @@ int ld_fwd(const float* packed_large, const gpode_cache_t* c, const float* x0, c
 extern "C" int gpode_dopri5_fwd_large(const float* packed_large, const gpode_cache_t* c, const float* x0, const double* t,
                                       int Tg, int64_t B, double rtol, double atol, float* xs, float* work,
                                       int32_t* stats_out, int max_attempts, void* stream) {
-    return ld_fwd(packed_large, c, x0, t, Tg, B, rtol, atol, xs, work, stats_out, max_attempts, nullptr, 0,
+    return ld_fwd(packed_large, c, x0, t, Tg, 1, B, rtol, atol, xs, work, stats_out, max_attempts, nullptr, 0,
                   (cudaStream_t)stream);
 }
 
@@ -622,8 +698,25 @@ extern "C" int gpode_dopri5_fwd_large_ckpt(const float* packed_large, const gpod
                                            float* work, int32_t* stats_out, int max_attempts, float* ckpt, int cap,
                                            void* stream) {
     GPODE_CHECK_ARG(ckpt != nullptr && cap > 0, "checkpointing needs a block and cap > 0 (cap=%d)", cap);
-    return ld_fwd(packed_large, c, x0, t, Tg, B, rtol, atol, xs, work, stats_out, max_attempts, ckpt, cap,
+    return ld_fwd(packed_large, c, x0, t, Tg, 1, B, rtol, atol, xs, work, stats_out, max_attempts, ckpt, cap,
                   (cudaStream_t)stream);
+}
+
+// n_sets draws of the "sets" cache (packed by gpode_pack_cache_large_sets), one controller each: draw q's rows of xs and
+// its stats are those of gpode_dopri5_fwd_large called on draw q alone
+extern "C" int gpode_dopri5_fwd_large_sets(const float* packed_large, const gpode_cache_t* c, int n_sets,
+                                           int64_t set_rows, const float* x0, const double* t, int Tg, double rtol,
+                                           double atol, float* xs, float* work, int32_t* stats_out, int max_attempts,
+                                           void* stream) {
+    GPODE_CHECK_ARG(n_sets >= 1 && n_sets <= 65535 && set_rows >= 0, "n_sets=%d outside 1..65535 or set_rows < 0",
+                    n_sets);
+    if (set_rows == 0) {
+        GPODE_CHECK_ARG(stats_out != nullptr, "stats_out is NULL");
+        GPODE_CUDA(cudaMemsetAsync(stats_out, 0, 4 * sizeof(int32_t) * n_sets, (cudaStream_t)stream));
+        return 0;
+    }
+    return ld_fwd(packed_large, c, x0, t, Tg, n_sets, set_rows, rtol, atol, xs, work, stats_out, max_attempts, nullptr,
+                  0, (cudaStream_t)stream);
 }
 
 // work: 11 B D floats (kb[0..6], yb0, stage input, cotangent, VJP result)

@@ -14,6 +14,8 @@
 //
 // Arithmetic replaced: DSVGP_Layer.rff_forward (reference src/core/dsvgp.py:124-137) for the upper sweep points of
 // BASELINE.json configs[4]. Output: f_rff [B, D]; gpode_rbf_fwd_large (or gpode_vf_fwd_large_add_rbf) adds the RBF term.
+// Batched prediction: both kernels take a draw index (GpodeDraws, common.cuh). The rows are those of n_sets draws, a
+// tile belongs to one draw, and its operand chunks / c = var nu come from that draw's packed block.
 #include "umma.cuh"
 
 namespace {
@@ -40,10 +42,16 @@ __host__ __device__ inline int lu_off(int rows, int r, int q) {
 __host__ __device__ inline int lu_kd(int D) { return (D + 7) & ~7; }     // padded K of the RBF GEMM
 __host__ __device__ inline int lu_nd(int D) { return (D + 15) & ~15; }   // padded N (outputs k)
 
+// blockIdx.y = draw q: omega, phase, w, nu of draw q at their per-draw strides -> block q at out + q * stride
 __global__ void pack_large_kernel(const int D, const int S, const int M, const float* __restrict__ omega,
                                   const float* __restrict__ phase, const float* __restrict__ w,
                                   const float* __restrict__ var, const float* __restrict__ ell,
-                                  const float* __restrict__ nu, float* __restrict__ out) {
+                                  const float* __restrict__ nu, float* __restrict__ out, const int64_t stride) {
+    omega += (int64_t)blockIdx.y * D * S * D;
+    phase += (int64_t)blockIdx.y * S * D;
+    w += (int64_t)blockIdx.y * S * D;
+    nu += (int64_t)blockIdx.y * D * M;
+    out += (int64_t)blockIdx.y * stride;
     const int NC = lu_nc(D);
     const int KP = lu_kp(D), SU = lu_su(D, S), NCH = SU / NC;
     const int64_t rec = lu_rec(D);
@@ -100,7 +108,7 @@ struct LuSmem {  // byte offsets
 
 __global__ void __launch_bounds__(kLuThreads)
 rff_large_umma_kernel(const float* __restrict__ packed, const int D, const int S, const float* __restrict__ x,
-                      float* __restrict__ f_rff, const int64_t B) {
+                      float* __restrict__ f_rff, const GpodeDraws dr) {
     extern __shared__ __align__(128) unsigned char smem[];
     uint64_t* bar_afull = reinterpret_cast<uint64_t*>(smem + LuSmem::bar_afull);
     uint64_t* bar_full = reinterpret_cast<uint64_t*>(smem + LuSmem::bar_full);
@@ -116,7 +124,6 @@ rff_large_umma_kernel(const float* __restrict__ packed, const int D, const int S
     float* a_hi = reinterpret_cast<float*>(smem + LuSmem::tiles);
     float* a_lo = a_hi + a_floats;
     float* ring = a_lo + a_floats;              // [kLuRing][b_floats]
-    const float* __restrict__ aw = packed + (int64_t)D * NCH * rec;
     const int tid = threadIdx.x, warp = tid >> 5;
 
     if (tid == 128) {
@@ -139,11 +146,11 @@ rff_large_umma_kernel(const float* __restrict__ packed, const int D, const int S
     tc_fence_after_sync();
     const uint32_t tmem_base = *tmem_ptr;
 
-    const int64_t n_tiles = (B + kLuRows - 1) / kLuRows;
+    const int64_t tpd = (dr.rows + kLuRows - 1) / kLuRows;   // tiles per draw
+    const int64_t n_tiles = tpd * dr.n;
     const int chunks_per_tile = D * NCH;
-    int64_t my_tiles = 0;
-    for (int64_t t = blockIdx.x; t < n_tiles; t += gridDim.x) ++my_tiles;
-    const int64_t total_chunks = my_tiles * chunks_per_tile;
+    // rows and producer skip the same tiles, so their chunk sequences still agree
+    auto skip = [&](const int64_t tile) { return dr.done != nullptr && dr.done[(tile / tpd) * dr.done_stride] != 0; };
     // every CTA walks the output dimensions in its own rotation, so that the SMs do not all pull the same operand
     // chunk from the same L2 lines at the same moment
     const int k_rot = (int)(blockIdx.x % (unsigned)D);
@@ -151,11 +158,14 @@ rff_large_umma_kernel(const float* __restrict__ packed, const int D, const int S
     if (warp < 4) {
         uint32_t g = 0;
         for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-            const int64_t row0 = tile * kLuRows;
+            if (skip(tile)) continue;
+            const int64_t q = tile / tpd, lr0 = (tile - q * tpd) * kLuRows;   // draw, its first row in this tile
+            const int64_t row0 = q * dr.rows + lr0, nr = dr.rows - lr0;       // rows r < nr of the tile exist
+            const float* __restrict__ aw = packed + q * dr.stride + (int64_t)D * NCH * rec;
             // ---- state tile -> shared memory (coalesced global reads), pre-split into tf32 hi / lo ----
             for (int i = tid; i < kLuRows * D; i += kLuRows) {
                 const int r = i / D, j = i - r * D;
-                const float v = row0 + r < B ? __ldg(x + row0 * D + i) : 0.f;
+                const float v = r < nr ? __ldg(x + row0 * D + i) : 0.f;
                 float hi, lo;
                 gpode_split_tf32_rn(v, hi, lo);
                 const int o = lu_off(kLuRows, r, j);
@@ -169,7 +179,6 @@ rff_large_umma_kernel(const float* __restrict__ packed, const int D, const int S
             }
             fence_proxy_async_smem();
             mbar_arrive(bar_afull);
-            const int64_t row = row0 + tid;
             for (int kk = 0; kk < D; ++kk) {
                 const int k = kk + k_rot < D ? kk + k_rot : kk + k_rot - D;
                 float acc0 = 0.f, acc1 = 0.f;
@@ -206,19 +215,27 @@ rff_large_umma_kernel(const float* __restrict__ packed, const int D, const int S
                         consume(rb, wg + cc + 32);
                     }
                 }
-                if (row < B) f_rff[row * D + k] = acc0 + acc1;
+                if (tid < nr) f_rff[(row0 + tid) * D + k] = acc0 + acc1;
             }
         }
     } else if (tid == 128) {
         // ---- producer: operand copies one chunk ahead, then the MMAs of the current chunk ----
         const uint32_t copy_bytes = (uint32_t)b_floats * 4u;
+        // copy cursor: chunk ld_ci of tile ld_tile is the next one to copy
+        int64_t ld_tile = blockIdx.x;
+        while (ld_tile < n_tiles && skip(ld_tile)) ld_tile += gridDim.x;
+        int ld_ci = 0;
         auto load = [&](const int64_t gq) {  // chunk gq of this CTA's sequence -> ring slot gq % kLuRing
+            if (ld_tile >= n_tiles) return;
             const int slot = (int)(gq % kLuRing);
             if (gq >= kLuRing) mbar_wait_bounded(bar_bfree + slot, (uint32_t)((gq / kLuRing - 1) & 1));
-            const int64_t local = gq % chunks_per_tile;              // (kk, c) of the tile, kk rotated like the rows do
-            const int kk = (int)(local / NCH), c = (int)(local - (int64_t)kk * NCH);
+            const int kk = ld_ci / NCH, c = ld_ci - kk * NCH;         // (kk, c) of the tile, kk rotated like the rows do
             const int k = kk + k_rot < D ? kk + k_rot : kk + k_rot - D;
-            const float* src = packed + ((int64_t)k * NCH + c) * rec;
+            const float* src = packed + (ld_tile / tpd) * dr.stride + ((int64_t)k * NCH + c) * rec;
+            if (++ld_ci == chunks_per_tile) {
+                ld_ci = 0;
+                do ld_tile += gridDim.x; while (ld_tile < n_tiles && skip(ld_tile));
+            }
             float* dst = ring + (size_t)slot * b_floats;
             asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(gpode_smem_u32(bar_bfull + slot)),
                          "r"(copy_bytes)
@@ -239,13 +256,15 @@ rff_large_umma_kernel(const float* __restrict__ packed, const int D, const int S
         const uint64_t step_a = (2u * lbo_a) >> 4, step_b = (2u * lbo_b) >> 4;  // one K-step = two K chunks
         int64_t gq = 0;
         uint32_t tile_it = 0;
-        for (int64_t q = 0; q < kLuRing - 1 && q < total_chunks; ++q) load(q);
-        for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++tile_it) {
+        for (int64_t q = 0; q < kLuRing - 1; ++q) load(q);
+        for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+            if (skip(tile)) continue;
             mbar_wait_bounded(bar_afull, tile_it & 1);
+            ++tile_it;
             tc_fence_after_sync();
             for (int ci = 0; ci < chunks_per_tile; ++ci, ++gq) {
                 const int slot = (int)(gq % kLuRing), tb = (int)(gq & 1);
-                if (gq + kLuRing - 1 < total_chunks) load(gq + kLuRing - 1);
+                load(gq + kLuRing - 1);
                 mbar_wait_bounded(bar_bfull + slot, (uint32_t)((gq / kLuRing) & 1));
                 if (gq >= 2) mbar_wait_bounded(bar_empty + tb, (uint32_t)(((gq >> 1) - 1) & 1));
                 tc_fence_after_sync();
@@ -303,7 +322,7 @@ template <int NDT>   // NDT = lu_nd(D): sizes the per-row accumulators, so small
 __global__ void __launch_bounds__(kRbThreads, NDT <= 16 ? 3 : (NDT <= 32 ? 2 : 1))
 rbf_large_umma_kernel(const float* __restrict__ packed, const int D, const int S, const int M,
                       const float* __restrict__ Z, const float* __restrict__ x, const float* __restrict__ f_rff,
-                      float* __restrict__ f_out, const int64_t B) {
+                      float* __restrict__ f_out, const GpodeDraws dr) {
     extern __shared__ __align__(128) unsigned char smem[];
     uint64_t* bar_afull = reinterpret_cast<uint64_t*>(smem + RbSmem::bar_afull);  // [2] 128 producer arrivals
     uint64_t* bar_afree = reinterpret_cast<uint64_t*>(smem + RbSmem::bar_afree);  // [2] commit
@@ -314,7 +333,7 @@ rbf_large_umma_kernel(const float* __restrict__ packed, const int D, const int S
     constexpr int ND = NDT;
     const int SU = lu_su(D, S), NCH = SU / lu_nc(D);
     const float* __restrict__ wt_g = packed + (int64_t)D * NCH * lu_rec(D) + (int64_t)D * SU;
-    const float* __restrict__ cp_g = wt_g + 2 * ND * KD;
+    const int64_t cp_off = (int64_t)D * NCH * lu_rec(D) + (int64_t)D * SU + 2 * ND * KD;   // c = var nu: per draw
     float* wt = reinterpret_cast<float*>(smem + RbSmem::data);   // [-W^T hi | lo], 2 ND KD floats
     float* zs = wt + 2 * ND * KD;                                 // [M][KD], zero padded
     float* xs = zs + M * KD;                                      // [K4][128][4]
@@ -344,12 +363,16 @@ rbf_large_umma_kernel(const float* __restrict__ packed, const int D, const int S
     __syncthreads();
     tc_fence_after_sync();
     const uint32_t tmem_base = *tmem_ptr;
-    const int64_t n_tiles = (B + kLuRows - 1) / kLuRows;
+    const int64_t tpd = (dr.rows + kLuRows - 1) / kLuRows;   // tiles per draw; -W^T and Z are shared by all draws
+    const int64_t n_tiles = tpd * dr.n;
+    auto skip = [&](const int64_t tile) { return dr.done != nullptr && dr.done[(tile / tpd) * dr.done_stride] != 0; };
 
     if (warp < 4) {
         // ---- consumers: exponent -> 2^e -> weighted sum over the inducing points ----
         uint32_t g = 0;
         for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+            if (skip(tile)) continue;
+            const float* __restrict__ cp_g = packed + (tile / tpd) * dr.stride + cp_off;
             float f[ND];
 #pragma unroll
             for (int k = 0; k < ND; ++k) f[k] = 0.f;
@@ -396,8 +419,8 @@ rbf_large_umma_kernel(const float* __restrict__ packed, const int D, const int S
                 }
                 }
             }
-            const int64_t row = tile * kLuRows + tid;
-            if (row < B) {
+            const int64_t q = tile / tpd, lr = (tile - q * tpd) * kLuRows + tid, row = q * dr.rows + lr;
+            if (lr < dr.rows) {
 #pragma unroll
                 for (int k = 0; k < ND; ++k)
                     if (k < D) f_out[row * D + k] = __ldg(f_rff + row * D + k) + f[k];
@@ -408,11 +431,13 @@ rbf_large_umma_kernel(const float* __restrict__ packed, const int D, const int S
         const int r = tid - 128;
         uint32_t g = 0;
         for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-            const int64_t row0 = tile * kLuRows;
+            if (skip(tile)) continue;
+            const int64_t q = tile / tpd, lr0 = (tile - q * tpd) * kLuRows;
+            const int64_t row0 = q * dr.rows + lr0, nr = dr.rows - lr0;
             asm volatile("bar.sync 1, 128;" ::: "memory");  // the previous tile's readers of xs are done
             for (int i = r; i < kLuRows * D; i += kLuRows) {
                 const int rr = i / D, j = i - rr * D;
-                xs[(j >> 2) * (kLuRows * 4) + rr * 4 + (j & 3)] = row0 + rr < B ? __ldg(x + row0 * D + i) : 0.f;
+                xs[(j >> 2) * (kLuRows * 4) + rr * 4 + (j & 3)] = rr < nr ? __ldg(x + row0 * D + i) : 0.f;
             }
             for (int j = D; j < KD; ++j) xs[(j >> 2) * (kLuRows * 4) + r * 4 + (j & 3)] = 0.f;
             asm volatile("bar.sync 1, 128;" ::: "memory");
@@ -451,6 +476,7 @@ rbf_large_umma_kernel(const float* __restrict__ packed, const int D, const int S
         const uint64_t step_a = (2u * lbo_a) >> 4, step_b = (2u * lbo_b) >> 4;
         uint32_t g = 0;
         for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+            if (skip(tile)) continue;
             for (int m = 0; m < M; ++m, ++g) {
                 const int slot = g & 1;
                 mbar_wait_bounded(bar_afull + slot, (g >> 1) & 1);
@@ -487,23 +513,36 @@ extern "C" int64_t gpode_packed_large_floats(int D, int M, int S) {
            (int64_t)M * lu_nd(D);
 }
 
-extern "C" int gpode_pack_cache_large(const gpode_cache_t* c, float* packed, void* stream) {
+int gpode_vf_large_add_rbf_draws(const gpode_cache_t* c, const float* x, const float* f_rff, float* f,
+                                 const GpodeDraws& dr, cudaStream_t st);  // large_d.cu
+
+// n_sets blocks back to back, gpode_packed_large_floats(D,M,S) floats apart; omega / phase / w / nu of the cache carry
+// the leading draw axis (a one-draw cache is the plain one)
+static int pack_large(const gpode_cache_t* c, int n_sets, float* packed, void* stream) {
     GPODE_CHECK_ARG(c != nullptr && packed != nullptr, "cache / packed is NULL");
     GPODE_CHECK_ARG(c->D > GPODE_MAX_D && c->D <= GPODE_MAX_D_LARGE, "large-D path needs %d < D <= %d, got %d",
                     GPODE_MAX_D, GPODE_MAX_D_LARGE, c->D);
+    GPODE_CHECK_ARG(n_sets >= 1 && n_sets <= 65535, "n_sets=%d outside 1..65535", n_sets);
     GPODE_CHECK_ARG(c->S >= 1 && c->M >= 1 && c->omega && c->phase && c->w && c->var && c->ell && c->nu,
                     "cache tensor is NULL");
-    pack_large_kernel<<<592, 256, 0, (cudaStream_t)stream>>>(c->D, c->S, c->M, c->omega, c->phase, c->w, c->var,
-                                                             c->ell, c->nu, packed);
+    const unsigned gx = n_sets < 592 ? 592u / (unsigned)n_sets : 1u;
+    pack_large_kernel<<<dim3(gx, n_sets), 256, 0, (cudaStream_t)stream>>>(
+        c->D, c->S, c->M, c->omega, c->phase, c->w, c->var, c->ell, c->nu, packed,
+        gpode_packed_large_floats(c->D, c->M, c->S));
     GPODE_LAUNCH_CHECK();
     return 0;
 }
 
-extern "C" int gpode_rff_fwd_large(const float* packed_large, int D, int S, const float* x, float* f_rff, int64_t B,
-                                   void* stream) {
-    GPODE_CHECK_ARG(packed_large && x && f_rff, "NULL argument");
-    GPODE_CHECK_ARG(D > GPODE_MAX_D && D <= GPODE_MAX_D_LARGE && S >= 1 && B >= 0, "bad sizes D=%d S=%d", D, S);
-    if (B == 0) return 0;
+extern "C" int gpode_pack_cache_large(const gpode_cache_t* c, float* packed, void* stream) {
+    return pack_large(c, 1, packed, stream);
+}
+
+extern "C" int gpode_pack_cache_large_sets(const gpode_cache_t* c, int n_sets, float* packed, void* stream) {
+    return pack_large(c, n_sets, packed, stream);
+}
+
+static int rff_launch(const float* packed_large, int D, int S, const float* x, float* f_rff, const GpodeDraws& dr,
+                      cudaStream_t st) {
     const int KP = lu_kp(D);
     const size_t smem = LuSmem::tiles + (size_t)(2 * KP * kLuRows + kLuRing * lu_rec(D)) * 4;
     GPODE_CUDA(cudaFuncSetAttribute(rff_large_umma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -516,22 +555,32 @@ extern "C" int gpode_rff_fwd_large(const float* packed_large, int D, int S, cons
         gpode_set_error("large-D tensor-core kernel does not fit on an SM (smem %zu bytes)", smem);
         return -2;
     }
-    const int64_t tiles = (B + kLuRows - 1) / kLuRows, cap = (int64_t)sms * occ;
-    rff_large_umma_kernel<<<(unsigned)(tiles < cap ? tiles : cap), kLuThreads, smem, (cudaStream_t)stream>>>(
-        packed_large, D, S, x, f_rff, B);
+    const int64_t tiles = (dr.rows + kLuRows - 1) / kLuRows * dr.n, cap = (int64_t)sms * occ;
+    rff_large_umma_kernel<<<(unsigned)(tiles < cap ? tiles : cap), kLuThreads, smem, st>>>(packed_large, D, S, x, f_rff,
+                                                                                         dr);
     GPODE_LAUNCH_CHECK();
     return 0;
 }
 
-extern "C" int gpode_rbf_fwd_large(const float* packed_large, int D, int M, int S, const float* Z, const float* x,
-                                   const float* f_rff, float* f, int64_t B, void* stream) {
-    GPODE_CHECK_ARG(packed_large && Z && x && f_rff && f, "NULL argument");
-    GPODE_CHECK_ARG(D > GPODE_MAX_D && D <= GPODE_MAX_D_LARGE && S >= 1 && M >= 1 && B >= 0, "bad sizes D=%d M=%d", D, M);
+extern "C" int gpode_rff_fwd_large(const float* packed_large, int D, int S, const float* x, float* f_rff, int64_t B,
+                                   void* stream) {
+    GPODE_CHECK_ARG(packed_large && x && f_rff, "NULL argument");
+    GPODE_CHECK_ARG(D > GPODE_MAX_D && D <= GPODE_MAX_D_LARGE && S >= 1 && B >= 0, "bad sizes D=%d S=%d", D, S);
     if (B == 0) return 0;
+    return rff_launch(packed_large, D, S, x, f_rff, gpode_one_draw(B), (cudaStream_t)stream);
+}
+
+static size_t rbf_smem(int D, int M) {
     const int KD = lu_kd(D), ND = lu_nd(D);
-    const size_t smem = RbSmem::data + (size_t)(2 * ND * KD + M * KD + KD * kLuRows + 4 * KD * kLuRows) * 4;
+    return RbSmem::data + (size_t)(2 * ND * KD + M * KD + KD * kLuRows + 4 * KD * kLuRows) * 4;
+}
+
+static int rbf_launch(const float* packed_large, int D, int M, int S, const float* Z, const float* x, const float* f_rff,
+                      float* f, const GpodeDraws& dr, cudaStream_t st) {
+    const int ND = lu_nd(D);
+    const size_t smem = rbf_smem(D, M);
     GPODE_CHECK_ARG(smem <= 227u * 1024u, "M=%d too large for the shared-memory copy of Z (needs %zu bytes)", M, smem);
-    void (*kern)(const float*, int, int, int, const float*, const float*, const float*, float*, int64_t) =
+    void (*kern)(const float*, int, int, int, const float*, const float*, const float*, float*, GpodeDraws) =
         ND == 16 ? rbf_large_umma_kernel<16> : ND == 32 ? rbf_large_umma_kernel<32>
         : ND == 48 ? rbf_large_umma_kernel<48> : rbf_large_umma_kernel<64>;
     GPODE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -548,20 +597,39 @@ extern "C" int gpode_rbf_fwd_large(const float* packed_large, int D, int M, int 
     const int reg_occ = 65536 / (((fa.numRegs + 7) & ~7) * kRbThreads);
     if (occ > reg_occ) occ = reg_occ;
     if (occ < 1) occ = 1;
-    const int64_t tiles = (B + kLuRows - 1) / kLuRows, cap = (int64_t)sms * occ;
-    kern<<<(unsigned)(tiles < cap ? tiles : cap), kRbThreads, smem, (cudaStream_t)stream>>>(
-        packed_large, D, S, M, Z, x, f_rff, f, B);
+    const int64_t tiles = (dr.rows + kLuRows - 1) / kLuRows * dr.n, cap = (int64_t)sms * occ;
+    kern<<<(unsigned)(tiles < cap ? tiles : cap), kRbThreads, smem, st>>>(packed_large, D, S, M, Z, x, f_rff, f, dr);
     GPODE_LAUNCH_CHECK();
     return 0;
 }
 
+extern "C" int gpode_rbf_fwd_large(const float* packed_large, int D, int M, int S, const float* Z, const float* x,
+                                   const float* f_rff, float* f, int64_t B, void* stream) {
+    GPODE_CHECK_ARG(packed_large && Z && x && f_rff && f, "NULL argument");
+    GPODE_CHECK_ARG(D > GPODE_MAX_D && D <= GPODE_MAX_D_LARGE && S >= 1 && M >= 1 && B >= 0, "bad sizes D=%d M=%d", D, M);
+    if (B == 0) return 0;
+    return rbf_launch(packed_large, D, M, S, Z, x, f_rff, f, gpode_one_draw(B), (cudaStream_t)stream);
+}
+
 // f = vf(x) for 8 < D <= 64: Fourier-feature term, then the RBF term added to it, both on the tcgen05 tensor cores (the
-// RBF term falls back to the tiled FP32 kernel when Z does not fit its shared-memory copy). tmp: B D floats.
+// RBF term falls back to the tiled FP32 kernel when Z does not fit its shared-memory copy). tmp: rows D floats.
+// dr: the draws (gpode_one_draw(B) for one function); dr.stride must be gpode_packed_large_floats(D,M,S).
 int gpode_vf_large_eval(const float* packed_large, const gpode_cache_t* c, const float* x, float* tmp, float* f,
-                        int64_t B, cudaStream_t st) {
-    if (int rc = gpode_rff_fwd_large(packed_large, c->D, c->S, x, tmp, B, st)) return rc;
-    const int KD = lu_kd(c->D), ND = lu_nd(c->D);
-    const size_t smem = RbSmem::data + (size_t)(2 * ND * KD + c->M * KD + KD * kLuRows + 4 * KD * kLuRows) * 4;
-    if (smem <= 227u * 1024u) return gpode_rbf_fwd_large(packed_large, c->D, c->M, c->S, c->Z, x, tmp, f, B, st);
-    return gpode_vf_fwd_large_add_rbf(c, x, tmp, f, B, st);
+                        const GpodeDraws& dr, cudaStream_t st) {
+    if (int rc = rff_launch(packed_large, c->D, c->S, x, tmp, dr, st)) return rc;
+    if (rbf_smem(c->D, c->M) <= 227u * 1024u) return rbf_launch(packed_large, c->D, c->M, c->S, c->Z, x, tmp, f, dr, st);
+    return gpode_vf_large_add_rbf_draws(c, x, tmp, f, dr, st);
+}
+
+extern "C" int gpode_vf_fwd_large_sets(const float* packed_large, const gpode_cache_t* c, int n_sets, int64_t set_rows,
+                                       const float* x, float* tmp, float* f, void* stream) {
+    GPODE_CHECK_ARG(c != nullptr && c->D > GPODE_MAX_D && c->D <= GPODE_MAX_D_LARGE, "large-D path needs %d < D <= %d",
+                    GPODE_MAX_D, GPODE_MAX_D_LARGE);
+    GPODE_CHECK_ARG(n_sets >= 1 && n_sets <= 65535 && set_rows >= 0, "n_sets=%d outside 1..65535 or set_rows < 0",
+                    n_sets);
+    GPODE_CHECK_ARG(c->M >= 1 && c->S >= 1 && c->Z && c->nu && c->ell && c->var, "cache tensor is NULL");
+    if (set_rows == 0) return 0;
+    GPODE_CHECK_ARG(packed_large && x && tmp && f, "NULL argument");
+    const GpodeDraws dr{n_sets, set_rows, gpode_packed_large_floats(c->D, c->M, c->S), nullptr, 0};
+    return gpode_vf_large_eval(packed_large, c, x, tmp, f, dr, (cudaStream_t)stream);
 }

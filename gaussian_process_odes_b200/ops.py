@@ -789,6 +789,17 @@ def dopri5_integrate(x0, t, Z, ell, var, nu, omega, phase, w, rtol=1e-6, atol=1e
     return _Dopri5.apply(x0, t, Z, ell, var, nu, omega, phase, w, rtol, atol, torch.is_grad_enabled())
 
 
+def _kzz_cholesky_large(Zd, ed, vd, jitter):
+    """float64 ``L (D,M,M) = chol(K(Z,Z) + jitter I)`` per output dimension for 8 < D <= 64 (``torch.linalg``)."""
+    D, M = ed.shape[0], Zd.shape[0]
+    Ks = []
+    for k0 in range(0, D, 8):   # direct-form squared distance, eight output dimensions at a time ((8, M, M, J) temporary)
+        d = (Zd[None, :, None, :] - Zd[None, None, :, :]) / ed[k0:k0 + 8, None, None, :]
+        Ks.append(vd[k0:k0 + 8, None, None] * torch.exp(-0.5 * (d * d).sum(-1)))
+    K = torch.cat(Ks, 0)
+    return torch.linalg.cholesky(K + jitter * torch.eye(M, dtype=torch.float64, device=Zd.device))
+
+
 def _whiten_large(Z, ell, var, u, omega, phase, w, jitter):
     """The same whitening for 8 < D <= 64, where the in-shared-memory Cholesky kernels (one CTA per output dimension, a
     cluster of D <= 8 CTAs in the backward) do not apply: D batched M x M factorisations and triangular solves through
@@ -796,15 +807,10 @@ def _whiten_large(Z, ell, var, u, omega, phase, w, jitter):
     the direct form, differentiated by autograd. At these state dimensions the step time is in the integrator kernels
     (tcgen05 vector field and VJP); this keeps ``DSVGP_Layer.build_cache`` -- and with it ``Flow`` and the model classes --
     usable up to D = 64 (reference src/core/dsvgp.py:92-122 has no dimension limit)."""
-    D, M = ell.shape[0], Z.shape[0]
+    D = ell.shape[0]
     S = w.shape[0]
     Zd, ed, vd = Z.double(), ell.double(), var.double()
-    Ks = []
-    for k0 in range(0, D, 8):   # direct-form squared distance, eight output dimensions at a time ((8, M, M, J) temporary)
-        d = (Zd[None, :, None, :] - Zd[None, None, :, :]) / ed[k0:k0 + 8, None, None, :]
-        Ks.append(vd[k0:k0 + 8, None, None] * torch.exp(-0.5 * (d * d).sum(-1)))
-    K = torch.cat(Ks, 0)
-    L = torch.linalg.cholesky(K + jitter * torch.eye(M, dtype=torch.float64, device=Z.device))
+    L = _kzz_cholesky_large(Zd, ed, vd, jitter)
     theta = torch.einsum('mj,jsk->msk', Zd, omega.double()) + phase.double().reshape(1, S, D)
     prior = (torch.cos(theta) * (w.double() * torch.sqrt(vd / S)).unsqueeze(0)).sum(1)  # rff_forward(Z): (M, D)
     a = torch.linalg.solve_triangular(L, prior.t().unsqueeze(2), upper=False)
@@ -836,8 +842,8 @@ def _sets_common(Z, ell, var, omega, phase, w):
         raise _lib.GpodeError("sets tensors need a leading n_sets axis: omega (n,D,S,D), w (n,S,D); got %s, %s"
                               % (tuple(oc.shape), tuple(wc.shape)))
     n, S = wc.shape[0], wc.shape[1]
-    if D > MAX_D_REGISTER:
-        raise _lib.GpodeError("batched prediction needs D <= %d, got %d" % (MAX_D_REGISTER, D))
+    if D > MAX_D_LARGE:
+        raise _lib.GpodeError("batched prediction needs D <= %d, got %d" % (MAX_D_LARGE, D))
     pc_ = f32(phase, "phase").reshape(n, S, D)
     if tuple(oc.shape) != (n, D, S, D) or tuple(wc.shape) != (n, S, D) or tuple(ec.shape) != (D, D):
         raise _lib.GpodeError("inconsistent sets shapes: omega %s w %s ell %s" % (
@@ -845,13 +851,37 @@ def _sets_common(Z, ell, var, omega, phase, w):
     return Zc, ec, vc, oc, pc_, wc, n, D, M, S
 
 
+def _whiten_large_sets(Zc, ec, vc, uc, oc, pc_, wc, jitter):
+    """``whiten_sets`` for 8 < D <= 64: one float64 Kzz factorisation for all draws (``_kzz_cholesky_large``, as
+    ``_whiten_large`` does for one draw), then the prior at Z and the two triangular solves per draw, a chunk of draws at
+    a time (the float64 angles are (n, M, S, D): 1.7 GB for 128 draws at M = 100, S = 256, D = 64)."""
+    n, S, D = wc.shape
+    M = Zc.shape[0]
+    Zd, ed, vd = Zc.double(), ec.double(), vc.double()
+    L = _kzz_cholesky_large(Zd, ed, vd, jitter)
+    a_scale = torch.sqrt(vd / S)
+    nu = torch.empty(n, D, M, dtype=torch.float32, device=Zc.device)
+    chunk = max(1, (1 << 25) // (M * S * D))   # draws per chunk: at most 256 MB of float64 angles
+    for q0 in range(0, n, chunk):
+        q1 = min(n, q0 + chunk)
+        theta = torch.einsum('mj,njsk->nmsk', Zd, oc[q0:q1].double()) + pc_[q0:q1].double().unsqueeze(1)
+        prior = (torch.cos(theta) * (wc[q0:q1].double() * a_scale).unsqueeze(1)).sum(2)   # rff_forward(Z): (c, M, D)
+        a = torch.linalg.solve_triangular(L, prior.transpose(1, 2).unsqueeze(3), upper=False)
+        nq = torch.linalg.solve_triangular(L.transpose(1, 2), uc[q0:q1].double().transpose(1, 2).unsqueeze(3) - a,
+                                           upper=True)
+        nu[q0:q1] = nq.squeeze(3).float()
+    return nu
+
+
 def whiten_sets(Z, ell, var, u, omega, phase, w, jitter=1e-5):
     """``u (n,M,D)`` and per-draw ``omega (n,D,S,D)``, ``phase (n,S,D)``, ``w (n,S,D)`` -> ``nu (n,D,M)``. One Kzz
-    factorisation for all draws (``gpode_whiten_fwd_sets``). No gradient."""
+    factorisation for all draws (``gpode_whiten_fwd_sets``; float64 ``torch.linalg`` for 8 < D <= 64). No gradient."""
     Zc, ec, vc, oc, pc_, wc, n, D, M, S = _sets_common(Z, ell, var, omega, phase, w)
     uc = f32(u, "u")
     if tuple(uc.shape) != (n, M, D):
         raise _lib.GpodeError("u must be (%d,%d,%d), got %s" % (n, M, D, tuple(uc.shape)))
+    if D > MAX_D_REGISTER:
+        return _whiten_large_sets(Zc, ec, vc, uc, oc, pc_, wc, jitter)
     st = _cache_struct(D, M, S, oc, pc_, wc, Zc, None, ec, vc)
     nu = torch.empty(n, D, M, dtype=torch.float32, device=Zc.device)
     L = torch.empty(D, M, M, dtype=torch.float64, device=Zc.device)
@@ -862,7 +892,8 @@ def whiten_sets(Z, ell, var, u, omega, phase, w, jitter=1e-5):
 
 
 class PackedCacheSets:
-    """``n`` sampled GP functions sharing Z and the hyper-parameters, packed back to back (``gpode_pack_cache_sets``)."""
+    """``n`` sampled GP functions sharing Z and the hyper-parameters, packed back to back (``gpode_pack_cache_sets``;
+    ``gpode_pack_cache_large_sets`` for 8 < D <= 64, whose kernels also read the "sets" cache ``struct``)."""
 
     def __init__(self, Z, ell, var, nu, omega, phase, w):
         lib = _lib.load()
@@ -870,10 +901,14 @@ class PackedCacheSets:
         Zc, ec, vc, oc, pc_, wc, self.n, self.D, self.M, self.S = self.keep
         nc = f32(nu, "nu").reshape(self.n, self.D, self.M)
         self.keep = self.keep + (nc,)
-        st = _cache_struct(self.D, self.M, self.S, oc, pc_, wc, Zc, nc, ec, vc)
-        stride = lib.gpode_packed_floats(self.D, self.M, self.S)
+        self.struct = _cache_struct(self.D, self.M, self.S, oc, pc_, wc, Zc, nc, ec, vc)
+        self.large = self.D > MAX_D_REGISTER
+        if self.large:
+            stride, pack = lib.gpode_packed_large_floats(self.D, self.M, self.S), "gpode_pack_cache_large_sets"
+        else:
+            stride, pack = lib.gpode_packed_floats(self.D, self.M, self.S), "gpode_pack_cache_sets"
         self.packed = torch.empty(self.n * stride, dtype=torch.float32, device=Zc.device)
-        _lib.call("gpode_pack_cache_sets", ctypes.byref(st), self.n, ptr(self.packed), stream_ptr())
+        _lib.call(pack, ctypes.byref(self.struct), self.n, ptr(self.packed), stream_ptr())
 
 
 def _rows_of_sets(x, pcs, name):
@@ -890,6 +925,10 @@ def vector_field_sets(x, Z, ell, var, nu, omega, phase, w):
     pcs = PackedCacheSets(Z, ell, var, nu, omega, phase, w)
     xc, N = _rows_of_sets(x, pcs, "x")
     f = torch.empty_like(xc)
+    if pcs.large:
+        _lib.call("gpode_vf_fwd_large_sets", ptr(pcs.packed), ctypes.byref(pcs.struct), pcs.n, N, ptr(xc),
+                  ptr(torch.empty_like(xc)), ptr(f), stream_ptr())
+        return f
     _lib.call("gpode_vf_fwd_sets", ptr(pcs.packed), pcs.D, pcs.M, pcs.S, pcs.n, N, ptr(xc), ptr(f), stream_ptr())
     return f
 
@@ -897,7 +936,9 @@ def vector_field_sets(x, Z, ell, var, nu, omega, phase, w):
 def integrate_sets(x0, t, Z, ell, var, nu, omega, phase, w, method="dopri5", rtol=1e-6, atol=1e-6):
     """``x0 (n,N,D)``, shared grid ``t (Tg,)`` -> ``(xs (n,N,Tg,D), stats)``: draw q integrates its own N trajectories
     with its own function, exactly as n separate ``odeint`` calls would (dopri5: one controller per draw), in ONE
-    launch. ``stats``: device int32 ``(n,4)`` [nfe, accepted, rejected, status] for dopri5, ``None`` for rk4."""
+    launch (8 < D <= 64: one sequence of launches of the large-D kernels, every launch covering all draws; draw q's
+    trajectories and stats are bitwise those of the single-draw call). ``stats``: device int32 ``(n,4)`` [nfe,
+    accepted, rejected, status] for dopri5, ``None`` for rk4."""
     if torch.is_grad_enabled() and any(a.requires_grad for a in (x0, Z, ell, var, nu)):
         raise _lib.GpodeError("the batched (sets) path is forward only: call it under torch.no_grad()")
     lib = _lib.load()
@@ -906,10 +947,23 @@ def integrate_sets(x0, t, Z, ell, var, nu, omega, phase, w, method="dopri5", rto
     Tg = t.shape[0]
     xs = torch.empty(Tg, pcs.n * N, pcs.D, dtype=torch.float32, device=xc.device)
     stats = None
-    if method == "rk4":
+    if method == "rk4" and pcs.large:
+        tc = f32(t.to(device=xc.device, dtype=torch.float32), "t")
+        tmp = torch.empty(6 * pcs.n * N * pcs.D, dtype=torch.float32, device=xc.device)
+        _lib.call("gpode_rk4_fwd_large_sets", ptr(pcs.packed), ctypes.byref(pcs.struct), pcs.n, N, ptr(xc), ptr(tc), Tg,
+                  ptr(xs), ptr(tmp), stream_ptr())
+        _lib.LAUNCH_COUNT["gpode_rk4_fwd_large_sets"] += 12 * max(Tg - 2, 0)   # counted once per call: the other steps
+    elif method == "rk4":
         tc = f32(t.to(device=xc.device, dtype=torch.float32), "t")
         _lib.call("gpode_rk4_fwd_sets", ptr(pcs.packed), pcs.D, pcs.M, pcs.S, pcs.n, N, ptr(xc), ptr(tc), Tg, ptr(xs),
                   stream_ptr())
+    elif method == "dopri5" and pcs.large:
+        t64 = t.detach().to(device=xc.device, dtype=torch.float64).contiguous()
+        work = torch.empty(lib.gpode_dopri5_large_sets_work_floats(pcs.D, pcs.n, N), dtype=torch.float32,
+                           device=xc.device)
+        stats = torch.zeros(pcs.n, 4, dtype=torch.int32, device=xc.device)
+        _lib.call("gpode_dopri5_fwd_large_sets", ptr(pcs.packed), ctypes.byref(pcs.struct), pcs.n, N, ptr(xc), ptr(t64),
+                  Tg, float(rtol), float(atol), ptr(xs), ptr(work), ptr(stats), 100000, stream_ptr())
     elif method == "dopri5":
         t64 = t.detach().to(device=xc.device, dtype=torch.float64).contiguous()
         work = torch.empty(lib.gpode_dopri5_work_floats(pcs.D, pcs.n * N), dtype=torch.float32, device=xc.device)

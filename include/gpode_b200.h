@@ -199,6 +199,28 @@ int gpode_rk4_fwd_sets(const float* packed, int D, int M, int S, int n_sets, int
 int gpode_dopri5_fwd_sets(const float* packed, int D, int M, int S, int n_sets, int64_t set_rows, const float* x0,
                           const double* t, int Tg, double rtol, double atol, float* xs, float* work,
                           int32_t* stats_out, void* stream);
+/* The same for 8 < D <= GPODE_MAX_D_LARGE, on the large-D kernels with a draw index (forward only):
+ *   gpode_pack_cache_large_sets: n_sets blocks of gpode_packed_large_floats(D,M,S) floats back to back (at M = 100,
+ *     S = 256: 0.81 / 2.7 / 9.6 MB per draw for D = 16 / 32 / 64, so 128 draws at D = 64 take 1.2 GB).
+ *   gpode_vf_fwd_large_sets: f = vf(x) of draw q on its set_rows rows; tmp: n_sets set_rows D floats. A 128-row tile
+ *     never straddles two draws (a draw's last tile is ragged); f[q] is bitwise gpode_rff_fwd_large +
+ *     gpode_rbf_fwd_large (or gpode_vf_fwd_large_add_rbf) on draw q alone.
+ *   gpode_rk4_fwd_large_sets: gpode_rk4_fwd_large_dev over all n_sets set_rows rows with that field; xs
+ *     [Tg, n_sets set_rows, D]; tmp: 6 n_sets set_rows D floats.
+ *   gpode_dopri5_fwd_large_sets: gpode_dopri5_fwd_large with one controller per draw (element-wise kernels on a
+ *     (blocks, draws) grid, one controller CTA per draw, the while loop runs until every draw is done; the tiles of a
+ *     finished draw are skipped). Draw q's rows of xs and its stats_out[q] ([n_sets,4] int32) are bitwise those of
+ *     gpode_dopri5_fwd_large on draw q alone. work: gpode_dopri5_large_sets_work_floats(D, n_sets, set_rows) floats.
+ *     Cannot be called inside a stream capture. */
+int gpode_pack_cache_large_sets(const gpode_cache_t* cache_sets, int n_sets, float* packed_large, void* stream);
+int gpode_vf_fwd_large_sets(const float* packed_large, const gpode_cache_t* cache_sets, int n_sets, int64_t set_rows,
+                            const float* x, float* tmp, float* f, void* stream);
+int gpode_rk4_fwd_large_sets(const float* packed_large, const gpode_cache_t* cache_sets, int n_sets, int64_t set_rows,
+                             const float* x0, const float* t, int Tg, float* xs, float* tmp, void* stream);
+int64_t gpode_dopri5_large_sets_work_floats(int D, int n_sets, int64_t set_rows);
+int gpode_dopri5_fwd_large_sets(const float* packed_large, const gpode_cache_t* cache_sets, int n_sets,
+                                int64_t set_rows, const float* x0, const double* t, int Tg, double rtol, double atol,
+                                float* xs, float* work, int32_t* stats_out, int max_attempts, void* stream);
 
 /* ---- ELBO side terms either side of the integrator (SURVEY.md section 8f items 1-2) -------------------------------
  * Full-rank Gaussian state posteriors N(mean_r, L_r L_r^T + jitter I), r < R, L_r given as the PACKED lower triangle

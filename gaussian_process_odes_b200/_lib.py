@@ -74,6 +74,7 @@ SIGNATURES = {
     "gpode_dopri5_bwd_large": (_I, [_P, _CP, _P, _I, _L, _P, _P, _I, _I, _P, _P, _P, _P]),
     "gpode_shoot_fwd": (_I, [_P, _I, _I, _I, ctypes.POINTER(GpodeShoot), _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "gpode_shoot_bwd": (_I, [_P, _I, _I, _I, ctypes.POINTER(GpodeShoot), _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "gpode_shoot_bwd_vrows": (_L, [_I, _I, _I, _L]),
     "gpode_acc_header_floats": (_L, []),
     "gpode_probe_fp32_fma": (_I, [ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double), _P, _P]),
     "gpode_dopri5_ckpt_floats": (_L, [_I, _L, _I, _I]),

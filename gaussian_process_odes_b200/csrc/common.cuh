@@ -119,23 +119,30 @@ __host__ __device__ inline GpodeLayout gpode_layout(int D, int M, int S) {
 // Accumulator block of the backward kernels. Shared-parameter gradients contract over every row of the batch; to keep
 // them BITWISE REPRODUCIBLE (no floating-point atomics anywhere) each CTA writes its partial sums to a row of its own
 // and gpode_grads_finalize adds the rows up in row order, in float64:
-//   [0, 4)            header (int32): hdr[0] = AV rows written, hdr[1] = TW rows written (zeroed by the caller)
+//   [0, 4)            header (int32): hdr[0] = AV rows written, hdr[1] = TW rows written, hdr[2] = RS rows written
+//                                     (zeroed by the caller)
 //   av rows           cap_av x (D*D + D):   A[k][j] | V[k]            one row per CTA of the adjoint / VJP kernel
 //   tw rows           cap_tw x M*(D + D*D): per inducing point m:  T[k] (k < D) | W[j][k] (j, k < D)
 //                                           one row per CTA (blockIdx.x) of param_grad_kernel
+//   OR rs rows        float64, M*2D each:   per inducing point m:  2 ln2 T[k] (k < D) | sum d_j tq_j (j < D)
+//                                           one row per CTA of the tensor-core shooting adjoint that sums the
+//                                           inducing-point gradients itself (rk4_bwd_mma_kernel<D, true, true>);
+//                                           they take the place of the tw rows (hdr[2] > 0 selects this form)
 #define GPODE_ACC_HDR 4
 #define GPODE_ACC_CAP_AV 4096
 #define GPODE_ACC_CAP_TW 1024
 struct GpodeAcc {
-    int n_av, n_tw_m;  // floats per AV row; floats per inducing point of a TW row
-    int64_t off_av, off_tw, total;
+    int n_av, n_tw_m, n_rs_m;  // floats per AV row; floats per inducing point of a TW row; doubles per m of an RS row
+    int64_t off_av, off_tw, off_rs, total;  // in floats; off_rs is even (8-byte aligned doubles)
 };
 __host__ __device__ inline GpodeAcc gpode_acc_layout(int D, int M) {
     GpodeAcc a;
     a.n_av = D * D + D;
     a.n_tw_m = D + D * D;
+    a.n_rs_m = 2 * D;
     a.off_av = GPODE_ACC_HDR;
     a.off_tw = a.off_av + (int64_t)GPODE_ACC_CAP_AV * a.n_av;
+    a.off_rs = a.off_tw;  // one row of 4 D M floats per SM at most: well inside the cap_tw x M (D + D^2) floats
     a.total = a.off_tw + (int64_t)GPODE_ACC_CAP_TW * M * a.n_tw_m;
     return a;
 }

@@ -18,7 +18,8 @@
                               int*, cudaStream_t);                                                                  \
     int gpode_shoot_bwd_d##D_(const float*, int, int, const float*, int64_t, const float*, const float*, float*,    \
                               float*, float*, const float*, const float*, const float*, float*, int64_t, int64_t,   \
-                              cudaStream_t);
+                              cudaStream_t);                                                                        \
+    bool gpode_shoot_row_sums_d##D_(int, int, int64_t);
 GPODE_FOR_EACH_D(GPODE_DECL)
 #undef GPODE_DECL
 
@@ -234,6 +235,20 @@ extern "C" int gpode_shoot_fwd(const float* packed, int D, int M, int S, const g
     return 0;
 }
 
+static bool shoot_row_sums(int D, int M, int S, int64_t B) {
+    switch (D) {
+#define CASE(D_) case D_: return gpode_shoot_row_sums_d##D_(M, S, B);
+        GPODE_FOR_EACH_D(CASE)
+#undef CASE
+        default: return false;
+    }
+}
+
+extern "C" int64_t gpode_shoot_bwd_vrows(int D, int M, int S, int64_t n_rows) {
+    if (D < 1 || D > GPODE_MAX_D || M < 1 || S < 1 || n_rows < 0) return -1;
+    return shoot_row_sums(D, M, S, n_rows) ? 0 : 4 * n_rows;
+}
+
 extern "C" int gpode_shoot_bwd(const float* packed, int D, int M, int S, const gpode_shoot_t* sh, const float* ss,
                                const float* t2, const float* kstages, const float* seeds, const float* g_ll,
                                const float* g_cons, float* grad_ss, float* vrows, float* acc, void* stream) {
@@ -241,15 +256,19 @@ extern "C" int gpode_shoot_bwd(const float* packed, int D, int M, int S, const g
     const int64_t B = sh->row_hi - sh->row_lo;
     if (int rc = check_common(packed, D, M, S, B)) return rc;
     if (B == 0) return 0;
-    GPODE_CHECK_ARG(ss && t2 && kstages && seeds && g_ll && g_cons && grad_ss && vrows && acc, "NULL argument");
+    GPODE_CHECK_ARG(ss && t2 && kstages && seeds && g_ll && g_cons && grad_ss && acc, "NULL argument");
+    GPODE_CHECK_ARG(vrows != nullptr || shoot_row_sums(D, M, S, B),
+                    "vrows is NULL, but this configuration needs %lld virtual rows (gpode_shoot_bwd_vrows)",
+                    (long long)(4 * B));
     const int64_t VR = 4 * B, n_total = (int64_t)sh->S_mc * sh->N * sh->T;
     const float* x0 = ss + sh->row_lo * D;
     cudaStream_t st = (cudaStream_t)stream;
+    float* vk = vrows ? vrows + VR * D : nullptr;
     switch (D) {
 #define CASE(D_)                                                                                                   \
     case D_:                                                                                                       \
-        return gpode_shoot_bwd_d##D_(packed, M, S, t2, B, x0, kstages, vrows, vrows + VR * D, acc, seeds, g_ll,     \
-                                     g_cons, grad_ss, sh->row_lo, n_total, st);
+        return gpode_shoot_bwd_d##D_(packed, M, S, t2, B, x0, kstages, vrows, vk, acc, seeds, g_ll, g_cons,         \
+                                     grad_ss, sh->row_lo, n_total, st);
         GPODE_FOR_EACH_D(CASE)
 #undef CASE
         default: break;

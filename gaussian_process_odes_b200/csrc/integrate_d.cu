@@ -42,3 +42,4 @@ int GPODE_CAT(gpode_shoot_bwd_d, GPODE_D)(const float* packed, int M, int S, con
     sb.seeds = seeds; sb.g_ll = g_ll; sb.g_cons = g_cons; sb.grad_ss = grad_ss; sb.row_lo = row_lo; sb.n_total = n_total;
     return launch_rk4_bwd<GPODE_D, true>(packed, M, S, t, 2, B, x0, kst, nullptr, nullptr, vy, vk, acc, st, sb);
 }
+bool GPODE_CAT(gpode_shoot_row_sums_d, GPODE_D)(int M, int S, int64_t B) { return use_mma_row_sums<GPODE_D>(M, S, B); }

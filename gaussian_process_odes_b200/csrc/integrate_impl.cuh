@@ -598,7 +598,9 @@ vf_bwd_warp_kernel(const float* __restrict__ packed, const int M, const int S, c
 // ---- tensor-core adjoint kernels (vjp_mma.cuh) -------------------------------------------------------------------
 // One CTA of kHWarps warps per SM (the f16 operand records take ~92 KB at D = 5, S = 256, so they are staged once per
 // SM); a warp owns 32 rows, lane = row.
-// dynamic shared memory: [0,16) mbarrier | [kern | il] | mmah records | (D*D + D) block-reduction floats | per-warp stage
+// dynamic shared memory: [0,16) mbarrier | [kern | il] | mmah records | (D*D + D) block-reduction floats | per-warp stage;
+// the RK4 adjoint drops the block-reduction floats (its reduction reuses the per-warp row state, dead by then) and
+// appends the per-warp row state and, when it sums the inducing-point gradients itself, the per-warp row sums
 #ifndef GPODE_HWARPS
 #define GPODE_HWARPS 12
 #endif
@@ -609,18 +611,24 @@ struct HParams {
     int M, S8P, off_kern, n_small, off_mmah, n_mmah;
 };
 
+constexpr int kHRowFields = 7;  // rk4_bwd_mma_kernel: adjoint state per row kept in shared memory (D floats each)
 template <int D>
 struct HSmem {
     const float* small;
     const uint32_t* mmah;
     float* red;
     float* stage;
-    __device__ __forceinline__ HSmem(unsigned char* smem_raw, const HParams& p) {
+    float* rows;  // rk4 adjoint: kHWarps x kHRowFields x D x 32 floats of row state, then kHWarps x M x 2D row sums
+    __device__ __forceinline__ HSmem(unsigned char* smem_raw, const HParams& p, const bool rk4 = false) {
         float* sp = reinterpret_cast<float*>(smem_raw + 16);
         small = sp;
         mmah = reinterpret_cast<const uint32_t*>(sp + p.n_small);
-        red = sp + p.n_small + p.n_mmah;
-        stage = red + kRedFloats<D> + (threadIdx.x >> 5) * HShape<D>::kStageFloats;
+        float* q = sp + p.n_small + p.n_mmah;
+        red = q;
+        if (!rk4) q += kRedFloats<D>;
+        stage = q + (threadIdx.x >> 5) * HShape<D>::kStageFloats;
+        rows = q + kHWarps * HShape<D>::kStageFloats;
+        if (rk4) red = rows;  // kHWarps * kHRowFields * D * 32 >= kRedFloats<D>
     }
 };
 
@@ -745,8 +753,9 @@ rk4_fwd_h_kernel(const float* __restrict__ packed, const HParams p, const float*
 // VJP runs (lambda, y, k1, k2 and the three running cotangent sums: 7 D floats per row) rests in shared memory
 // ([field][component][lane], conflict-free), so the VJP has the 168 registers of a 12-warp CTA to itself -- with that
 // state in registers ptxas spilled inside the VJP loops (3.82 ms; 8 warps at 239 registers: 3.69 ms).
-constexpr int kHRowFields = 7;
-template <int D, bool kShoot = false>
+// kRowSums: no virtual rows; the VJPs sum the inducing-point gradients over the warp's rows (vf_vjp_h) into a per-warp
+// shared-memory accumulator, and the CTA adds its warps in warp order, in float64, into its row-sum row of `acc`.
+template <int D, bool kShoot = false, bool kRowSums = false>
 __global__ void __launch_bounds__(kHThreads, 1)
 rk4_bwd_mma_kernel(const float* __restrict__ packed, const HParams p, const float* __restrict__ ts, const int Tg,
                    const int64_t B, const float* __restrict__ xs, const float* __restrict__ kst,
@@ -754,14 +763,20 @@ rk4_bwd_mma_kernel(const float* __restrict__ packed, const HParams p, const floa
                    float* __restrict__ vk, float* __restrict__ acc, const ShootBwd sb) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     stage_params_h(smem_raw, packed, p.off_kern, p.n_small, p.off_mmah, p.n_mmah);
-    const HSmem<D> sm(smem_raw, p);
+    const HSmem<D> sm(smem_raw, p, true);
     HAcc<D> qa;
     qa.clear();
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     constexpr int R = 1;
     enum { F_LAM = 0, F_Y = 1, F_K1 = 2, F_K2 = 3, F_SUM = 4, F_YB4 = 5, F_Y23 = 6 };
-    float* __restrict__ rs = sm.red + kRedFloats<D> + kHWarps * HShape<D>::kStageFloats +
-                             warp * (kHRowFields * D * 32) + lane;
+    float* __restrict__ rs = sm.rows + warp * (kHRowFields * D * 32) + lane;
+    constexpr int NV = 2 * D;
+    float* __restrict__ rsum_all = sm.rows + kHWarps * kHRowFields * D * 32;
+    float* __restrict__ rsum = rsum_all + warp * p.M * NV;
+    if constexpr (kRowSums) {
+        for (int i = lane; i < p.M * NV; i += 32) rsum[i] = 0.f;
+        __syncwarp();
+    }
     auto put = [&](const int f, const float (&v)[R][D]) {
 #pragma unroll
         for (int j = 0; j < D; ++j) rs[(f * D + j) * 32] = v[0][j];
@@ -784,8 +799,6 @@ rk4_bwd_mma_kernel(const float* __restrict__ packed, const HParams p, const floa
         for (int i = Tg - 2; i >= 0; --i) {
             const float h = __fsub_rn(__ldg(ts + i + 1), __ldg(ts + i));
             const float* kb = kst + (int64_t)i * 4 * plane;
-            float* vyi = vy + (int64_t)i * 4 * plane;
-            float* vki = vk + (int64_t)i * 4 * plane;
             float ks[R][D], ys[R][D], kbar[R][D], yb[R][D];
             {
                 float t[R][D];
@@ -827,9 +840,11 @@ rk4_bwd_mma_kernel(const float* __restrict__ packed, const HParams p, const floa
                         }
                     }
                 }
-                store_rows<D, R>(ys, vyi + (int64_t)(st - 1) * plane, row0, B, 0);
-                store_rows<D, R>(kbar, vki + (int64_t)(st - 1) * plane, row0, B, 0);
-                vf_vjp_h<D>(sm.small, sm.mmah, sm.stage, p.M, p.S8P, ys, kbar, ks, yb, qa, lane);
+                if constexpr (!kRowSums) {
+                    store_rows<D, R>(ys, vy + ((int64_t)i * 4 + st - 1) * plane, row0, B, 0);
+                    store_rows<D, R>(kbar, vk + ((int64_t)i * 4 + st - 1) * plane, row0, B, 0);
+                }
+                vf_vjp_h<D, kRowSums>(sm.small, sm.mmah, sm.stage, p.M, p.S8P, ys, kbar, ks, yb, qa, lane, rsum);
                 float lam[R][D];
                 get(F_LAM, lam);
                 if (st == 4) {
@@ -879,7 +894,17 @@ rk4_bwd_mma_kernel(const float* __restrict__ packed, const HParams p, const floa
         if constexpr (kShoot) shoot_store_grad<D, R>(lam, sb, row0, B, 0);
         else store_rows<D, R>(lam, gx0, row0, B, 0);
     }
-    hacc_reduce<D>(qa, sm.small, p.M, acc, sm.red);
+    hacc_reduce<D>(qa, sm.small, p.M, acc, sm.red);   // its barrier also orders every warp's row sums before the reads
+    if constexpr (kRowSums) {
+        const GpodeAcc a = gpode_acc_layout(D, p.M);
+        double* __restrict__ row = reinterpret_cast<double*>(acc + a.off_rs) + (size_t)blockIdx.x * p.M * NV;
+        for (int i = threadIdx.x; i < p.M * NV; i += blockDim.x) {
+            double s = 0.0;
+            for (int w = 0; w < kHWarps; ++w) s += (double)rsum_all[w * p.M * NV + i];
+            row[i] = s;
+        }
+        if (blockIdx.x == 0 && threadIdx.x == 0) reinterpret_cast<int*>(acc)[2] = (int)gridDim.x;
+    }
 }
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -975,9 +1000,20 @@ inline HParams h_params(const GpodeLayout& L) {
     return p;
 }
 template <int D>
-inline size_t h_smem(const HParams& p, bool rk4 = true, int warps = kHWarps) {
-    return 16 + ((size_t)p.n_small + p.n_mmah + kRedFloats<D> + (size_t)warps * HShape<D>::kStageFloats +
-                 (rk4 ? (size_t)warps * kHRowFields * D * 32 : 0)) * 4;
+inline size_t h_smem(const HParams& p, bool rk4 = true, int warps = kHWarps, bool row_sums = false) {
+    return 16 + ((size_t)p.n_small + p.n_mmah + (rk4 ? 0 : kRedFloats<D>) + (size_t)warps * HShape<D>::kStageFloats +
+                 (rk4 ? (size_t)warps * kHRowFields * D * 32 : 0) + (row_sums ? (size_t)warps * p.M * 2 * D : 0)) * 4;
+}
+// The shooting adjoint sums the inducing-point gradients inside the tensor-core kernel (no virtual rows, no
+// gpode_param_grad) when that kernel is selected and its per-warp row sums fit in shared memory next to the operand
+// records: at S = 256, D = 5 up to M = 101 inducing points, D = 4 up to M = 201.
+template <int D>
+inline bool use_mma_row_sums(int M, int S, int64_t B) {
+    if constexpr (kMmaBwd<D>) {
+        return use_mma_bwd(B) && h_smem<D>(h_params<D>(gpode_layout(D, M, S)), true, kHWarps, true) <= 227 * 1024;
+    } else {
+        return false;
+    }
 }
 template <typename K>
 inline int h_grid(K kernel, int64_t B, size_t smem, int* grid, int threads = kHThreads) {
@@ -1097,6 +1133,15 @@ int launch_rk4_bwd(const float* packed, int M, int S, const float* t, int Tg, in
     constexpr int RW = RowsBwd<D>::value;
     if constexpr (kMmaBwd<D>) {
         const HParams hp = h_params<D>(L);
+        if (kShoot && vy == nullptr) {   // no virtual rows: the caller checked use_mma_row_sums (gpode_shoot_bwd)
+            const size_t hs = h_smem<D>(hp, true, kHWarps, true);
+            int grid = 0;
+            if (int rc = h_grid(rk4_bwd_mma_kernel<D, true, true>, B, hs, &grid)) return rc;
+            rk4_bwd_mma_kernel<D, true, true><<<grid, kHThreads, hs, st>>>(packed, hp, t, Tg, B, xs, kst, gxs, gx0,
+                                                                          nullptr, nullptr, acc, sb);
+            GPODE_LAUNCH_CHECK();
+            return 0;
+        }
         if (use_mma_bwd(B) && h_smem<D>(hp) <= 227 * 1024) {
             int grid = 0;
             if (int rc = h_grid(rk4_bwd_mma_kernel<D, kShoot>, B, h_smem<D>(hp), &grid)) return rc;

@@ -208,6 +208,19 @@ grads_finalize_kernel(const int D, const int M, const float* __restrict__ nu, co
     const bool av = (int)blockIdx.x == n_mg;
     const int NE = a.n_tw_m;
     const int m0 = blockIdx.x * kFinM, cnt = av ? 0 : (M - m0 < kFinM ? M - m0 : kFinM);
+    if (!av && hdr[2] > 0) {   // row sums of the tensor-core shooting adjoint (float64 rows, common.cuh)
+        const int NR = a.n_rs_m;
+        const double* __restrict__ rs = reinterpret_cast<const double*>(acc + a.off_rs) + (size_t)m0 * NR;
+        gpode_sum_rows_ordered<kFinPerLane>(rs, (size_t)M * NR, hdr[2], cnt * NR, kFinMaxChunk, &part[0][0], tot);
+        const double inv_2ln2 = 1.0 / (double)(-GPODE_NEG_2LN2);   // the kernel's float factor 2 ln2, exactly
+        for (int i = threadIdx.x; i < cnt * D; i += blockDim.x) {
+            const int mm = i / D, k = i - mm * D;
+            g_nu[k * M + m0 + mm] = (float)((double)var[k] * tot[mm * NR + k] * inv_2ln2);   // var_k T[k][m]
+            // grad_Z[m][j] = sum_k c_km W[k][m][j] / ell_kj^2 = -sum_rows d_j tq_j
+            g_Z[(m0 + mm) * D + k] = (float)(-tot[mm * NR + D + k]);
+        }
+        return;
+    }
     const int chunk = av ? a.n_av : cnt * NE;                       // contiguous floats of every row this CTA adds up
     const int n_rows = av ? hdr[0] : hdr[1];
     const size_t stride = av ? (size_t)a.n_av : (size_t)M * NE;

@@ -94,13 +94,54 @@ __device__ __forceinline__ void gpode_mma_f16_acc(float (&d)[4], const uint32_t 
         : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
 }
 
+// Sum over the warp's lanes of v[i], returned on lane i for i < N (other lanes: unspecified). Each level halves the
+// values a lane holds: the lane keeps the half its lane bit selects and adds the partner's copy of that half, so N = 32
+// values cost 31 shuffles where a butterfly per value costs 160. A pair whose upper value no lane holds (i >= N) takes
+// a plain butterfly; its upper lane ends with a copy that belongs to no i < N. Fixed order: bitwise reproducible.
+template <int N>
+__device__ __forceinline__ float gpode_warp_sum_transposed(float (&v)[32], const int lane) {
+    static_assert(N >= 1 && N <= 32, "one value per lane at most");
+#pragma unroll
+    for (int h = 16; h >= 1; h >>= 1) {
+        const bool up = (lane & h) != 0;
+        float keep[16], recv[16];
+#pragma unroll
+        for (int r = 0; r < h && r < N; ++r) {
+            if (r + h < N) {
+                const float send = up ? v[r] : v[r + h];
+                keep[r] = up ? v[r + h] : v[r];
+                recv[r] = __shfl_xor_sync(0xffffffffu, send, h);
+            } else {
+                keep[r] = v[r];
+                recv[r] = __shfl_xor_sync(0xffffffffu, v[r], h);
+            }
+        }
+#pragma unroll
+        for (int r = 0; r < h && r < N; r += 2) {
+            if (r + 1 < h && r + 1 < N) {
+                const float2 s = fadd2(make_float2(keep[r], keep[r + 1]), make_float2(recv[r], recv[r + 1]));
+                v[r] = s.x;
+                v[r + 1] = s.y;
+            } else {
+                v[r] = keep[r] + recv[r];
+            }
+        }
+    }
+    return v[0];
+}
+
 // xb = J(x)^T kb for the lane's row; parameter partial sums go to `acc`. fst = f(x) from the forward pass.
 // small: staged [kern | il]; mmah: staged f16 operand records (GpodeLayout::mmah); stage: this warp's HShape stage.
-template <int D>
+// kRowSums: the per-inducing-point gradients are summed here as well, over the warp's 32 rows, into the warp's
+// shared-memory accumulator rsum[m][2D] = {2 ln2 sum kb_k K_km (k < D), sum d_j tq_j (j < D)}: grad_nu and grad_Z
+// without the virtual rows and the second kernel (gpode_grads_finalize applies the factors). W[k][m][j] of that kernel
+// is only ever contracted with c_km / ell_kj^2, and sum_k c_km kb_k K_km d_j / ell_kj^2 = -d_j tq_j, the per-m term the
+// cotangent takes anyway; so 2D sums per (row, m) replace its D + D^2 and nothing is recomputed.
+template <int D, bool kRowSums = false>
 __device__ __forceinline__ void vf_vjp_h(const float* __restrict__ small, const uint32_t* __restrict__ mmah,
                                          float* __restrict__ stage, const int M, const int S8P, const float (&x)[1][D],
                                          const float (&kb)[1][D], const float (&fst)[1][D], float (&xb)[1][D],
-                                         HAcc<D>& acc, const int lane) {
+                                         HAcc<D>& acc, const int lane, float* __restrict__ rsum = nullptr) {
     static_assert(D <= GPODE_MMAH_MAX_D, "x_hi | x_hi | x_lo must fit the 16 contraction slots");
     constexpr int KS = VfShape<D>::KS, WP = VfShape<D>::WP, SXS = HShape<D>::SXS;
     const float* __restrict__ kern = small;
@@ -243,7 +284,9 @@ __device__ __forceinline__ void vf_vjp_h(const float* __restrict__ small, const 
         }
         if constexpr (kOdd) acc.Vq[KF].x = fmaf(kbn[D - 1], fst[0][D - 1], acc.Vq[KF].x);
     };
-    auto rbf_step = [&](const int m) {
+    // e0: start of the exponent sums, -inf for the padding steps of the last row-sum group (K = 0: adds nothing)
+    // pz: the step's 2D row-sum values (kRowSums)
+    auto rbf_step = [&](const int m, const float e0, float* __restrict__ pz) {
         float kp_[KS];
         lds_vec<KS>(kp_, kern + m * KS);
         float d[D], dd[D];
@@ -261,12 +304,16 @@ __device__ __forceinline__ void vf_vjp_h(const float* __restrict__ small, const 
         }
 #pragma unroll
         for (int kp = 0; kp < KF; ++kp) {
-            float2 e = make_float2(0.f, 0.f);
+            float2 e = make_float2(e0, e0);
 #pragma unroll
             for (int j = 0; j < D; ++j) e = ffma2(dd[j], wn[j][kp], e);
             const float2 K = make_float2(gpode_ex2(e.x), gpode_ex2(e.y));
-            const float2 cK = fmul2(make_float2(kp_[D + 2 * kp], kp_[D + 2 * kp + 1]), K);
-            const float2 q = fmul2(kb2[kp], cK);   // q' = 2 ln2 kb c K
+            const float2 p = fmul2(kb2[kp], K);    // 2 ln2 kb K
+            const float2 q = fmul2(make_float2(kp_[D + 2 * kp], kp_[D + 2 * kp + 1]), p);   // q' = 2 ln2 kb c K
+            if constexpr (kRowSums) {
+                pz[2 * kp] = p.x;
+                pz[2 * kp + 1] = p.y;
+            }
             acc.Vq[kp] = fadd2(acc.Vq[kp], q);
 #pragma unroll
             for (int j = 0; j < D; ++j) {
@@ -275,10 +322,12 @@ __device__ __forceinline__ void vf_vjp_h(const float* __restrict__ small, const 
             }
         }
         if constexpr (kOdd) {
-            float e = 0.f;
+            float e = e0;
 #pragma unroll
             for (int j = 0; j < D; ++j) e = fmaf(dd[j], wl[j], e);
-            const float q = kbn[D - 1] * (kp_[2 * D - 1] * gpode_ex2(e));
+            const float p = kbn[D - 1] * gpode_ex2(e);
+            const float q = kp_[2 * D - 1] * p;
+            if constexpr (kRowSums) pz[D - 1] = p;
             acc.Vq[KF].x += q;
 #pragma unroll
             for (int j = 0; j < D; ++j) {
@@ -287,7 +336,11 @@ __device__ __forceinline__ void vf_vjp_h(const float* __restrict__ small, const 
             }
         }
 #pragma unroll
-        for (int j = 0; j < D; ++j) xbp[j] = fmaf(d[j], (tq[j].x + tq[j].y) + tl[j], xbp[j]);
+        for (int j = 0; j < D; ++j) {
+            const float t = (tq[j].x + tq[j].y) + tl[j];
+            if constexpr (kRowSums) pz[D + j] = d[j] * t;
+            xbp[j] = fmaf(d[j], t, xbp[j]);
+        }
     };
 
 #pragma unroll 1
@@ -310,8 +363,26 @@ __device__ __forceinline__ void vf_vjp_h(const float* __restrict__ small, const 
             rff_end();
         } else {
             rbf_begin();
+            if constexpr (kRowSums) {
+                // G inducing points per group fill up to 32 values; one transposed warp sum per group leaves value i of
+                // the group on lane i, which adds it to rsum[m0][i] (the group's values are contiguous there)
+                constexpr int NV = 2 * D, G = 32 / NV;
+#pragma unroll 1
+                for (int m0 = 0; m0 < M; m0 += G) {
+                    float v[32];
+#pragma unroll
+                    for (int g = 0; g < G; ++g) {
+                        const bool real = m0 + g < M;
+                        rbf_step(real ? m0 + g : M - 1, real ? 0.f : -INFINITY, v + g * NV);
+                    }
+                    const float s = gpode_warp_sum_transposed<G * NV>(v, lane);
+                    const int i = m0 * NV + lane;
+                    if (lane < G * NV && i < M * NV) rsum[i] += s;
+                }
+            } else {
 #pragma unroll 2
-            for (int m = 0; m < M; ++m) rbf_step(m);
+                for (int m = 0; m < M; ++m) rbf_step(m, 0.f, nullptr);
+            }
         }
     }
     __syncwarp();

@@ -431,11 +431,13 @@ class _ShootStep(torch.autograd.Function):
         g_cons = f32(g_cons, "grad") if g_cons is not None else zero()
         g_ss = torch.empty_like(sc) if ctx.full else torch.zeros_like(sc)
         acc = pc.new_acc()
-        vrows = torch.empty(lib.gpode_vrow_floats(D, 4 * B), dtype=torch.float32, device=dev)
+        # 0 virtual rows: the tensor-core adjoint sums the inducing-point gradients itself (no gpode_param_grad)
+        n_vr = lib.gpode_shoot_bwd_vrows(pc.D, pc.M, pc.S, B)
+        vrows = torch.empty(lib.gpode_vrow_floats(D, n_vr), dtype=torch.float32, device=dev) if n_vr else None
         _lib.call("gpode_shoot_bwd", ptr(pc.packed), pc.D, pc.M, pc.S, ctypes.byref(sh), ptr(sc), ptr(tc), ptr(kst),
                   ptr(seeds), ptr(g_ll), ptr(g_cons), ptr(g_ss), ptr(vrows), ptr(acc), stream_ptr())
-        if B:
-            _lib.call("gpode_param_grad", ptr(pc.packed), pc.D, pc.M, pc.S, ptr(vrows), ptr(vrows[4 * B * D:]), 4 * B,
+        if n_vr:
+            _lib.call("gpode_param_grad", ptr(pc.packed), pc.D, pc.M, pc.S, ptr(vrows), ptr(vrows[n_vr * D:]), n_vr,
                       ptr(acc), stream_ptr())
         g_Z, g_ell, g_var, g_nu = pc.finalize(acc)
         g_lik = (gvar * g_ll).reshape(ctx.var_shape)

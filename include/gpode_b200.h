@@ -340,7 +340,11 @@ int gpode_shoot_fwd(const float* packed, int D, int M, int S, const gpode_shoot_
  * device scalars), writes grad_ss [S_mc,N,T,D] for rows [row_lo, row_hi) -- dynamics plus the constraint's pull on the
  * next state -- and for row row_hi when the range ends inside a sequence (the caller zeroes grad_ss first when the
  * range is not the whole batch); lengthscale / variance partial sums and virtual rows as gpode_rk4_bwd
- * (vrows: gpode_vrow_floats(D, 4 B) floats). Follow with gpode_param_grad over 4 B rows and gpode_grads_finalize. */
+ * (vrows: gpode_vrow_floats(D, 4 B) floats). Follow with gpode_param_grad over 4 B rows and gpode_grads_finalize.
+ * vrows may be NULL when gpode_shoot_bwd_vrows(D, M, S, B) returns 0 (B = row_hi - row_lo): the tensor-core adjoint
+ * (4 <= D <= 5, batches that fill the GPU) then sums the inducing-point gradients itself into `acc`, and only
+ * gpode_grads_finalize follows. */
+int64_t gpode_shoot_bwd_vrows(int D, int M, int S, int64_t n_rows);
 int gpode_shoot_bwd(const float* packed, int D, int M, int S, const gpode_shoot_t* sh, const float* ss, const float* t2,
                     const float* kstages, const float* seeds, const float* g_ll, const float* g_cons, float* grad_ss,
                     float* vrows, float* acc, void* stream);

@@ -43,6 +43,18 @@ CASES = [
     dict(D=2, M=16, S=64, N=4, T=10000, S_mc=4, dt=0.01),
     # tensor-core kernels (D = 5, B >= 56 832)
     dict(D=5, M=100, S=256, N=2, T=6000, S_mc=5, D_obs=50, dt=0.01, ell0=1.25),
+    # the other state dimensions, warp per row
+    dict(D=1, M=9, S=33, N=2, T=9, S_mc=3),
+    dict(D=4, M=33, S=100, N=2, T=13, S_mc=2),
+    dict(D=6, M=21, S=47, N=1, T=17, S_mc=3),
+    dict(D=7, M=17, S=41, N=2, T=6, S_mc=2, D_obs=9),
+    dict(D=8, M=30, S=64, N=2, T=5, S_mc=3),
+    # ... and one row per thread: just above 16 384 rows, below the wide and the tensor-core kernels
+    dict(D=1, M=9, S=33, N=3, T=2731, S_mc=2, dt=0.01),
+    dict(D=4, M=33, S=100, N=3, T=3001, S_mc=2, dt=0.01),
+    dict(D=6, M=21, S=47, N=2, T=4201, S_mc=2, dt=0.01),
+    dict(D=7, M=17, S=41, N=3, T=3001, S_mc=2, D_obs=9, dt=0.01),
+    dict(D=8, M=30, S=64, N=3, T=3001, S_mc=2, dt=0.01),
 ]
 
 
@@ -107,12 +119,23 @@ def test_time_sharded_terms_and_gradients_add_up(kw, world):
         assert relerr(g_sum[k], g_all[k]) <= 2e-5, (k, relerr(g_sum[k], g_all[k]))
 
 
-def test_fused_step_against_the_oracle_at_medium_batch():
-    """18 000 segments (row-per-thread kernels) against the oracle port with the float64 arbiter."""
-    kw = dict(D=3, M=24, S=64, N=3, T=3000, S_mc=2, D_obs=7, dt=0.01)
-    rows = elbo_errors("shooting", kw, "rk4", {}, 9)
+def _assert_matches_oracle(kw, seed):
+    rows = elbo_errors("shooting", kw, "rk4", {}, seed)
     for k, (e_cuda64, e_ref64, e_cuda32) in rows.items():
         assert e_cuda32 <= TOL_GRAD or e_cuda64 <= max(TOL_GRAD, 1.5 * e_ref64), (k, e_cuda64, e_ref64, e_cuda32)
+
+
+def test_fused_step_against_the_oracle_at_medium_batch():
+    """18 000 segments (row-per-thread kernels) against the oracle port with the float64 arbiter."""
+    _assert_matches_oracle(dict(D=3, M=24, S=64, N=3, T=3000, S_mc=2, D_obs=7, dt=0.01), 9)
+
+
+@pytest.mark.parametrize("kw", [k for k in CASES if k['D'] in (4, 7) and k['S_mc'] * k['N'] * k['T'] > 16384],
+                         ids=lambda k: "D%d_B%d" % (k['D'], k['S_mc'] * k['N'] * k['T']))
+def test_fused_step_against_the_oracle_at_even_and_odd_d(kw):
+    """rk4_fwd_kernel / rk4_bwd_kernel <D, 1, true> at D = 4 (output pairs only) and D = 7 (pairs and the scalar odd
+    output) against the oracle port with the float64 arbiter."""
+    _assert_matches_oracle(kw, 10 + kw['D'])
 
 
 def test_end_points_on_request():

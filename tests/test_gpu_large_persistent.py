@@ -13,18 +13,16 @@ summed). The large ones run on the device, as plain torch ops in float32 and flo
 import numpy as np
 import pytest
 import torch
-from torch.utils.checkpoint import checkpoint
 
 import gpode_oracle as O
-from util import TOL_GRAD, TOL_TRAJ, TOL_VF, assert_parity, oracle_cache, to_dev
+from util import (GRAD_KEYS, TOL_GRAD, TOL_TRAJ, TOL_VF, assert_grads, assert_parity, chunked_oracle, cuda_args,
+                  cuda_grads, lazy, oracle_cache, oracle_dopri5, oracle_rk4, oracle_vf, time_grid)
 
 pytestmark = pytest.mark.gpu
 
 ROWS = 128                # rows per tile of the tcgen05 kernels, vjp_large_kernel and rbf_vjp_large_kernel
 SMEM = 227 * 1024         # the launchers' shared-memory limit per CTA
 LD_THREADS = 2368 * 256   # ld_grid (large_dopri5.cu): at most 2368 blocks x 256 threads, grid-stride over B * D
-CHUNK = 4096              # oracle rows per chunk
-KEYS = ("x", "Z", "ell", "var", "nu")
 
 
 def _sms():
@@ -115,84 +113,8 @@ def _setup(D, M, S, B, seed, nu_scale=0.1):
     return gp, c, x
 
 
-def _cuda_args(gp, c, grad=False):
-    d = to_dev(dict(Z=gp['Z'], ell=gp['ell'], var=gp['var'], nu=c['nu'], omega=c['rff_omega'], phase=c['rff_phase'],
-                    w=c['rff_weights']))
-    return [d[k].float().contiguous().requires_grad_(grad and i < 4)
-            for i, k in enumerate(("Z", "ell", "var", "nu", "omega", "phase", "w"))]
-
-
-def _cuda_grads(fn, gp, c, x, cot):
-    args = _cuda_args(gp, c, True)
-    xc = x.cuda().requires_grad_(True)
-    out = fn(xc, args)
-    out.backward(cot.cuda())
-    return out.detach(), dict(x=xc.grad, Z=args[0].grad, ell=args[1].grad, var=args[2].grad, nu=args[3].grad)
-
-
-def _leaves(gp, c, x, dtype, dev):
-    leaves = dict(x=x.to(dev, dtype).clone().requires_grad_(True))
-    for k in ("Z", "ell", "var"):
-        leaves[k] = gp[k].to(dev, dtype).clone().requires_grad_(True)
-    leaves['nu'] = c['nu'].to(dev, dtype).clone().requires_grad_(True)
-    # omega = eps / ell stays attached to ell (kernels.py:110-112): rebuild it from eps
-    eps = (c['rff_omega'].double() * gp['ell'].double().T.unsqueeze(1)).to(dev, dtype)
-    cc = dict(rff_omega=eps / leaves['ell'].T.unsqueeze(1), rff_phase=c['rff_phase'].to(dev, dtype),
-              rff_weights=c['rff_weights'].to(dev, dtype), nu=leaves['nu'])
-    return leaves, cc
-
-
-def _vf(l, cc, y):
-    return O.vf_forward(y, l['Z'], l['ell'], l['var'], cc)
-
-
-def _rk4(ts):
-    return lambda l, cc: O.odeint(lambda t, y: _vf(l, cc, y), l['x'], ts.to(l['x']), method='rk4')
-
-
-def chunked_oracle(fn, gp, c, x, cot, dtype, row_dim, dev="cuda"):
-    """fn(leaves, cache) over row chunks of x: -> (output, {x, Z, ell, var, nu: gradient of (output * cot).sum()}) with
-    the outputs and x-gradients concatenated and the parameter gradients summed over chunks (in float64). Exact for a
-    row-separable fn (the vector field, fixed-grid RK4)."""
-    outs, gx, gsum = [], [], {}
-    for r0 in range(0, x.shape[0], CHUNK):
-        l, cc = _leaves(gp, c, x[r0:r0 + CHUNK], dtype, dev)
-        out = fn(l, cc)
-        out.backward(cot.narrow(row_dim, r0, l['x'].shape[0]).to(dev, dtype))
-        outs.append(out.detach().cpu())
-        gx.append(l['x'].grad.cpu())
-        for k in KEYS[1:]:
-            g = l[k].grad.double().cpu()
-            gsum[k] = gsum[k] + g if k in gsum else g
-    grads = {k: v.to(dtype) for k, v in gsum.items()}
-    grads['x'] = torch.cat(gx)
-    return torch.cat(outs, row_dim), grads
-
-
-def lazy(fn):
-    memo = []
-
-    def get():
-        if not memo:
-            memo.append(fn())
-        return memo[0]
-    return get
-
-
-def assert_grads(name, got, ref32, ref64, tol):
-    for k in KEYS:
-        assert_parity("%s grad %s" % (name, k), got[k].cpu().reshape(ref32[k].shape), ref32[k],
-                      lambda k=k: ref64()[k], tol)
-
-
 def _tile_rows(tiles, B):
     return torch.cat([torch.arange(t * ROWS, min((t + 1) * ROWS, B)) for t in tiles])
-
-
-def _grid(Tg, h, seed):
-    rng = np.random.default_rng(seed)
-    steps = h * (1 + 0.3 * rng.uniform(-1, 1, size=Tg - 1))
-    return torch.tensor(np.concatenate([[0.0], np.cumsum(steps)]), dtype=torch.float32)
 
 
 # ---- forward ----------------------------------------------------------------------------------------------------------
@@ -205,8 +127,8 @@ def test_forward_multi_tile_equals_single_tile_launches_and_oracle(D, M, S, tail
     ctas = max(rff_fwd_ctas(D), rbf_fwd_ctas_max(D, M))
     B = multi_tile_batch(ctas, tail)
     gp, c, x = _setup(D, M, S, B, seed=D + 5)
-    args = _cuda_args(gp, c)
-    ts = _grid(3, 0.05, D)
+    args = cuda_args(gp, c)
+    ts = time_grid(3, 0.05, D)
     xc = x.cuda()
     with torch.no_grad():
         f = ops.vector_field(xc, *args)
@@ -253,13 +175,12 @@ def test_vjp_multi_tile_matches_chunked_oracle(D, M, S, tail):
     gp, c, x = _setup(D, M, S, B, seed=D + 11)
     cot = torch.tensor(np.random.default_rng(D).normal(size=(B, D)), dtype=torch.float32)
     fn = lambda xc, a: ops.vector_field(xc, *a)
-    f, got = _cuda_grads(fn, gp, c, x, cot)
-    _, again = _cuda_grads(fn, gp, c, x, cot)
-    for k in KEYS:
+    f, got = cuda_grads(fn, gp, c, x, cot)
+    _, again = cuda_grads(fn, gp, c, x, cot)
+    for k in GRAD_KEYS:
         assert torch.equal(got[k], again[k]), "two backward passes differ in grad " + k
-    vf = lambda l, cc: _vf(l, cc, l['x'])
-    out32, ref32 = chunked_oracle(vf, gp, c, x, cot, torch.float32, 0)
-    ref64 = lazy(lambda: chunked_oracle(vf, gp, c, x, cot, torch.float64, 0))
+    out32, ref32 = chunked_oracle(oracle_vf, gp, c, x, cot, torch.float32, 0)
+    ref64 = lazy(lambda: chunked_oracle(oracle_vf, gp, c, x, cot, torch.float64, 0))
     assert_parity("multi-tile vf D=%d" % D, f.cpu(), out32, lambda: ref64()[0], TOL_VF)
     assert_grads("multi-tile vf D=%d" % D, got, ref32, lambda: ref64()[1], TOL_GRAD)
 
@@ -270,28 +191,16 @@ def test_rk4_backward_multi_tile_matches_chunked_oracle(D, M, S, tail):
     from gaussian_process_odes_b200 import ops
     B = _vjp_batch(D)
     gp, c, x = _setup(D, M, S, B, seed=D + 17)
-    ts = _grid(3, 0.05, 3)
+    ts = time_grid(3, 0.05, 3)
     cot = torch.tensor(np.random.default_rng(D + 1).normal(size=(3, B, D)), dtype=torch.float32)
-    xs, got = _cuda_grads(lambda xc, a: ops.rk4_integrate(xc, ts.cuda(), *a), gp, c, x, cot)
-    out32, ref32 = chunked_oracle(_rk4(ts), gp, c, x, cot, torch.float32, 1)
-    ref64 = lazy(lambda: chunked_oracle(_rk4(ts), gp, c, x, cot, torch.float64, 1))
+    xs, got = cuda_grads(lambda xc, a: ops.rk4_integrate(xc, ts.cuda(), *a), gp, c, x, cot)
+    out32, ref32 = chunked_oracle(oracle_rk4(ts), gp, c, x, cot, torch.float32, 1)
+    ref64 = lazy(lambda: chunked_oracle(oracle_rk4(ts), gp, c, x, cot, torch.float64, 1))
     assert_parity("multi-tile rk4 D=%d" % D, xs.cpu(), out32, lambda: ref64()[0], TOL_TRAJ)
     assert_grads("multi-tile rk4 D=%d" % D, got, ref32, lambda: ref64()[1], TOL_GRAD)
 
 
 # ---- dopri5 -----------------------------------------------------------------------------------------------------------
-def _oracle_dopri5(gp, c, x, ts, cot, dtype):
-    """autograd through the restated dopri5 on the device; every vector-field evaluation is checkpointed (recomputed in
-    the backward pass), so the graph holds one state per evaluation instead of its [D, B, D] intermediates. The error
-    norm spans the whole batch: this oracle is not chunked."""
-    l, cc = _leaves(gp, c, x, dtype, "cuda")
-    st = {}
-    f = lambda t, y: checkpoint(lambda yy: _vf(l, cc, yy), y, use_reentrant=False)
-    out = O.odeint(f, l['x'], ts.cuda().to(dtype), method='dopri5', rtol=1e-6, atol=1e-6, stats=st)
-    (out * cot.to("cuda", dtype)).sum().backward()
-    return out.detach().cpu(), {k: v.grad.detach().cpu() for k, v in l.items()}, st
-
-
 def test_dopri5_grid_stride_kernels_run_several_passes():
     """D = 63, M = 9, S = 16 (one chunk that the features do not fill). B * D > 2 * 2368 * 256: every thread of the ld_*
     kernels (forward controller norms, stage algebra, adjoint stages) makes >= 2 grid-stride passes and its float64
@@ -303,14 +212,14 @@ def test_dopri5_grid_stride_kernels_run_several_passes():
     gp, c, x = _setup(D, M, S, B, seed=63)
     ts = torch.tensor([0.0, 0.05, 0.32], dtype=torch.float32)
     cot = torch.tensor(np.random.default_rng(8).normal(size=(3, B, D)), dtype=torch.float32)
-    args = _cuda_args(gp, c, True)
+    args = cuda_args(gp, c, True)
     xc = x.cuda().requires_grad_(True)
     xs, stats = ops.dopri5_integrate(xc, ts.cuda(), *args)
     (xs * cot.cuda()).sum().backward()
     got = dict(x=xc.grad, Z=args[0].grad, ell=args[1].grad, var=args[2].grad, nu=args[3].grad)
     torch.cuda.reset_peak_memory_stats()
-    out32, ref32, st = _oracle_dopri5(gp, c, x, ts, cot, torch.float32)
-    ref64 = lazy(lambda: _oracle_dopri5(gp, c, x, ts, cot, torch.float64))
+    out32, ref32, st = oracle_dopri5(gp, c, x, ts, cot, torch.float32)
+    ref64 = lazy(lambda: oracle_dopri5(gp, c, x, ts, cot, torch.float64))
     nfe, acc, rej, status = [int(v) for v in stats.cpu()]
     assert status == 0 and nfe == 2 + 6 * (acc + rej)
     assert abs(acc - st['accepted']) <= 1 and abs(rej - st['rejected']) <= 1, (acc, rej, st)

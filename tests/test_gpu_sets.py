@@ -31,7 +31,8 @@ def _shared(gp):
     return [gp[k].cuda().contiguous() for k in ("Z", "ell", "var")]
 
 
-@pytest.mark.parametrize("D,M,S,n,N", [(2, 16, 256, 7, 1), (5, 100, 256, 5, 6), (3, 24, 63, 4, 37), (8, 30, 64, 3, 2)])
+@pytest.mark.parametrize("D,M,S,n,N", [(2, 16, 256, 7, 1), (5, 100, 256, 5, 6), (3, 24, 63, 4, 37), (8, 30, 64, 3, 2),
+                                       (1, 9, 33, 5, 3), (4, 33, 100, 3, 7), (6, 21, 47, 4, 5), (7, 17, 41, 3, 9)])
 def test_vf_sets_matches_per_draw(D, M, S, n, N):
     from gaussian_process_odes_b200 import ops
     gp, sets = _draw_sets(D, M, S, n, seed=D + n)
@@ -66,7 +67,8 @@ def test_whiten_sets_matches_per_draw(D, M, S, n):
 
 
 @pytest.mark.parametrize("method", ["rk4", "dopri5"])
-@pytest.mark.parametrize("D,M,S,n,N", [(2, 16, 256, 6, 1), (5, 100, 256, 3, 6), (3, 24, 64, 4, 11)])
+@pytest.mark.parametrize("D,M,S,n,N", [(2, 16, 256, 6, 1), (5, 100, 256, 3, 6), (3, 24, 64, 4, 11), (1, 9, 33, 5, 3),
+                                       (4, 33, 100, 3, 6), (6, 21, 47, 3, 5), (7, 17, 41, 4, 3), (8, 30, 64, 3, 2)])
 def test_integrate_sets_matches_per_draw(method, D, M, S, n, N):
     from gaussian_process_odes_b200 import ops
     gp, sets = _draw_sets(D, M, S, n, seed=21 + D)

@@ -72,6 +72,107 @@ def oracle_cache(p, draws, dtype=torch.float32):
     return gp, c
 
 
+# ---- gradients of the CUDA ops and of the oracle evaluated over row chunks, on the device --------------------------
+GRAD_KEYS = ("x", "Z", "ell", "var", "nu")
+
+
+def cuda_args(gp, c, grad=False):
+    """the seven cache tensors of the ops in their order, on the device; Z, ell, var and nu require grad if ``grad``"""
+    d = to_dev(dict(Z=gp['Z'], ell=gp['ell'], var=gp['var'], nu=c['nu'], omega=c['rff_omega'], phase=c['rff_phase'],
+                    w=c['rff_weights']))
+    return [d[k].float().contiguous().requires_grad_(grad and i < 4)
+            for i, k in enumerate(("Z", "ell", "var", "nu", "omega", "phase", "w"))]
+
+
+def cuda_grads(fn, gp, c, x, cot):
+    """fn(x, cache args) on the device -> (output, {x, Z, ell, var, nu: gradient of (output * cot).sum()})"""
+    args = cuda_args(gp, c, True)
+    xc = x.cuda().requires_grad_(True)
+    out = fn(xc, args)
+    out.backward(cot.cuda())
+    return out.detach(), dict(x=xc.grad, Z=args[0].grad, ell=args[1].grad, var=args[2].grad, nu=args[3].grad)
+
+
+def oracle_leaves(gp, c, x, dtype, dev):
+    """x, Z, ell, var, nu as leaves in ``dtype`` on ``dev`` and the cache built on them"""
+    leaves = dict(x=x.to(dev, dtype).clone().requires_grad_(True))
+    for k in ("Z", "ell", "var"):
+        leaves[k] = gp[k].to(dev, dtype).clone().requires_grad_(True)
+    leaves['nu'] = c['nu'].to(dev, dtype).clone().requires_grad_(True)
+    # omega = eps / ell stays attached to ell (kernels.py:110-112): rebuild it from eps
+    eps = (c['rff_omega'].double() * gp['ell'].double().T.unsqueeze(1)).to(dev, dtype)
+    cc = dict(rff_omega=eps / leaves['ell'].T.unsqueeze(1), rff_phase=c['rff_phase'].to(dev, dtype),
+              rff_weights=c['rff_weights'].to(dev, dtype), nu=leaves['nu'])
+    return leaves, cc
+
+
+def oracle_vf(l, cc):
+    return O.vf_forward(l['x'], l['Z'], l['ell'], l['var'], cc)
+
+
+def oracle_rk4(ts):
+    return lambda l, cc: O.odeint(lambda t, y: O.vf_forward(y, l['Z'], l['ell'], l['var'], cc), l['x'], ts.to(l['x']),
+                                  method='rk4')
+
+
+def chunked_oracle(fn, gp, c, x, cot, dtype, row_dim, dev="cuda", chunk=4096):
+    """fn(leaves, cache) over row chunks of x: -> (output, {x, Z, ell, var, nu: gradient of (output * cot).sum()}) with
+    the outputs and x-gradients concatenated and the parameter gradients summed over chunks (in float64). Exact for a
+    row-separable fn (the vector field, fixed-grid RK4)."""
+    outs, gx, gsum = [], [], {}
+    for r0 in range(0, x.shape[0], chunk):
+        l, cc = oracle_leaves(gp, c, x[r0:r0 + chunk], dtype, dev)
+        out = fn(l, cc)
+        out.backward(cot.narrow(row_dim, r0, l['x'].shape[0]).to(dev, dtype))
+        outs.append(out.detach().cpu())
+        gx.append(l['x'].grad.cpu())
+        for k in GRAD_KEYS[1:]:
+            g = l[k].grad.double().cpu()
+            gsum[k] = gsum[k] + g if k in gsum else g
+    grads = {k: v.to(dtype) for k, v in gsum.items()}
+    grads['x'] = torch.cat(gx)
+    return torch.cat(outs, row_dim), grads
+
+
+def oracle_dopri5(gp, c, x, ts, cot, dtype, dev="cuda", rtol=1e-6, atol=1e-6):
+    """autograd through the restated dopri5 -> (xs, {x, Z, ell, var, nu: gradient}, accept/reject counts). Every
+    vector-field evaluation is checkpointed (recomputed in the backward pass), so the graph holds one state per
+    evaluation instead of its [D, B, D] intermediates. The error norm spans the whole batch: this oracle is not
+    chunked."""
+    from torch.utils.checkpoint import checkpoint
+    l, cc = oracle_leaves(gp, c, x, dtype, dev)
+    st = {}
+    f = lambda t, y: checkpoint(lambda yy: O.vf_forward(yy, l['Z'], l['ell'], l['var'], cc), y, use_reentrant=False)
+    out = O.odeint(f, l['x'], ts.to(dev, dtype), method='dopri5', rtol=rtol, atol=atol, stats=st)
+    (out * cot.to(dev, dtype)).sum().backward()
+    return out.detach().cpu(), {k: v.grad.detach().cpu() for k, v in l.items()}, st
+
+
+def lazy(fn):
+    """fn() evaluated on the first call only"""
+    memo = []
+
+    def get():
+        if not memo:
+            memo.append(fn())
+        return memo[0]
+    return get
+
+
+def assert_grads(name, got, ref32, ref64, tol):
+    """assert_parity of every gradient; ``ref64``: callable returning the float64 gradients"""
+    for k in GRAD_KEYS:
+        assert_parity("%s grad %s" % (name, k), got[k].cpu().reshape(ref32[k].shape), ref32[k],
+                      lambda k=k: ref64()[k], tol)
+
+
+def time_grid(Tg, h, seed):
+    """Tg float32 points with steps h (1 +- 0.3 u)"""
+    rng = np.random.default_rng(seed)
+    steps = h * (1 + 0.3 * rng.uniform(-1, 1, size=Tg - 1))
+    return torch.tensor(np.concatenate([[0.0], np.cumsum(steps)]), dtype=torch.float32)
+
+
 # ---- building the product model from the shared unconstrained-parameter dict, and injecting random draws ----------
 class _Queue:
     def __init__(self, items, what):

@@ -97,6 +97,10 @@ SIGNATURES = {
     "gpode_rk4_fwd_large_sets": (_I, [_P, _CP, _I, _L, _P, _P, _I, _P, _P, _P]),
     "gpode_dopri5_large_sets_work_floats": (_L, [_I, _I, _L]),
     "gpode_dopri5_fwd_large_sets": (_I, [_P, _CP, _I, _L, _P, _P, _I, _D, _D, _P, _P, _P, _I, _P]),
+    "gpode_whiten_blocked_work_doubles": (_L, [_I, _I, _I]),
+    "gpode_whiten_fwd_blocked": (_I, [_CP, _P, _F, _P, _P, _P, _P, _P]),
+    "gpode_whiten_fwd_sets_blocked": (_I, [_CP, _P, _F, _I, _P, _P, _P, _P, _P]),
+    "gpode_whiten_bwd_blocked": (_I, [_CP, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
 }
 
 _lib = None
@@ -215,10 +219,19 @@ def total_launches():
     return sum(LAUNCH_COUNT.values())
 
 
-def call(name, *args):
-    """Invoke one C-ABI entry point on the current stream, check its return code, count its kernel launches."""
+def whiten_blocked_launches(M, bwd=False):
+    """Kernels enqueued by gpode_whiten_{fwd,fwd_sets,bwd}_blocked at this M (csrc/whiten_blocked.cu): with
+    P = ceil(M / 64) panels, the Cholesky and every triangular solve take 2 P - 1 launches; the forward adds four
+    element-wise kernels to one Cholesky and two solves, the backward five to four solves."""
+    per = 2 * ((M + 63) // 64) - 1
+    return 5 + 4 * per if bwd else 4 + 3 * per
+
+
+def call(name, *args, launches=None):
+    """Invoke one C-ABI entry point on the current stream, check its return code, count its kernel launches
+    (``launches`` for the entry points whose count depends on the shape)."""
     fn = getattr(load(), name)
-    LAUNCH_COUNT[name] = LAUNCH_COUNT.get(name, 0) + KERNELS_PER_CALL[name]
+    LAUNCH_COUNT[name] = LAUNCH_COUNT.get(name, 0) + (KERNELS_PER_CALL[name] if launches is None else launches)
     if _PROFILE is None:
         check(fn(*args))
         return

@@ -21,7 +21,7 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", 
               "-Xcompiler", "-fPIC", "-Xptxas", "-v", "-I", INCLUDE]
 
 # (source, extra defines, object name)
-UNITS = [("pack.cu", [], "pack.o"), ("param_grad.cu", [], "param_grad.o"), ("whiten.cu", [], "whiten.o"),
+UNITS = [("pack.cu", [], "pack.o"), ("param_grad.cu", [], "param_grad.o"), ("whiten.cu", [], "whiten.o"), ("whiten_blocked.cu", [], "whiten_blocked.o"),
          ("integrate.cu", [], "integrate.o"), ("dopri5.cu", [], "dopri5.o"), ("probe.cu", [], "probe.o"), ("side_terms.cu", [], "side_terms.o"), ("large_d.cu", [], "large_d.o"), ("large_umma.cu", [], "large_umma.o"), ("large_bwd.cu", [], "large_bwd.o"), ("large_rffb.cu", [], "large_rffb.o"), ("large_dopri5.cu", [], "large_dopri5.o")] + \
         [("integrate_d.cu", ["-DGPODE_D=%d" % d], "integrate_d%d.o" % d) for d in range(1, 9)] + \
         [("dopri5_d.cu", ["-DGPODE_D=%d" % d], "dopri5_d%d.o" % d) for d in range(1, 9)]

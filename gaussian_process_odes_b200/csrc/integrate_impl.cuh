@@ -926,10 +926,21 @@ inline int num_sms() {
     return g_num_sms;
 }
 
+// A packed block above the 227 KB a CTA can opt into (large M or S) is an argument error, reported before
+// cudaFuncSetAttribute would fail on it and leave its error pending for the next launch check.
+inline int check_smem_fits(size_t smem) {
+    if (smem > 227 * 1024) {
+        gpode_set_error("kernel does not fit on an SM (smem %zu bytes)", smem);
+        return -2;
+    }
+    return 0;
+}
+
 template <typename K>
 inline int shape_for(K kernel, int R, int64_t B, size_t smem, LaunchShape* out) {
     // small batches: narrow CTAs so the rows spread over more SMs; large: 128 threads, grid = SMs x resident CTAs
     int threads = (B <= (int64_t)num_sms() * 32 * R) ? 32 : kThreads;
+    if (int rc = check_smem_fits(smem)) return rc;
     GPODE_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int occ = 0;
     GPODE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, threads, smem));
@@ -957,6 +968,7 @@ constexpr int64_t kWarpPathMaxRows = 16384;
 
 template <typename K>
 inline int warp_shape_for(K kernel, int64_t B, size_t smem, LaunchShape* out) {
+    if (int rc = check_smem_fits(smem)) return rc;
     GPODE_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int occ = 0;
     GPODE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, kWarpsPerCta * 32, smem));

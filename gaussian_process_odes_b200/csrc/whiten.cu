@@ -11,67 +11,22 @@
 // The M x M tiles live in shared memory in float64 (M <= GPODE_MAX_M_F64) or float32 (M <= GPODE_MAX_M): Kzz + 1e-5 I
 // has a condition number around 1e5, so float64 accumulation keeps nu at the float64-arbiter level instead of adding
 // this kernel's round-off on top of the reference's (tests/ arbitrate with the float64 oracle).
-#include "common.cuh"
+#include "whiten.cuh"
 #include <cooperative_groups.h>
-#include <math.h>
 namespace cg = cooperative_groups;
 
 namespace {
 
 __device__ __forceinline__ int ld_for(int M) { return (M & 1) ? M : M + 1; }
 
-// K_k(Z_m, Z_n) in double from the float32 parameters (direct squared-distance form)
-__device__ __forceinline__ double rbf_entry(const float* __restrict__ Z, const double* __restrict__ inv_l, double vark,
-                                            int D, int m, int n) {
-    double e = 0.0;
-    for (int j = 0; j < D; ++j) {
-        const double d = ((double)Z[m * D + j] - (double)Z[n * D + j]) * inv_l[j];
-        e += d * d;
-    }
-    return vark * exp(-0.5 * e);
-}
-
-// p_m = sum_s a_sk cos(theta_msk): one warp per inducing point, lanes over features, float32 angle like the
-// reference (dsvgp.py:131-136) but double accumulation.
+// p_m = rff_forward(Z)_{m,k} for every inducing point: one warp per point (rff_at_point)
 __device__ void rff_at_Z(const gpode_cache_t& c, int k, double* p_out) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
-    const int D = c.D, S = c.S, M = c.M;
-    const float ak = sqrtf(c.var[k] / (float)S);
-    for (int m = warp; m < M; m += nwarps) {
-        double acc = 0.0;
-        for (int s = lane; s < S; s += 32) {
-            float th = c.phase[s * D + k];
-            for (int j = 0; j < D; ++j) th = fmaf(c.Z[m * D + j], c.omega[((size_t)j * S + s) * D + k], th);
-            acc += (double)(c.w[s * D + k] * ak) * (double)gpode_cos_cw(th);   // 9e-8 at any angle, no libm slow path
-        }
-        for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+    const float ak = sqrtf(c.var[k] / (float)c.S);
+    for (int m = warp; m < c.M; m += nwarps) {
+        const double acc = rff_at_point(c, k, m, ak);
         if (lane == 0) p_out[m] = acc;
     }
-}
-
-// In-place right-looking Cholesky of the leading M x M block of A (row-major, leading dim ld); `rows` >= M extra
-// rows below the block are carried along, so row r >= M ends up holding (L^-1 a_r)^T.
-// dinv[c] receives 1 / L_cc: the triangular solves multiply by it instead of dividing (a float64 division is a ~40
-// instruction dependent chain, and the column loop is the critical path of the whole kernel).
-template <typename Real>
-__device__ void chol_inplace(Real* A, int M, int rows, int ld, Real* dinv) {
-    const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5, ny = blockDim.x >> 5;
-    for (int c = 0; c < M; ++c) {
-        __syncthreads();
-        const Real acc_ = A[c * ld + c];
-        const Real inv = rsqrt(acc_);        // one reciprocal square root instead of sqrt + division
-        const Real dcc = acc_ * inv;
-        if (threadIdx.x == 0) dinv[c] = inv;
-        for (int i = c + 1 + ty; i < rows; i += ny) {
-            const Real lic = A[i * ld + c] * inv;
-            const int jmax = i < M ? i : M - 1;
-            for (int j = c + 1 + tx; j <= jmax; j += 32) A[i * ld + j] -= lic * (A[j * ld + c] * inv);
-        }
-        __syncthreads();
-        for (int i = c + 1 + threadIdx.x; i < rows; i += blockDim.x) A[i * ld + c] *= inv;
-        if (threadIdx.x == 0) A[c * ld + c] = dcc;
-    }
-    __syncthreads();
 }
 
 // v <- L^-1 v (warp 0 only; caller syncs the CTA afterwards)
@@ -303,14 +258,8 @@ __global__ void whiten_bwd_kernel(const gpode_cache_t c, const float* __restrict
         const float ak = sqrtf(c.var[k] / (float)S);
         for (int m = warp; m < M; m += nwarps) {
             double G[GPODE_MAX_D];
-            for (int j = 0; j < D; ++j) G[j] = 0.0;
             const double pbm = (double)pb[m];
-            for (int s = lane; s < S; s += 32) {
-                float th = c.phase[s * D + k];
-                for (int j = 0; j < D; ++j) th = fmaf(c.Z[m * D + j], c.omega[((size_t)j * S + s) * D + k], th);
-                const double g = -pbm * (double)(c.w[s * D + k] * ak) * (double)gpode_sin_cw(th);
-                for (int j = 0; j < D; ++j) G[j] += g * (double)c.omega[((size_t)j * S + s) * D + k];
-            }
+            rff_vjp_at_point(c, k, m, pbm, ak, G);
             for (int j = 0; j < D; ++j) {
                 double v = G[j];
                 for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

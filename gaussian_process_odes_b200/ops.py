@@ -136,8 +136,23 @@ class _RK4(torch.autograd.Function):
         return gx0, None, g_Z, g_ell, g_var, g_nu.reshape(ctx.nu_shape), None, None, None, None
 
 
+MAX_M = 160           # GPODE_MAX_M: whitening in one CTA's shared memory (gpode_whiten_fwd / _bwd)
+MAX_M_BLOCKED = 2048  # GPODE_MAX_M_BLOCKED: blocked float64 whitening above MAX_M (gpode_whiten_*_blocked)
+
+
+def _whiten_work(D, M, n_sets, device):
+    """float64 workspace of the blocked whitening (n_sets = 0: the backward's); a caching-allocator tensor, so the
+    call stays capturable in a CUDA graph. Raises GpodeError naming the limit when M > MAX_M_BLOCKED."""
+    n = _lib.load().gpode_whiten_blocked_work_doubles(D, M, n_sets)
+    if n < 0:
+        raise _lib.GpodeError("blocked whitening needs D <= 8 and 1 <= M <= %d (GPODE_MAX_M_BLOCKED), got D=%d, M=%d"
+                              % (MAX_M_BLOCKED, D, M))
+    return torch.empty(n, dtype=torch.float64, device=device)
+
+
 class _Whiten(torch.autograd.Function):
-    """nu = Kzz^-1-whitening of build_cache (reference src/core/dsvgp.py:110-122) via gpode_whiten_fwd / _bwd."""
+    """nu = Kzz^-1-whitening of build_cache (reference src/core/dsvgp.py:110-122) via gpode_whiten_fwd / _bwd, or
+    gpode_whiten_fwd_blocked / _bwd_blocked above MAX_M inducing points."""
 
     @staticmethod
     def forward(ctx, Z, ell, var, u, omega, phase, w, jitter):
@@ -151,7 +166,13 @@ class _Whiten(torch.autograd.Function):
         nu = torch.empty(D, M, dtype=torch.float32, device=Zc.device)
         L = torch.empty(D, M, M, dtype=torch.float64, device=Zc.device)
         sp = torch.empty(D, 2, M, dtype=torch.float64, device=Zc.device)
-        _lib.call("gpode_whiten_fwd", ctypes.byref(st), ptr(uc), float(jitter), ptr(nu), ptr(L), ptr(sp), stream_ptr())
+        if M > MAX_M:
+            work = _whiten_work(D, M, 1, Zc.device)
+            _lib.call("gpode_whiten_fwd_blocked", ctypes.byref(st), ptr(uc), float(jitter), ptr(nu), ptr(L), ptr(sp),
+                      ptr(work), stream_ptr(), launches=_lib.whiten_blocked_launches(M))
+        else:
+            _lib.call("gpode_whiten_fwd", ctypes.byref(st), ptr(uc), float(jitter), ptr(nu), ptr(L), ptr(sp),
+                      stream_ptr())
         ctx.keep = (st, Zc, ec, vc, uc, oc, pc_, wc)
         ctx.save_for_backward(L, sp)
         return nu
@@ -167,8 +188,14 @@ class _Whiten(torch.autograd.Function):
         g_Z = torch.empty(M, D, dtype=torch.float32, device=Zc.device)
         g_ell = torch.empty(D, D, dtype=torch.float32, device=Zc.device)
         g_var = torch.empty(D, dtype=torch.float32, device=Zc.device)
-        _lib.call("gpode_whiten_bwd", ctypes.byref(st), ptr(uc), ptr(L), ptr(sp), ptr(gnu), ptr(g_u), ptr(g_Z),
-                                   ptr(g_ell), ptr(g_var), stream_ptr())
+        if M > MAX_M:
+            work = _whiten_work(D, M, 0, Zc.device)
+            _lib.call("gpode_whiten_bwd_blocked", ctypes.byref(st), ptr(uc), ptr(L), ptr(sp), ptr(gnu), ptr(g_u),
+                      ptr(g_Z), ptr(g_ell), ptr(g_var), ptr(work), stream_ptr(),
+                      launches=_lib.whiten_blocked_launches(M, bwd=True))
+        else:
+            _lib.call("gpode_whiten_bwd", ctypes.byref(st), ptr(uc), ptr(L), ptr(sp), ptr(gnu), ptr(g_u), ptr(g_Z),
+                      ptr(g_ell), ptr(g_var), stream_ptr())
         return g_Z, g_ell, g_var, g_u, None, None, None, None
 
 
@@ -877,7 +904,8 @@ def _whiten_large_sets(Zc, ec, vc, uc, oc, pc_, wc, jitter):
 
 def whiten_sets(Z, ell, var, u, omega, phase, w, jitter=1e-5):
     """``u (n,M,D)`` and per-draw ``omega (n,D,S,D)``, ``phase (n,S,D)``, ``w (n,S,D)`` -> ``nu (n,D,M)``. One Kzz
-    factorisation for all draws (``gpode_whiten_fwd_sets``; float64 ``torch.linalg`` for 8 < D <= 64). No gradient."""
+    factorisation for all draws (``gpode_whiten_fwd_sets``, ``gpode_whiten_fwd_sets_blocked`` above MAX_M inducing
+    points; float64 ``torch.linalg`` for 8 < D <= 64). No gradient."""
     Zc, ec, vc, oc, pc_, wc, n, D, M, S = _sets_common(Z, ell, var, omega, phase, w)
     uc = f32(u, "u")
     if tuple(uc.shape) != (n, M, D):
@@ -888,8 +916,13 @@ def whiten_sets(Z, ell, var, u, omega, phase, w, jitter=1e-5):
     nu = torch.empty(n, D, M, dtype=torch.float32, device=Zc.device)
     L = torch.empty(D, M, M, dtype=torch.float64, device=Zc.device)
     sp = torch.empty(D, 2, M, dtype=torch.float64, device=Zc.device)
-    _lib.call("gpode_whiten_fwd_sets", ctypes.byref(st), ptr(uc), float(jitter), n, ptr(nu), ptr(L), ptr(sp),
-              stream_ptr())
+    if M > MAX_M:
+        work = _whiten_work(D, M, n, Zc.device)
+        _lib.call("gpode_whiten_fwd_sets_blocked", ctypes.byref(st), ptr(uc), float(jitter), n, ptr(nu), ptr(L),
+                  ptr(sp), ptr(work), stream_ptr(), launches=_lib.whiten_blocked_launches(M))
+    else:
+        _lib.call("gpode_whiten_fwd_sets", ctypes.byref(st), ptr(uc), float(jitter), n, ptr(nu), ptr(L), ptr(sp),
+                  stream_ptr())
     return nu
 
 

@@ -31,6 +31,7 @@ extern "C" {
 #define GPODE_MAX_D_LARGE 64   /* the large-D kernels (tcgen05 forward, large-D VJP) cover 8 < D <= 64 */
 #define GPODE_MAX_M_F64 112    /* whitening backward keeps two MxM float64 tiles in shared memory */
 #define GPODE_MAX_M 160        /* ... and falls back to float32 tiles up to this M */
+#define GPODE_MAX_M_BLOCKED 2048  /* blocked float64 whitening (matrices in global memory) for D <= GPODE_MAX_D */
 
 /* One sampled GP function = the reference's "cache" (DSVGP_Layer.build_cache, src/core/dsvgp.py:92-122) plus the
  * kernel hyper-parameters it closes over (RBF, src/core/kernels.py:33-51). */
@@ -113,6 +114,24 @@ int gpode_whiten_fwd(const gpode_cache_t* cache_without_nu, const float* u, floa
 int gpode_whiten_bwd(const gpode_cache_t* cache_with_nu, const float* u, const double* L_f64, const double* s_f64,
                      const float* grad_nu, float* grad_u, float* grad_Z, float* grad_ell, float* grad_var,
                      void* stream);
+/* The same three operations (gpode_whiten_fwd, gpode_whiten_fwd_sets below, gpode_whiten_bwd) for 1 <= M <=
+ * GPODE_MAX_M_BLOCKED at D <= GPODE_MAX_D, blocked: the M x M matrices live in global memory (L_f64 and the caller-owned
+ * float64 workspace `work`), Cholesky in panels of 64 columns, blocked triangular solves, FP64 throughout. Arguments and
+ * outputs mean what they mean for the tile kernels; the backward is bitwise reproducible and a draw of the sets form
+ * gets bitwise the nu of the single-draw call. The launch sequence depends on (D, M, n_sets) only -- no host read, no
+ * allocation -- so the calls can be captured in a CUDA graph. The library selects nothing itself: callers use these
+ * above GPODE_MAX_M (ops.whiten / ops.whiten_sets do).
+ *   gpode_whiten_blocked_work_doubles: float64 elements of `work` for the forward with n_sets >= 1 draws (D M n_sets),
+ *     or, for n_sets = 0, for the backward (D M (M + D + 2) + D ceil(M/64) (D+1)); -1 for arguments out of range.
+ *     Pure host arithmetic. */
+int64_t gpode_whiten_blocked_work_doubles(int D, int M, int n_sets);
+int gpode_whiten_fwd_blocked(const gpode_cache_t* cache_without_nu, const float* u, float jitter, float* nu_out,
+                             double* L_f64, double* s_f64, double* work, void* stream);
+int gpode_whiten_fwd_sets_blocked(const gpode_cache_t* cache_sets_without_nu, const float* u, float jitter, int n_sets,
+                                  float* nu_out, double* L_f64, double* s_f64, double* work, void* stream);
+int gpode_whiten_bwd_blocked(const gpode_cache_t* cache_with_nu, const float* u, const double* L_f64,
+                             const double* s_f64, const float* grad_nu, float* grad_u, float* grad_Z, float* grad_ell,
+                             float* grad_var, double* work, void* stream);
 
 /* Whitened KL of DSVGP_Layer.kl (src/core/dsvgp.py:199-230), q_diag=False:
  *   kl = 0.5 * sum_k [ |Um_k|^2 + |tril(Ls_k)|_F^2 - sum_i log Ls_k,ii^2 - M ],  Ls given PACKED as the optvar of

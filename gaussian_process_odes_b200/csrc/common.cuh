@@ -38,6 +38,17 @@ void gpode_set_error(const char* fmt, ...);
         }                                                                                         \
     } while (0)
 
+// A packed block above the 227 KB a CTA can opt into (large M or S) is an argument error, reported before
+// cudaFuncSetAttribute would fail on it and leave its error pending for the next launch check. static_bytes: the
+// kernel's own __shared__ arrays, which count against the same 227 KB.
+inline int check_smem_fits(size_t smem, size_t static_bytes = 0) {
+    if (smem + static_bytes > 227 * 1024) {
+        gpode_set_error("kernel does not fit on an SM (smem %zu bytes)", smem + static_bytes);
+        return -2;
+    }
+    return 0;
+}
+
 // ------------------------------------------------------------------------------------------------------------------
 // process-wide kernel-selection options (gpode_set_option / gpode_get_option, include/gpode_b200.h): the library's only
 // mutable global state. Defaults come from the environment ONCE, when the first option is read (GPODE_BWD_MMA,

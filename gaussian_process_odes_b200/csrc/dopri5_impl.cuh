@@ -381,6 +381,8 @@ int launch_dopri5_sets(const float* packed, int M, int S, int n_sets, int64_t se
 // a batch this small is one "set": a single CTA (one warp per row, __syncthreads instead of the grid barrier) runs the
 // whole solve -- the reference's own plain-GPODE shapes (N = 1 / 6 trajectories)
 constexpr int64_t kDpOneCtaRows = 16;
+// dopri5_kernel's own __shared__ arrays (sred, sset): they count against the 227 KB next to the packed block
+constexpr size_t kDpStaticSmem = sizeof(double) * (kDpSetThreads / 32 + 4);
 
 template <int D>
 int launch_dopri5(const float* packed, int M, int S, const float* x0, const double* t, int Tg, int64_t B, double rtol,
@@ -392,6 +394,7 @@ int launch_dopri5(const float* packed, int M, int S, const float* x0, const doub
     // small batches: one warp per row (the reference's N = 1 / 6 trajectories, a few thousand shooting segments)
     const bool warp_mode = B <= 1024;
     const void* kern = warp_mode ? (const void*)dopri5_kernel<D, true> : (const void*)dopri5_kernel<D, false>;
+    if (int rc = check_smem_fits(smem, kDpStaticSmem)) return rc;
     GPODE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int occ = 0, sms = 148, dev = 0;
     GPODE_CUDA(cudaGetDevice(&dev));
@@ -433,7 +436,16 @@ int launch_dopri5_sets(const float* packed, int M, int S, int n_sets, int64_t se
                        cudaStream_t st, float* ckpt, int cap) {
     const GpodeLayout L = gpode_layout(D, M, S);
     const size_t smem = 16 + (size_t)L.total * 4;
+    int warps = (int)(set_rows < kDpSetThreads / 32 ? set_rows : kDpSetThreads / 32);
+    if (warps < 1) warps = 1;
+    if (int rc = check_smem_fits(smem, kDpStaticSmem)) return rc;
     GPODE_CUDA(cudaFuncSetAttribute(dopri5_kernel<D, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int occ = 0;
+    GPODE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, dopri5_kernel<D, true, true>, warps * 32, smem));
+    if (occ < 1) {
+        gpode_set_error("dopri5 kernel does not fit on an SM (smem %zu bytes)", smem);
+        return -2;
+    }
     Dopri5Args a;
     a.packed = packed; a.M = M; a.S = S; a.total = L.total; a.x0 = x0; a.t = t; a.Tg = Tg;
     a.B = set_rows * n_sets;
@@ -445,8 +457,6 @@ int launch_dopri5_sets(const float* packed, int M, int S, int n_sets, int64_t se
     a.set_stride = L.n_packed;
     a.max_attempts = 1 << 20;
     dopri5_set_ckpt(a, n_sets == 1 ? ckpt : nullptr, cap, a.B * D, Tg);  // checkpoints: single-set (training) use only
-    int warps = (int)(set_rows < kDpSetThreads / 32 ? set_rows : kDpSetThreads / 32);
-    if (warps < 1) warps = 1;
     dopri5_kernel<D, true, true><<<n_sets, warps * 32, smem, st>>>(a);
     GPODE_LAUNCH_CHECK();
     return 0;
@@ -608,6 +618,7 @@ int launch_dopri5_bwd(const float* packed, int M, int S, const double* t, int Tg
                       float* acc, cudaStream_t st) {
     const GpodeLayout L = gpode_layout(D, M, S);
     const size_t smem = 16 + (size_t)L.total * 4 + (size_t)kWarpAccDoubles<D>(kDpThreads / 32) * 8;
+    if (int rc = check_smem_fits(smem)) return rc;
     GPODE_CUDA(cudaFuncSetAttribute(dopri5_bwd_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int occ = 0, sms = 148, dev = 0;
     GPODE_CUDA(cudaGetDevice(&dev));

@@ -926,16 +926,6 @@ inline int num_sms() {
     return g_num_sms;
 }
 
-// A packed block above the 227 KB a CTA can opt into (large M or S) is an argument error, reported before
-// cudaFuncSetAttribute would fail on it and leave its error pending for the next launch check.
-inline int check_smem_fits(size_t smem) {
-    if (smem > 227 * 1024) {
-        gpode_set_error("kernel does not fit on an SM (smem %zu bytes)", smem);
-        return -2;
-    }
-    return 0;
-}
-
 template <typename K>
 inline int shape_for(K kernel, int R, int64_t B, size_t smem, LaunchShape* out) {
     // small batches: narrow CTAs so the rows spread over more SMs; large: 128 threads, grid = SMs x resident CTAs
@@ -1123,6 +1113,7 @@ int launch_fwd_sets(const float* packed, int M, int S, int n_sets, int64_t set_r
     if (want > per_set) want = per_set;
     if (want < 1) want = 1;
     const dim3 grid((unsigned)want, (unsigned)n_sets);
+    if (int rc = check_smem_fits(smem)) return rc;
     if (t == nullptr) {
         GPODE_CUDA(cudaFuncSetAttribute(vf_fwd_sets_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         vf_fwd_sets_kernel<D><<<grid, threads, smem, st>>>(packed, M, S, L.total, L.n_packed, set_rows, x0, out);

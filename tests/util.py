@@ -299,3 +299,77 @@ def elbo_errors(kind, kw, solver, extra, seed):
     return rows
 
 
+# ---- shared memory of the D <= 8 integrator kernels, restated from their launchers ---------------------------------
+# (csrc/common.cuh gpode_layout, csrc/integrate_impl.cuh launch_* / h_smem, csrc/dopri5_impl.cuh). Every CTA of these
+# kernels stages the whole packed block, so its size grows with M (the kern records, KS floats per inducing point); a
+# block above the 227 KB a CTA can opt into either hands the batch to the next kernel or is refused ("does not fit").
+SMEM_OPTIN = 227 * 1024     # check_smem_fits
+MAX_M_BLOCKED = 2048        # GPODE_MAX_M_BLOCKED: the largest M the whitening (and so training) accepts
+TC_WARPS = 12               # kHWarps = kHFWarps: warps of the tensor-core kernels (D = 4, 5)
+TC_ROW_FIELDS = 7           # kHRowFields
+RED_WARPS = 16              # kRedWarps
+DP_STATIC_SMEM = 96         # kDpStaticSmem: dopri5_kernel's own __shared__ arrays
+ADJ_WARPS = 4               # kWarpsPerCta = kDpThreads / 32: warps of the warp-per-row adjoints
+
+
+def packed_layout(D, M, S):
+    """gpode_layout in floats: total (the block the FFMA2 kernels stage), n_small (kern + il records), n_mmah (the
+    tensor-core operand records, D <= 5) and n_packed (gpode_packed_floats)"""
+    r4 = lambda x: (x + 3) & ~3
+    S2P = (((S + 1) // 2) + 31) & ~31
+    RP, KS, WP = r4(2 * D + 4), r4(D + 2 * ((D + 1) // 2)), r4(2 * ((D + 1) // 2))
+    n_small = M * KS + D * WP
+    total = D * S2P * RP + n_small
+    n_mmah = D * ((((S + 7) // 8) + 1) & ~1) * 152
+    return dict(total=total, n_small=n_small, n_mmah=n_mmah, n_packed=total + (n_mmah if D <= 5 else 0))
+
+
+def _red_floats(D):
+    return (RED_WARPS * (D * D + D) + 3) & ~3
+
+
+def _warp_acc_bytes(D, warps=ADJ_WARPS):
+    return warps * 33 * (D * D + D) * 8     # kWarpAccDoubles<D>: a 32-lane slab and a row of D*D + D per warp
+
+
+def _tc_smem(D, M, S, rk4, row_sums=False):
+    """h_smem<D>(hp, rk4, kHWarps, row_sums)"""
+    L = packed_layout(D, M, S)
+    stage = 2 * 32 * (D | 1) + 32 * 8
+    return 16 + 4 * (L['n_small'] + L['n_mmah'] + (0 if rk4 else _red_floats(D)) + TC_WARPS * stage
+                     + (TC_WARPS * TC_ROW_FIELDS * D * 32 if rk4 else 0) + (TC_WARPS * M * 2 * D if row_sums else 0))
+
+
+# family -> (state dimensions, bytes(D, M, S), the kernels that stage that many bytes)
+SMEM_FAMILIES = {
+    "fwd": (range(1, 9), lambda D, M, S: 16 + 4 * packed_layout(D, M, S)['total'],
+            "vf_fwd / rk4_fwd kernels (warp, row, wide) and the vf / rk4 *_sets kernels"),
+    "dopri5_fwd": (range(1, 9), lambda D, M, S: 16 + 4 * packed_layout(D, M, S)['total'] + DP_STATIC_SMEM,
+                   "dopri5_kernel, all three forms"),
+    "bwd": (range(1, 9), lambda D, M, S: 16 + 4 * (packed_layout(D, M, S)['total'] + _red_floats(D)),
+            "vf_bwd_kernel / rk4_bwd_kernel (row per thread, wide)"),
+    "bwd_warp": (range(1, 9), lambda D, M, S: 16 + 4 * packed_layout(D, M, S)['total'] + _warp_acc_bytes(D),
+                 "vf_bwd_warp_kernel / rk4_bwd_warp_kernel and dopri5_bwd_kernel"),
+    "tc_fwd": ((4, 5), lambda D, M, S: _tc_smem(D, M, S, rk4=False), "vf_fwd_h_kernel / rk4_fwd_h_kernel"),
+    "tc_bwd": ((4, 5), lambda D, M, S: _tc_smem(D, M, S, rk4=True),
+               "rk4_bwd_mma_kernel; the bound on which vf_bwd_mma_kernel is chosen too"),
+    "tc_row_sums": ((4, 5), lambda D, M, S: _tc_smem(D, M, S, rk4=True, row_sums=True),
+                    "rk4_bwd_mma_kernel<D, true, true>: the shooting adjoint that sums the inducing-point gradients"),
+}
+
+
+def kernel_smem(family, D, M, S):
+    return SMEM_FAMILIES[family][1](D, M, S)
+
+
+def max_inducing(family, D, S):
+    """M*: the largest M whose block fits (0 if not even M = 1 does), or None when M = MAX_M_BLOCKED fits -- that
+    family cannot run out of shared memory at this S"""
+    fits = lambda M: kernel_smem(family, D, M, S) <= SMEM_OPTIN
+    if fits(MAX_M_BLOCKED):
+        return None
+    lo, hi = 0, MAX_M_BLOCKED          # fits(lo) or lo == 0; not fits(hi): the size grows with M
+    while hi - lo > 1:
+        mid = (lo + hi) // 2
+        lo, hi = (mid, hi) if fits(mid) else (lo, mid)
+    return lo

@@ -48,12 +48,13 @@ class Flow(nn.Module):
         self.rtol = rtol
         self.use_adjoint = use_adjoint
 
-    def forward(self, x0, ts, return_divergence=False):
-        """IVP solution ``(N,T,D)`` for initial states ``x0 (N,D)`` on the time sequence ``ts (T,)``."""
+    def forward(self, x0, ts, return_divergence=False, rebuild_cache=True):
+        """IVP solution ``(N,T,D)`` for initial states ``x0 (N,D)`` on the time sequence ``ts (T,)``. A new GP function
+        is drawn per call unless ``rebuild_cache=False`` (the current draw is integrated)."""
         if return_divergence:
             raise NotImplementedError("divergence integration is not part of GPODE (dead branch, flow.py:70-80)")
         odeint = odeint_adjoint if self.use_adjoint else odeint_nonadjoint
-        self.odefunc.before_odeint(return_divergence=False, rebuild_cache=True)
+        self.odefunc.before_odeint(return_divergence=False, rebuild_cache=rebuild_cache)
         xs = odeint(self.odefunc, x0, ts, atol=self.atol, rtol=self.rtol, method=self.solver)
         return xs.permute(1, 0, 2)
 

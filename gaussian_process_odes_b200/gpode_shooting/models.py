@@ -52,6 +52,10 @@ class BaseSequenceModel(nn.Module):
         return self.flow.forward_sets(x0, dense, rng=rng)[:, :, ::self.ts_dense_scale - 1, :]
 
 
+class _FusedDoesNotFit(Exception):
+    """The fused shooting step refused its launch for shared memory; the cache of this step's GP draw is built."""
+
+
 class UniformSequenceModel(BaseSequenceModel):
     """Observations on a uniform time grid: every segment spans ``ts[:2]`` (reference ``models.py:88-146``)."""
 
@@ -66,7 +70,9 @@ class UniformSequenceModel(BaseSequenceModel):
     def _fused_terms(self, ss_samples, ys, ts, halo=False, T_global=None):
         """Observation log-likelihood mean and constraint total through ONE integrator launch with the two terms
         evaluated on the segment end points inside the kernel (``ops.shooting_step``), or None when the configuration
-        has no fused kernel (solver other than rk4, D > 8, non-affine decoder, trainable constraint scale, CPU)."""
+        has no fused kernel (solver other than rk4, D > 8, non-affine decoder, trainable constraint scale, CPU). Raises
+        _FusedDoesNotFit, with this step's GP cache already built, when the fused forward does not fit in shared
+        memory."""
         from ..core.dsvgp import DSVGP_Layer
         from ..core.constraints import _ScaleFamily
         flow, lik, cons = self.flow, self.likelihood, self.constraint
@@ -85,6 +91,7 @@ class UniformSequenceModel(BaseSequenceModel):
         if W.shape[0] != D or Dobs > 128 or tuple(ys.shape) != (N, T, Dobs):
             return None
         from .. import ops
+        from .._lib import GpodeError
         var = lik.variance
         if var.numel() != Dobs:
             var = var.expand(Dobs)
@@ -93,8 +100,16 @@ class UniformSequenceModel(BaseSequenceModel):
             from ..distributed import shard_range
             rows = shard_range(S * N * T, *self.row_shard)
         flow.odefunc.before_odeint(return_divergence=False, rebuild_cache=True)
-        ll_sum, cons_sum, _ = ops.shooting_step(ss_samples, ts[:2], *layer.cache_tensors(), ys, W, b, var,
-                                                cons.scale.detach(), laplace=cons._laplace, rows=rows, halo=halo)
+        try:
+            ll_sum, cons_sum, _ = ops.shooting_step(ss_samples, ts[:2], *layer.cache_tensors(), ys, W, b, var,
+                                                    cons.scale.detach(), laplace=cons._laplace, rows=rows, halo=halo)
+        except GpodeError as e:
+            # the epilogue's shared memory comes on top of the integrator's block: at many inducing points the fused
+            # forward is refused (before any launch) where the separate integrator and side-term kernels still fit. A
+            # sharded step has no unfused form: there the refusal is the error to report.
+            if "does not fit" not in str(e) or self.row_shard is not None or T_global is not None:
+                raise
+            raise _FusedDoesNotFit() from e
         flow.odefunc.count_evals(4)
         return ll_sum / float(S * N * (T if T_global is None else T_global) * Dobs), cons_sum / S
 
@@ -136,7 +151,11 @@ class UniformSequenceModel(BaseSequenceModel):
             return self._time_sharded_terms(ys, ts, num_samples)
         ss_samples = self.state_distribution.sample(num_samples=num_samples)  # (S,N,T,D)
         (S, N, T, D) = ss_samples.shape
-        fused = self._fused_terms(ss_samples, ys, ts)
+        rebuild_cache = True
+        try:
+            fused = self._fused_terms(ss_samples, ys, ts)
+        except _FusedDoesNotFit:
+            fused, rebuild_cache = None, False   # integrate with the GP draw the fused attempt built
         if fused is not None:
             observation_loglik_mean, constraint_total = fused
             state_entropy = self.state_distribution.entropy()  # (N,T-1)
@@ -148,7 +167,7 @@ class UniformSequenceModel(BaseSequenceModel):
             raise RuntimeError("row sharding needs the fused shooting step (rk4, affine decoder, frozen constraint "
                                "scale, D <= 8)")
         # one launch: S*N*T independent one-interval IVPs sharing one GP function draw
-        predicted_xs = self.flow(x0=stack_segments(ss_samples), ts=ts[:2])  # (S*N*T, 2, D)
+        predicted_xs = self.flow(x0=stack_segments(ss_samples), ts=ts[:2], rebuild_cache=rebuild_cache)  # (S*N*T, 2, D)
         predicted_xs = unstack_segments(predicted_xs[:, -1], (S, N, T, D))
         # mean log-likelihood: one fused decode + log-density kernel when the likelihood offers it
         mean_fn = getattr(self.likelihood, "log_prob_mean", None)

@@ -25,8 +25,9 @@ from test_gpu_small_d_mappings import (WARP_MAX_ROWS, grids_of, mma_min_rows, pr
 from test_gpu_small_d_mappings import dopri5_kernel as dopri5_kernel_name
 from test_gpu_whiten_blocked import _lattice
 from test_many_inducing_cpu import oversized_calls
-from util import (TOL_GRAD, TOL_TRAJ, TOL_VF, assert_grads, assert_parity, chunked_oracle, cuda_args, cuda_grads,
-                  lazy, max_inducing, oracle_dopri5, oracle_leaves, oracle_rk4, oracle_vf, relerr, time_grid)
+from util import (GRAD_KEYS, TOL_GRAD, TOL_TRAJ, TOL_VF, assert_grads, assert_parity, chunked_oracle, cuda_args, cuda_grads,
+                  lazy, max_inducing, oracle_dopri5, oracle_leaves, oracle_rk4, oracle_vf, relerr, shoot_cuda,
+                  shoot_inputs, shoot_oracle, time_grid)
 
 pytestmark = pytest.mark.gpu
 
@@ -186,59 +187,6 @@ def test_dopri5_forms_and_adjoint_at_large_m(D, mapping, M):
 
 
 # ---- the fused shooting step (rk4_*_kernel<..., kShoot = true>) ----------------------------------------------------
-def _shoot_inputs(D, S_mc, N, T, seed):
-    rng = np.random.default_rng(seed)
-    t = lambda a: torch.tensor(np.asarray(a), dtype=torch.float32)
-    Dobs = D + 1
-    return dict(t2=t([0.0, 0.07]), ys=t(rng.normal(size=(N, T, Dobs))), W=t(rng.normal(size=(D, Dobs)) * 0.5),
-                bias=t(rng.normal(size=Dobs) * 0.1), lik_var=t(0.5 + rng.uniform(size=Dobs)), scale=t([0.3]))
-
-
-def _shoot_cuda(gp, c, ss, si, a_ll, a_c):
-    """ops.shooting_step -> (ll, cons, {x: grad ss, Z, ell, var, nu}) of a_ll ll + a_c cons"""
-    from gaussian_process_odes_b200 import ops
-    args = cuda_args(gp, c, True)
-    sc = ss.cuda().requires_grad_(True)
-    ll, cons, _ = ops.shooting_step(sc, si['t2'].cuda(), *args, si['ys'].cuda(), si['W'].cuda(), si['bias'].cuda(),
-                                    si['lik_var'].cuda(), si['scale'].cuda())
-    (a_ll * ll + a_c * cons).backward()
-    return ll.detach().cpu(), cons.detach().cpu(), dict(x=sc.grad, Z=args[0].grad, ell=args[1].grad,
-                                                        var=args[2].grad, nu=args[3].grad)
-
-
-def _shoot_oracle(gp, c, ss, si, a_ll, a_c, dtype, chunk, dev="cuda"):
-    """the same step through the oracle over row chunks: pred = one RK4 interval from every row, ll = sum of
-    gauss_loglik(pred W + bias), cons = sum over t < T-1 of normal_logprob(ss[t+1] | pred, scale). The constraint's
-    neighbour state is a leaf of its own per chunk; its gradient lands on the next row of ss."""
-    S_mc, N, T, D = ss.shape
-    x = ss.reshape(-1, D)
-    B = x.shape[0]
-    tt = torch.arange(B) % T
-    nxt = torch.cat([x[1:], x[:1]])     # row r's neighbour ss[s, n, t + 1] is row r + 1 (masked at t = T - 1)
-    ys = si['ys'].unsqueeze(0).expand(S_mc, N, T, -1).reshape(B, -1)
-    W, bias, var, scale = [si[k].to(dev, dtype) for k in ("W", "bias", "lik_var", "scale")]
-    step = oracle_rk4(si['t2'])
-    ll = cons = 0.0
-    gx, gn, gsum = [], [], {}
-    for r0 in range(0, B, chunk):
-        l, cc = oracle_leaves(gp, c, x[r0:r0 + chunk], dtype, dev)
-        nb = nxt[r0:r0 + chunk].to(dev, dtype).requires_grad_(True)
-        pred = step(l, cc)[1]
-        lli = O.gauss_loglik(pred @ W + bias, ys[r0:r0 + chunk].to(dev, dtype), var).sum()
-        mask = (tt[r0:r0 + chunk] < T - 1).to(dev, dtype).unsqueeze(1)
-        ci = (O.normal_logprob(nb, pred, scale) * mask).sum()
-        (a_ll * lli + a_c * ci).backward()
-        ll, cons = ll + float(lli.detach()), cons + float(ci.detach())
-        gx.append(l['x'].grad.cpu())
-        gn.append(nb.grad.cpu())
-        for k in ("Z", "ell", "var", "nu"):
-            g = l[k].grad.double().cpu()
-            gsum[k] = gsum[k] + g if k in gsum else g
-    g = {k: v.to(dtype) for k, v in gsum.items()}
-    g['x'] = (torch.cat(gx) + torch.cat([torch.cat(gn)[-1:], torch.cat(gn)[:-1]])).reshape(S_mc, N, T, D)
-    return torch.tensor([ll, cons], dtype=torch.float64), g
-
-
 def _shoot_case(D, M, S, S_mc, N, T, seed, names, absent=(), monkeypatch=None, vrows=False):
     """the fused step against the oracle; vrows: force the virtual-row adjoint (gpode_shoot_bwd with vrows +
     gpode_param_grad) where the tensor-core adjoint would sum the inducing-point gradients itself"""
@@ -246,11 +194,11 @@ def _shoot_case(D, M, S, S_mc, N, T, seed, names, absent=(), monkeypatch=None, v
     B = S_mc * N * T
     gp, c, x = _problem(D, M, S, B, seed)
     ss = x.reshape(S_mc, N, T, D)
-    si = _shoot_inputs(D, S_mc, N, T, seed)
+    si = shoot_inputs(D, S_mc, N, T, seed)
     a_ll, a_c = 0.7, 1.3
     if vrows:
         monkeypatch.setattr(_lib.load(), "gpode_shoot_bwd_vrows", lambda D_, M_, S_, n: 4 * n)
-    (ll, cons, got), kernels = profiled(lambda: _shoot_cuda(gp, c, ss, si, a_ll, a_c))
+    (ll, cons, got), kernels = profiled(lambda: shoot_cuda(gp, c, ss, si, a_ll, a_c))
     if vrows:
         monkeypatch.undo()
     for n in names:
@@ -259,11 +207,11 @@ def _shoot_case(D, M, S, S_mc, N, T, seed, names, absent=(), monkeypatch=None, v
         with pytest.raises(AssertionError):
             grids_of(kernels, n)
     chunk = _chunk(D, M)
-    sums32, ref32 = _shoot_oracle(gp, c, ss, si, a_ll, a_c, torch.float32, chunk)
-    ref64 = lazy(lambda: _shoot_oracle(gp, c, ss, si, a_ll, a_c, torch.float64, chunk))
+    sums32, ref32 = shoot_oracle(gp, c, ss, si, a_ll, a_c, torch.float32, chunk)
+    ref64 = lazy(lambda: shoot_oracle(gp, c, ss, si, a_ll, a_c, torch.float64, chunk))
     name = "shoot D=%d M=%d S=%d B=%d%s" % (D, M, S, B, " vrows" if vrows else "")
     assert_parity(name + " sums", torch.stack([ll, cons]).double(), sums32, lambda: ref64()[0], TOL_GRAD)
-    assert_grads(name, got, ref32, lambda: ref64()[1], TOL_GRAD)
+    assert_grads(name, got, ref32, lambda: ref64()[1], TOL_GRAD, keys=GRAD_KEYS + ("lik_var",))
     return got
 
 

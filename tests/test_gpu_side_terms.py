@@ -9,7 +9,7 @@ from util import relerr
 pytestmark = pytest.mark.gpu
 
 
-@pytest.mark.parametrize("D", [1, 2, 3, 5, 8])
+@pytest.mark.parametrize("D", range(1, 9))
 @pytest.mark.parametrize("batch", [(1,), (6, 99), (3, 1)])
 def test_state_sample_and_entropy(D, batch):
     from gaussian_process_odes_b200 import ops
@@ -39,7 +39,9 @@ def test_state_sample_and_entropy(D, batch):
     assert relerr(lc.grad, l64.grad) <= 2e-4
 
 
-@pytest.mark.parametrize("D,Dobs,S,lead", [(5, 50, 3, (2, 20)), (2, 2, 5, (1, 25)), (5, 50, 1, (6, 100)), (3, 128, 2, (4, 7))])
+@pytest.mark.parametrize("D,Dobs,S,lead", [(5, 50, 3, (2, 20)), (2, 2, 5, (1, 25)), (5, 50, 1, (6, 100)), (3, 128, 2, (4, 7)),
+                                           (1, 3, 2, (2, 11)), (4, 33, 4, (3, 9)), (6, 64, 5, (1, 40)),
+                                           (7, 97, 9, (2, 5)), (8, 128, 3, (3, 8))])
 @pytest.mark.parametrize("with_bias", [False, True])
 def test_loglik_mean(D, Dobs, S, lead, with_bias):
     from gaussian_process_odes_b200 import ops

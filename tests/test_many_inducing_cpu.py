@@ -16,10 +16,11 @@ S_TABLE = (64, 256, 512)
 LIMITS = {
     64: {("tc_row_sums", 4): 341, ("tc_row_sums", 5): 239},
     256: {("bwd_warp", 7): 1584, ("bwd_warp", 8): 1159, ("tc_bwd", 5): 1116, ("tc_row_sums", 4): 201,
-          ("tc_row_sums", 5): 101},
+          ("tc_row_sums", 5): 101, ("shoot_tc_fwd", 5): 1851},
     512: {("fwd", 7): 1388, ("fwd", 8): 1067, ("dopri5_fwd", 7): 1386, ("dopri5_fwd", 8): 1066, ("bwd", 7): 1332,
           ("bwd", 8): 995, ("bwd_warp", 6): 1866, ("bwd_warp", 7): 464, ("bwd_warp", 8): 0, ("tc_fwd", 4): 1493,
-          ("tc_fwd", 5): 169, ("tc_bwd", 4): 189, ("tc_bwd", 5): 0, ("tc_row_sums", 4): 14, ("tc_row_sums", 5): 0},
+          ("tc_fwd", 5): 169, ("tc_bwd", 4): 189, ("tc_bwd", 5): 0, ("tc_row_sums", 4): 14, ("tc_row_sums", 5): 0,
+          ("shoot_fwd", 7): 1243, ("shoot_fwd", 8): 914, ("shoot_tc_fwd", 4): 991, ("shoot_tc_fwd", 5): 0},
 }
 
 
@@ -40,16 +41,18 @@ def test_limit_table(S):
 
 def test_limit_table_orders_the_families():
     """a kernel that stages more than another runs out of room first: the row-sum adjoint before the tensor-core
-    adjoint, the warp adjoints (float64 slabs) before the row-per-thread ones, dopri5 (its static arrays) before the
-    other forward kernels"""
+    adjoint, the warp adjoints (float64 slabs) before the row-per-thread ones, dopri5 (its static arrays) and the fused
+    shooting forward (its epilogue) before the other forward kernels"""
     big = MAX_M_BLOCKED + 1
     m = lambda f, D, S: big if max_inducing(f, D, S) is None else max_inducing(f, D, S)
     for S in (33, 64, 129, 256, 512):
         for D in range(1, 9):
             assert m("bwd_warp", D, S) <= m("bwd", D, S) <= m("fwd", D, S)
             assert m("dopri5_fwd", D, S) <= m("fwd", D, S)
+            assert m("shoot_fwd", D, S) <= m("fwd", D, S)
         for D in (4, 5):
             assert m("tc_row_sums", D, S) <= m("tc_bwd", D, S) <= m("tc_fwd", D, S)
+            assert m("shoot_tc_fwd", D, S) <= m("tc_fwd", D, S)
 
 
 @pytest.mark.parametrize("S", [1, 33, 64, 129, 256, 512])

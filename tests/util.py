@@ -159,11 +159,88 @@ def lazy(fn):
     return get
 
 
-def assert_grads(name, got, ref32, ref64, tol):
+def assert_grads(name, got, ref32, ref64, tol, keys=GRAD_KEYS):
     """assert_parity of every gradient; ``ref64``: callable returning the float64 gradients"""
-    for k in GRAD_KEYS:
+    for k in keys:
         assert_parity("%s grad %s" % (name, k), got[k].cpu().reshape(ref32[k].shape), ref32[k],
                       lambda k=k: ref64()[k], tol)
+
+
+# ---- the fused shooting step (ops.shooting_step) and its oracle ----------------------------------------------------
+def shoot_inputs(D, S_mc, N, T, seed, Dobs=None, bias=True, scale=0.3):
+    """observations, decoder, likelihood variance and constraint scale of a shooting step (Dobs = D + 1 unless
+    given); ``bias=False``: no decoder bias (the draws stay the same)"""
+    rng = np.random.default_rng(seed)
+    t = lambda a: torch.tensor(np.asarray(a), dtype=torch.float32)
+    Dobs = D + 1 if Dobs is None else Dobs
+    si = dict(t2=t([0.0, 0.07]), ys=t(rng.normal(size=(N, T, Dobs))), W=t(rng.normal(size=(D, Dobs)) * 0.5),
+              bias=t(rng.normal(size=Dobs) * 0.1), lik_var=t(0.5 + rng.uniform(size=Dobs)), scale=t([scale]))
+    if not bias:
+        si['bias'] = None
+    return si
+
+
+def shoot_cuda(gp, c, ss, si, a_ll, a_c, laplace=False, rows=None, halo=False):
+    """ops.shooting_step -> (ll, cons, {x: grad ss, Z, ell, var, nu, lik_var}) of a_ll ll + a_c cons"""
+    from gaussian_process_odes_b200 import ops
+    args = cuda_args(gp, c, True)
+    sc = ss.cuda().requires_grad_(True)
+    lv = si['lik_var'].cuda().requires_grad_(True)
+    bias = si['bias'].cuda() if si['bias'] is not None else None
+    ll, cons, _ = ops.shooting_step(sc, si['t2'].cuda(), *args, si['ys'].cuda(), si['W'].cuda(), bias, lv,
+                                    si['scale'].cuda(), laplace=laplace, rows=rows, halo=halo)
+    (a_ll * ll + a_c * cons).backward()
+    return ll.detach().cpu(), cons.detach().cpu(), dict(x=sc.grad, Z=args[0].grad, ell=args[1].grad,
+                                                        var=args[2].grad, nu=args[3].grad, lik_var=lv.grad)
+
+
+def cons_logprob(y, loc, scale, laplace):
+    """the shooting constraint's density (reference src/core/constraints.py:26-36, 56-66), elementwise"""
+    dist = torch.distributions.Laplace if laplace else torch.distributions.Normal
+    return dist(loc=loc, scale=scale).log_prob(y)
+
+
+def shoot_oracle(gp, c, ss, si, a_ll, a_c, dtype, chunk, dev="cuda", laplace=False, rows=None, halo=False):
+    """the same step through the oracle over row chunks of ``rows = (lo, hi)`` (all rows by default): pred = one RK4
+    interval from every row, ll = sum of gauss_loglik(pred W + bias) over the rows that carry an observation (with
+    ``halo`` not the last time index of a sequence), cons = sum over t < T-1 of the constraint's log-density of
+    ss[t+1] given pred. The constraint's neighbour state is a leaf of its own per chunk; its gradient lands on the next
+    row of ss (row hi included). -> (float64 [ll, cons], {x: grad of all of ss, Z, ell, var, nu, lik_var})"""
+    S_mc, N, T, D = ss.shape
+    x = ss.reshape(-1, D)
+    B = x.shape[0]
+    lo, hi = (0, B) if rows is None else rows
+    tt = torch.arange(B) % T
+    nxt = torch.cat([x[1:], x[:1]])     # row r's neighbour ss[s, n, t + 1] is row r + 1 (masked at t = T - 1)
+    ys = si['ys'].unsqueeze(0).expand(S_mc, N, T, -1).reshape(B, -1)
+    W, scale = [si[k].to(dev, dtype) for k in ("W", "scale")]
+    bias = si['bias'].to(dev, dtype) if si['bias'] is not None else 0.0
+    var = si['lik_var'].to(dev, dtype).requires_grad_(True)
+    step = oracle_rk4(si['t2'])
+    ll = cons = 0.0
+    gx = torch.zeros(B + 1, D, dtype=dtype)
+    gsum = {}
+    for r0 in range(lo, hi, chunk):
+        r1 = min(r0 + chunk, hi)
+        l, cc = oracle_leaves(gp, c, x[r0:r1], dtype, dev)
+        nb = nxt[r0:r1].to(dev, dtype).requires_grad_(True)
+        pred = step(l, cc)[1]
+        obs = torch.ones(r1 - r0) if not halo else (tt[r0:r1] < T - 1).to(torch.float32)
+        lli = (O.gauss_loglik(pred @ W + bias, ys[r0:r1].to(dev, dtype), var)
+               * obs.to(dev, dtype).unsqueeze(1)).sum()
+        mask = (tt[r0:r1] < T - 1).to(dev, dtype).unsqueeze(1)
+        ci = (cons_logprob(nb, pred, scale, laplace) * mask).sum()
+        (a_ll * lli + a_c * ci).backward()
+        ll, cons = ll + float(lli.detach()), cons + float(ci.detach())
+        gx[r0:r1] += l['x'].grad.cpu()
+        gx[r0 + 1:r1 + 1] += nb.grad.cpu()
+        for k in ("Z", "ell", "var", "nu"):
+            g = l[k].grad.double().cpu()
+            gsum[k] = gsum[k] + g if k in gsum else g
+    g = {k: v.to(dtype) for k, v in gsum.items()}
+    g['x'] = gx[:B].reshape(S_mc, N, T, D)
+    g['lik_var'] = var.grad.cpu() if var.grad is not None else torch.zeros(var.shape, dtype=dtype)
+    return torch.tensor([ll, cons], dtype=torch.float64), g
 
 
 def time_grid(Tg, h, seed):
@@ -340,6 +417,23 @@ def _tc_smem(D, M, S, rk4, row_sums=False):
                      + (TC_WARPS * TC_ROW_FIELDS * D * 32 if rk4 else 0) + (TC_WARPS * M * 2 * D if row_sums else 0))
 
 
+SHOOT_MAX_DOBS = 128        # GPODE_SHOOT_MAX_DOBS: the largest observed dimension the fused shooting step takes
+THREAD_WARPS = 4            # kThreads / 32 = kWarpsPerCta: warps of the row-per-thread and warp-per-row kernels
+
+
+def shoot_smem_bytes(D, Dobs, warps):
+    """csrc/shoot.cuh shoot_smem_bytes: W, bias, 1/var and log(2 pi var) with Dobs padded to 4, then one float64 row of
+    [2 + Dobs] accumulators per warp -- staged by the fused shooting forward on top of the integrator's block"""
+    DP = (Dobs + 3) & ~3
+    return (D + 3) * DP * 4 + warps * (2 + Dobs) * 8
+
+
+def _shoot_tc_fwd(D, M, S):
+    """launch_rk4_fwd<D, kShoot = true> on the tensor cores: the forward block rounded up to 16 bytes, then the
+    epilogue's region for kHFWarps warps"""
+    return ((_tc_smem(D, M, S, rk4=False) + 15) & ~15) + shoot_smem_bytes(D, SHOOT_MAX_DOBS, TC_WARPS)
+
+
 # family -> (state dimensions, bytes(D, M, S), the kernels that stage that many bytes)
 SMEM_FAMILIES = {
     "fwd": (range(1, 9), lambda D, M, S: 16 + 4 * packed_layout(D, M, S)['total'],
@@ -355,6 +449,11 @@ SMEM_FAMILIES = {
                "rk4_bwd_mma_kernel; the bound on which vf_bwd_mma_kernel is chosen too"),
     "tc_row_sums": ((4, 5), lambda D, M, S: _tc_smem(D, M, S, rk4=True, row_sums=True),
                     "rk4_bwd_mma_kernel<D, true, true>: the shooting adjoint that sums the inducing-point gradients"),
+    "shoot_fwd": (range(1, 9), lambda D, M, S: 16 + 4 * packed_layout(D, M, S)['total']
+                  + shoot_smem_bytes(D, SHOOT_MAX_DOBS, THREAD_WARPS),
+                  "rk4_fwd_warp_kernel / rk4_fwd_kernel <..., true> at Dobs = 128: the fused shooting forward"),
+    "shoot_tc_fwd": ((4, 5), _shoot_tc_fwd,
+                     "rk4_fwd_h_kernel<D, true> at Dobs = 128: the fused shooting forward on the tensor cores"),
 }
 
 

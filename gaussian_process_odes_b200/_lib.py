@@ -75,6 +75,9 @@ SIGNATURES = {
     "gpode_shoot_fwd": (_I, [_P, _I, _I, _I, ctypes.POINTER(GpodeShoot), _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "gpode_shoot_bwd": (_I, [_P, _I, _I, _I, ctypes.POINTER(GpodeShoot), _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "gpode_shoot_bwd_vrows": (_L, [_I, _I, _I, _L]),
+    "gpode_shoot_large_work_doubles": (_L, [_I, _L]),
+    "gpode_shoot_fwd_large": (_I, [_P, _CP, ctypes.POINTER(GpodeShoot), _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "gpode_shoot_bwd_large": (_I, [_P, _CP, ctypes.POINTER(GpodeShoot), _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "gpode_acc_header_floats": (_L, []),
     "gpode_probe_fp32_fma": (_I, [ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double), _P, _P]),
     "gpode_dopri5_ckpt_floats": (_L, [_I, _L, _I, _I]),
@@ -189,6 +192,8 @@ KERNELS_PER_CALL = {
     "gpode_dopri5_fwd_large_sets": 10 + 22,
     # per accepted step: 6 VJPs (2 kernels each) + 7 element-wise kernels; once: the VJP at x0 + the grad_x0 kernel
     "gpode_dopri5_bwd_large": 19 + 3,
+    # shooting step above D = 8: one RK4 interval + the epilogue and its ordered sum; seed kernel + adjoint + pull kernel
+    "gpode_shoot_fwd_large": 12 + 2, "gpode_shoot_bwd_large": 1 + 16 + 1,
 }
 assert all(isinstance(v, int) for v in KERNELS_PER_CALL.values()), "KERNELS_PER_CALL holds launch counts"
 assert set(KERNELS_PER_CALL) <= set(SIGNATURES), sorted(set(KERNELS_PER_CALL) - set(SIGNATURES))

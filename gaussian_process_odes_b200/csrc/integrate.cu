@@ -184,8 +184,9 @@ shoot_sum_kernel(const double* __restrict__ work, const int n_rows, const int co
     if (g_var != nullptr)
         for (int i = threadIdx.x; i + 2 < cols; i += blockDim.x) g_var[i] = (float)tot[2 + i];
 }
+}  // namespace
 
-int check_shoot(const gpode_shoot_t* sh, int D) {
+int gpode_check_shoot(const gpode_shoot_t* sh) {
     GPODE_CHECK_ARG(sh != nullptr, "shooting descriptor is NULL");
     GPODE_CHECK_ARG(sh->S_mc >= 1 && sh->N >= 1 && sh->T >= 1, "bad batch shape S_mc=%d N=%d T=%d", sh->S_mc, sh->N, sh->T);
     GPODE_CHECK_ARG(sh->D_obs >= 1 && sh->D_obs <= GPODE_SHOOT_MAX_DOBS, "observed dimension %d outside 1..%d", sh->D_obs,
@@ -195,17 +196,21 @@ int check_shoot(const gpode_shoot_t* sh, int D) {
     GPODE_CHECK_ARG(sh->row_lo >= 0 && sh->row_lo <= sh->row_hi && sh->row_hi <= n_total,
                     "row range [%lld,%lld) outside the %lld rows of the batch", (long long)sh->row_lo,
                     (long long)sh->row_hi, (long long)n_total);
-    (void)D;
     return 0;
 }
-}  // namespace
+
+int gpode_shoot_sum_launch(const double* work, int n_rows, int cols, double* sums, float* g_var, cudaStream_t st) {
+    shoot_sum_kernel<<<1, 256, 0, st>>>(work, n_rows, cols, sums, g_var);
+    GPODE_LAUNCH_CHECK();
+    return 0;
+}
 
 extern "C" int64_t gpode_shoot_work_doubles(void) { return (int64_t)kShootMaxCtas * kShootCols; }
 
 extern "C" int gpode_shoot_fwd(const float* packed, int D, int M, int S, const gpode_shoot_t* sh, const float* ss,
                                const float* t2, float* kstages, float* pred_out, float* seeds, double* sums_out,
                                float* grad_lik_var, double* work, void* stream) {
-    if (int rc = check_shoot(sh, D)) return rc;
+    if (int rc = gpode_check_shoot(sh)) return rc;
     const int64_t B = sh->row_hi - sh->row_lo;
     if (int rc = check_common(packed, D, M, S, B)) return rc;
     GPODE_CHECK_ARG(ss && t2 && sums_out && work, "NULL argument");
@@ -230,9 +235,7 @@ extern "C" int gpode_shoot_fwd(const float* packed, int D, int M, int S, const g
         default: break;
     }
     if (rc != 0) return rc;
-    shoot_sum_kernel<<<1, 256, 0, st>>>(work, grid, 2 + sh->D_obs, sums_out, grad_lik_var);
-    GPODE_LAUNCH_CHECK();
-    return 0;
+    return gpode_shoot_sum_launch(work, grid, 2 + sh->D_obs, sums_out, grad_lik_var, st);
 }
 
 static bool shoot_row_sums(int D, int M, int S, int64_t B) {
@@ -252,7 +255,7 @@ extern "C" int64_t gpode_shoot_bwd_vrows(int D, int M, int S, int64_t n_rows) {
 extern "C" int gpode_shoot_bwd(const float* packed, int D, int M, int S, const gpode_shoot_t* sh, const float* ss,
                                const float* t2, const float* kstages, const float* seeds, const float* g_ll,
                                const float* g_cons, float* grad_ss, float* vrows, float* acc, void* stream) {
-    if (int rc = check_shoot(sh, D)) return rc;
+    if (int rc = gpode_check_shoot(sh)) return rc;
     const int64_t B = sh->row_hi - sh->row_lo;
     if (int rc = check_common(packed, D, M, S, B)) return rc;
     if (B == 0) return 0;

@@ -45,6 +45,11 @@ __host__ __device__ inline size_t shoot_smem_bytes(int D, int Dobs, int nwarps) 
 }
 #define GPODE_SHOOT_MAX_DOBS 128
 
+// integrate.cu, shared with the large-D step (large_shoot.cu): checks of the descriptor and its row range; the ordered
+// float64 sum of the per-CTA partial rows [n_rows][cols] (cols = 2 + D_obs) into sums[2] and g_var[D_obs] (may be NULL)
+int gpode_check_shoot(const gpode_shoot_t* sh);
+int gpode_shoot_sum_launch(const double* work, int n_rows, int cols, double* sums, float* g_var, cudaStream_t st);
+
 #ifdef __CUDACC__
 template <int D>
 struct ShootSmem {

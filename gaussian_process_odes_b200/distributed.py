@@ -118,7 +118,8 @@ def sharded_shooting_loss(model, ys_local, ts, num_samples, n_global, world):
 # replicated sample tensor, no exchange -- and the only collective is ONE all-reduce(sum) of the flattened gradient of
 # every parameter: a rank's gradient w.r.t. the sampled states is non-zero only on its rows (+ the halo row).
 def enable_row_sharding(model, rank=None, world=None):
-    """Make ``model.build_lowerbound_terms`` integrate only this rank's block of segment rows (fused shooting step)."""
+    """Make ``model.build_lowerbound_terms`` integrate only this rank's block of segment rows (fused shooting step:
+    rk4, an affine decoder with D_obs <= 128 and a frozen constraint scale, at every state dimension 1 <= D <= 64)."""
     if rank is None:
         rank = dist.get_rank() if dist.is_available() and dist.is_initialized() else 0
         world = dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
@@ -146,7 +147,8 @@ def row_sharded_shooting_loss(model, ys, ts, num_samples, world=None):
 # all-reduce(sum) of all gradients delivers it. Every rank draws the same noise (full shape, same order, then sliced),
 # so the result equals the unsharded one.
 def enable_time_sharding(model, rank=None, world=None):
-    """Make ``model.build_lowerbound_terms`` evaluate only this rank's slice of the time axis (fused shooting step)."""
+    """Make ``model.build_lowerbound_terms`` evaluate only this rank's slice of the time axis (fused shooting step:
+    rk4, an affine decoder with D_obs <= 128 and a frozen constraint scale, at every state dimension 1 <= D <= 64)."""
     if rank is None:
         rank = dist.get_rank() if dist.is_available() and dist.is_initialized() else 0
         world = dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1

@@ -70,17 +70,19 @@ class UniformSequenceModel(BaseSequenceModel):
     def _fused_terms(self, ss_samples, ys, ts, halo=False, T_global=None):
         """Observation log-likelihood mean and constraint total through ONE integrator launch with the two terms
         evaluated on the segment end points inside the kernel (``ops.shooting_step``), or None when the configuration
-        has no fused kernel (solver other than rk4, D > 8, non-affine decoder, trainable constraint scale, CPU). Raises
+        has no fused kernel (solver other than rk4, D > 64, D_obs > 128, non-affine decoder, trainable constraint scale,
+        CPU). Above D = 8 the step runs on the large-D kernels (tcgen05 vector field, one epilogue kernel). Raises
         _FusedDoesNotFit, with this step's GP cache already built, when the fused forward does not fit in shared
         memory."""
         from ..core.dsvgp import DSVGP_Layer
         from ..core.constraints import _ScaleFamily
+        from ..ops import MAX_D_LARGE
         flow, lik, cons = self.flow, self.likelihood, self.constraint
         layer = flow.odefunc.diffeq
         S, N, T, D = ss_samples.shape
         affine = getattr(lik, "_affine", None)
         if not (self.fuse_elbo and ss_samples.is_cuda and flow.solver == "rk4" and isinstance(layer, DSVGP_Layer)
-                and D <= 8 and affine is not None and isinstance(cons, _ScaleFamily)
+                and D <= MAX_D_LARGE and affine is not None and isinstance(cons, _ScaleFamily)
                 and not cons.unconstrained_scale.requires_grad and cons.unconstrained_scale.numel() == 1):
             return None
         aff = affine(ss_samples)
@@ -136,8 +138,8 @@ class UniformSequenceModel(BaseSequenceModel):
         ss_loc = sd.sample_time_slice(num_samples, lo, hi + int(halo))          # (S, N, hi - lo (+1), D)
         fused = self._fused_terms(ss_loc, ys[:, lo:hi + int(halo)].contiguous(), ts, halo=halo, T_global=T)
         if fused is None:
-            raise RuntimeError("time sharding needs the fused shooting step (rk4, affine decoder, frozen constraint "
-                               "scale, D <= 8)")
+            raise RuntimeError("time sharding needs the fused shooting step (rk4, affine decoder with D_obs <= 128, "
+                               "frozen constraint scale, D <= 64)")
         observation_loglik_mean, constraint_total = fused
         entropy = sd.entropy_time_slice(lo, hi).sum()
         return (observation_loglik_mean, constraint_total / self.num_observations, entropy / self.num_observations,
@@ -164,8 +166,8 @@ class UniformSequenceModel(BaseSequenceModel):
             return (observation_loglik_mean, constraint_total / self.num_observations,
                     state_entropy.sum() / self.num_observations, initial_state_kl / self.num_observations)
         if self.row_shard is not None:
-            raise RuntimeError("row sharding needs the fused shooting step (rk4, affine decoder, frozen constraint "
-                               "scale, D <= 8)")
+            raise RuntimeError("row sharding needs the fused shooting step (rk4, affine decoder with D_obs <= 128, "
+                               "frozen constraint scale, D <= 64)")
         # one launch: S*N*T independent one-interval IVPs sharing one GP function draw
         predicted_xs = self.flow(x0=stack_segments(ss_samples), ts=ts[:2], rebuild_cache=rebuild_cache)  # (S*N*T, 2, D)
         predicted_xs = unstack_segments(predicted_xs[:, -1], (S, N, T, D))

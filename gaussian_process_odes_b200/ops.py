@@ -393,6 +393,31 @@ def loglik_mean(pred, ys, W, bias, var):
     return _LoglikMean.apply(pred, ys, W, bias, var)
 
 
+def _shoot_descriptor(ss, t2, D, ys, W, bias, lik_var, cons_scale, flags, row_lo, row_hi):
+    """Checked float32 views of the shooting-step inputs and their ``gpode_shoot_t`` -> (sh, tensors, row_lo, row_hi)"""
+    sc, tc = f32(ss, "ss"), f32(t2, "ts[:2]")
+    if sc.ndim != 4 or sc.shape[3] != D:
+        raise _lib.GpodeError("ss must be (S_mc,N,T,%d), got %s" % (D, tuple(sc.shape)))
+    if tc.numel() != 2:
+        raise _lib.GpodeError("the fused shooting step integrates one interval: ts[:2], got %d points" % tc.numel())
+    S_mc, N, T, _ = sc.shape
+    yc, Wc, vc, kc = f32(ys, "ys"), f32(W, "W"), f32(lik_var, "likelihood variance"), f32(cons_scale, "scale")
+    bc = f32(bias, "bias") if bias is not None else None
+    Dobs = Wc.shape[1]
+    if tuple(yc.shape) != (N, T, Dobs) or Wc.shape[0] != D or vc.numel() != Dobs or kc.numel() != 1 \
+            or (bc is not None and bc.numel() != Dobs):
+        raise _lib.GpodeError("inconsistent shooting shapes: ss %s ys %s W %s var %s scale %s" % (
+            tuple(sc.shape), tuple(yc.shape), tuple(Wc.shape), tuple(vc.shape), tuple(kc.shape)))
+    n_total = S_mc * N * T
+    row_lo, row_hi = int(row_lo), int(n_total if row_hi is None else row_hi)
+    sh = GpodeShoot()
+    sh.S_mc, sh.N, sh.T, sh.D_obs, sh.laplace = S_mc, N, T, Dobs, int(flags)   # bit 0 Laplace, bit 1 halo
+    sh.ys, sh.W, sh.bias = ptr(yc).value, ptr(Wc).value, (ptr(bc).value if bc is not None else None)
+    sh.lik_var, sh.cons_scale = ptr(vc).value, ptr(kc).value
+    sh.row_lo, sh.row_hi = row_lo, row_hi
+    return sh, (sc, tc, yc, Wc, bc, vc, kc), row_lo, row_hi
+
+
 class _ShootStep(torch.autograd.Function):
     """The integrator launch of the multiple-shooting ELBO with its two end-point terms fused in (``gpode_shoot_fwd`` /
     ``gpode_shoot_bwd``; reference ``src/gpode_shooting/models.py:119-135``): -> (log-likelihood SUM, constraint SUM,
@@ -403,29 +428,13 @@ class _ShootStep(torch.autograd.Function):
                 row_hi, want_grad, want_pred):
         lib = _lib.load()
         pc = PackedCache(Z, ell, var, nu, omega, phase, w)
-        sc, tc = f32(ss, "ss"), f32(t2, "ts[:2]")
-        if sc.ndim != 4 or sc.shape[3] != pc.D:
-            raise _lib.GpodeError("ss must be (S_mc,N,T,%d), got %s" % (pc.D, tuple(sc.shape)))
-        if tc.numel() != 2:
-            raise _lib.GpodeError("the fused shooting step integrates one interval: ts[:2], got %d points" % tc.numel())
-        S_mc, N, T, D = sc.shape
-        yc, Wc, vc, kc = f32(ys, "ys"), f32(W, "W"), f32(lik_var, "likelihood variance"), f32(cons_scale, "scale")
-        bc = f32(bias, "bias") if bias is not None else None
-        Dobs = Wc.shape[1]
-        if tuple(yc.shape) != (N, T, Dobs) or Wc.shape[0] != D or vc.numel() != Dobs or kc.numel() != 1 \
-                or (bc is not None and bc.numel() != Dobs):
-            raise _lib.GpodeError("inconsistent shooting shapes: ss %s ys %s W %s var %s scale %s" % (
-                tuple(sc.shape), tuple(yc.shape), tuple(Wc.shape), tuple(vc.shape), tuple(kc.shape)))
+        D = pc.D
+        sh, keep, row_lo, row_hi = _shoot_descriptor(ss, t2, D, ys, W, bias, lik_var, cons_scale, laplace, row_lo,
+                                                     row_hi)
+        sc, tc = keep[0], keep[1]
         if ctx.needs_input_grad[13]:
             raise _lib.GpodeError("the fused shooting step treats the constraint scale as a constant")
-        n_total = S_mc * N * T
-        row_lo, row_hi = int(row_lo), int(n_total if row_hi is None else row_hi)
-        B = row_hi - row_lo
-        sh = GpodeShoot()
-        sh.S_mc, sh.N, sh.T, sh.D_obs, sh.laplace = S_mc, N, T, Dobs, int(laplace)   # bit 0 Laplace, bit 1 halo
-        sh.ys, sh.W, sh.bias = ptr(yc).value, ptr(Wc).value, (ptr(bc).value if bc is not None else None)
-        sh.lik_var, sh.cons_scale = ptr(vc).value, ptr(kc).value
-        sh.row_lo, sh.row_hi = row_lo, row_hi
+        B, Dobs = row_hi - row_lo, sh.D_obs
         need_grad = want_grad and any(ctx.needs_input_grad)
         dev = sc.device
         kst = torch.empty(1, 4, B, D, dtype=torch.float32, device=dev) if need_grad else None
@@ -436,8 +445,8 @@ class _ShootStep(torch.autograd.Function):
         work = torch.empty(lib.gpode_shoot_work_doubles(), dtype=torch.float64, device=dev)
         _lib.call("gpode_shoot_fwd", ptr(pc.packed), pc.D, pc.M, pc.S, ctypes.byref(sh), ptr(sc), ptr(tc), ptr(kst),
                   ptr(pred), ptr(seeds), ptr(sums), ptr(gvar), ptr(work), stream_ptr())
-        ctx.pc, ctx.nu_shape, ctx.sh, ctx.keep = pc, nu.shape, sh, (yc, Wc, bc, vc, kc)
-        ctx.full = (row_lo == 0 and row_hi == n_total)
+        ctx.pc, ctx.nu_shape, ctx.sh, ctx.keep = pc, nu.shape, sh, keep
+        ctx.full = (row_lo == 0 and row_hi == sc.shape[0] * sc.shape[1] * sc.shape[2])
         ctx.var_shape = lik_var.shape
         if need_grad:
             ctx.save_for_backward(sc, tc, kst, seeds, gvar)
@@ -485,8 +494,73 @@ def shooting_step(ss, t2, Z, ell, var, nu, omega, phase, w, ys, W, bias, lik_var
     # ``halo``: the last time index of every sequence of this (time-sharded) batch is the next rank's first state --
     # the constraint's neighbour only, no observation term (flag bit 1 of gpode_shoot_t.laplace)
     flags = int(bool(laplace)) | (2 if halo else 0)
-    return _ShootStep.apply(ss, t2, Z, ell, var, nu, omega, phase, w, ys, W, bias, lik_var, cons_scale, flags, lo, hi,
-                            torch.is_grad_enabled(), want_pred)
+    D = Z.shape[1]
+    if D > MAX_D_REGISTER:
+        if D > MAX_D_LARGE:
+            raise _lib.GpodeError("the shooting step covers state dimensions up to %d, got D=%d" % (MAX_D_LARGE, D))
+        fn = _ShootStepLarge
+    else:
+        fn = _ShootStep
+    return fn.apply(ss, t2, Z, ell, var, nu, omega, phase, w, ys, W, bias, lik_var, cons_scale, flags, lo, hi,
+                    torch.is_grad_enabled(), want_pred)
+
+
+class _ShootStepLarge(torch.autograd.Function):
+    """``_ShootStep`` for 8 < D <= 64 (``gpode_shoot_fwd_large`` / ``gpode_shoot_bwd_large``): one RK4 interval on the
+    tcgen05 vector field, the two end-point terms and their seeds in one epilogue kernel, the large-D adjoint seeded
+    on the device. Same arguments and results."""
+
+    @staticmethod
+    def forward(ctx, ss, t2, Z, ell, var, nu, omega, phase, w, ys, W, bias, lik_var, cons_scale, laplace, row_lo,
+                row_hi, want_grad, want_pred):
+        lib = _lib.load()
+        field = LargeField(Z, ell, var, nu, omega, phase, w)
+        D = field.D
+        sh, keep, row_lo, row_hi = _shoot_descriptor(ss, t2, D, ys, W, bias, lik_var, cons_scale, laplace, row_lo,
+                                                     row_hi)
+        sc, tc = keep[0], keep[1]
+        if ctx.needs_input_grad[13]:
+            raise _lib.GpodeError("the fused shooting step treats the constraint scale as a constant")
+        B, Dobs = row_hi - row_lo, sh.D_obs
+        need_grad = want_grad and any(ctx.needs_input_grad)
+        dev = sc.device
+        kst = torch.empty(1, 4, B, D, dtype=torch.float32, device=dev) if need_grad else None
+        seeds = torch.empty(2, B, D, dtype=torch.float32, device=dev) if need_grad else None
+        pred = torch.empty(B, D, dtype=torch.float32, device=dev) if want_pred else None
+        sums = torch.empty(2, dtype=torch.float64, device=dev)
+        gvar = torch.empty(Dobs, dtype=torch.float32, device=dev) if need_grad else None
+        work = torch.empty(lib.gpode_shoot_large_work_doubles(D, B), dtype=torch.float64, device=dev)
+        _lib.call("gpode_shoot_fwd_large", ptr(field.packed), ctypes.byref(field.struct), ctypes.byref(sh), ptr(sc),
+                  ptr(tc), ptr(kst), ptr(pred), ptr(seeds), ptr(sums), ptr(gvar), ptr(work), stream_ptr())
+        ctx.field, ctx.nu_shape, ctx.sh, ctx.keep = field, nu.shape, sh, keep
+        ctx.full = (row_lo == 0 and row_hi == sc.shape[0] * sc.shape[1] * sc.shape[2])
+        ctx.var_shape = lik_var.shape
+        if need_grad:
+            ctx.save_for_backward(sc, tc, kst, seeds, gvar)
+        out32 = sums.to(torch.float32)
+        if pred is not None:
+            ctx.mark_non_differentiable(pred)
+        return out32[0], out32[1], pred
+
+    @staticmethod
+    def backward(ctx, g_ll, g_cons, _g_pred):
+        field, sh = ctx.field, ctx.sh
+        sc, tc, kst, seeds, gvar = ctx.saved_tensors
+        B = seeds.shape[1]
+        dev = sc.device
+        zero = lambda: torch.zeros((), dtype=torch.float32, device=dev)
+        g_ll = f32(g_ll, "grad") if g_ll is not None else zero()
+        g_cons = f32(g_cons, "grad") if g_cons is not None else zero()
+        g_ss = torch.empty_like(sc) if ctx.full else torch.zeros_like(sc)
+        acc = field.new_acc()
+        work = torch.empty(_lib.load().gpode_shoot_large_work_doubles(field.D, B), dtype=torch.float64, device=dev)
+        _lib.call("gpode_shoot_bwd_large", ptr(field.packed_bwd), ctypes.byref(field.struct), ctypes.byref(sh),
+                  ptr(sc), ptr(tc), ptr(kst), ptr(seeds), ptr(g_ll), ptr(g_cons), ptr(g_ss), ptr(acc), ptr(work),
+                  stream_ptr())
+        g_Z, g_ell, g_var, g_nu = field.finalize(acc, B)
+        g_lik = (gvar * g_ll).reshape(ctx.var_shape)
+        return (g_ss, None, g_Z, g_ell, g_var, g_nu.reshape(ctx.nu_shape), None, None, None, None, None, None, g_lik,
+                None, None, None, None, None, None)
 
 
 MAX_D_REGISTER = 8    # GPODE_MAX_D: differentiable register-resident kernels

@@ -368,6 +368,27 @@ int gpode_shoot_bwd(const float* packed, int D, int M, int S, const gpode_shoot_
                     const float* kstages, const float* seeds, const float* g_ll, const float* g_cons, float* grad_ss,
                     float* vrows, float* acc, void* stream);
 
+/* The same step for 8 < D <= GPODE_MAX_D_LARGE, with the same descriptor, row range, flag word, sums, grad_lik_var,
+ * seeds [2,B,D], kstages [1,4,B,D] and optional pred_out: the interval runs through gpode_rk4_fwd_large_dev (pred_out is
+ * bitwise its xs[1]), then ONE epilogue kernel (one warp per row, decoder in shared memory) evaluates both terms and the
+ * seeds on the end points; no [B,D_obs] tensor is written. kstages and seeds are both NULL or both given.
+ *   gpode_shoot_bwd_large: grad_xs = [0, g_ll seeds[0] + g_cons seeds[1]] (scalars read on the device), then
+ *     gpode_rk4_bwd_large into grad_ss[row_lo:row_hi] (parameter partial sums added to acc_large, zeroed by the caller;
+ *     follow with gpode_grads_finalize_large over B = row_hi - row_lo rows), then the constraint's pull on the next
+ *     state with the rules of gpode_shoot_bwd (row row_hi included; the caller zeroes grad_ss for a partial range).
+ *   gpode_shoot_large_work_doubles: float64 elements of `work` either call needs for n_rows = row_hi - row_lo (-1 for
+ *     D outside 9..64). Pure host arithmetic; forward and backward may share one block.
+ * Sums and gradients are bitwise reproducible (per-CTA partial rows added in a fixed order, no atomics); launch sizes
+ * follow from the host shapes (no host read, no allocation). */
+int64_t gpode_shoot_large_work_doubles(int D, int64_t n_rows);
+int gpode_shoot_fwd_large(const float* packed_large, const gpode_cache_t* cache, const gpode_shoot_t* sh,
+                          const float* ss, const float* t2, float* kstages, float* pred_out, float* seeds,
+                          double* sums_out, float* grad_lik_var, double* work, void* stream);
+int gpode_shoot_bwd_large(const float* packed_bwd, const gpode_cache_t* cache, const gpode_shoot_t* sh,
+                          const float* ss, const float* t2, const float* kstages, const float* seeds,
+                          const float* g_ll, const float* g_cons, float* grad_ss, float* acc_large, double* work,
+                          void* stream);
+
 /* Kernel-selection options (the library's only process-wide mutable state). Defaults are read from the environment
  * once (GPODE_BWD_MMA, GPODE_FWD_MMA); names:
  *   "bwd_mma" / "fwd_mma" (1): tensor-core adjoint / forward at D = 4, 5 and B >= SMs x 384 rows; 0 = FFMA2 kernels.
